@@ -297,7 +297,7 @@ def run_ours(args):
             return c.mstep(threshold=-1.0)  # reads sum_logp / n_utt / updated back: the step's result
         return em_iteration
 
-    def timed(c, fn, steps, warmup, kernel_names=()):
+    def timed(c, fn, steps, warmup, kernel_names=(), last=None):
         st = torch.cuda.ExternalStream(c.stream(), device=local)
         for _ in range(warmup):
             fn()
@@ -320,13 +320,15 @@ def run_ours(args):
                 with torch.cuda.stream(st):
                     dist.all_reduce(align)
             ev[i][0].record(st)
-            fn()
+            out = fn()
             ev[i][1].record(st)
             c.synchronize()
             for k in kernel_names:
                 kms[k].append(c.kernel_ms(k))
         torch.cuda.synchronize()
         wall = time.perf_counter() - wall0
+        if last is not None:  # what the last timed step returned
+            last.append(out)
         if world > 1:
             dist.barrier()
         total_ms = sum(a.elapsed_time(b) for a, b in ev)
@@ -363,8 +365,11 @@ def run_ours(args):
 
     sampler = ClockSampler(local)
     sampler.start()
-    tot_ms, launches, _, wall = timed(ctx, step_resident, args.steps, args.warmup)
+    last_step = []
+    tot_ms, launches, _, wall = timed(ctx, step_resident, args.steps, args.warmup, last=last_step)
     clocks = sampler.stop()
+    if args.dump_outputs and rank == 0:   # before the passes below re-estimate the models further
+        dump_outputs(args.dump_outputs, last_step[0], ctx.get_models(D))
     kms, ar_ms = kernel_pass(ctx, labels, max(3, min(args.steps, 20)))
     ar_alone_ms = None
     if world > 1 and ctx._ar is not None:
@@ -566,6 +571,18 @@ def run_ours(args):
         print(json.dumps(out))
     if world > 1:
         dist.destroy_process_group()
+
+
+def dump_outputs(out_dir, step_result, models):
+    """What the last timed EM iteration hands its caller, one float64 array per DIR/<name>.npy: the M-step's per-word
+    results (sum of the utterance log-likelihoods, utterance count, re-estimated flag) and the re-estimated model set.
+    The workload is generated from fixed seeds, so two builds run with the same arguments can be compared file by file."""
+    os.makedirs(out_dir, exist_ok=True)
+    lp, nu, upd = step_result
+    arrays = {"sum_logp": lp, "n_utt": nu, "updated": upd,
+              "A": models.A, "c": models.c, "mu": models.mu, "inv_var": models.iv, "det": models.det}
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), np.asarray(a, dtype=np.float64))
 
 
 def training_rooflines(kms, F, N, M, V, pk, tf32_peak, traffic, acc_h=False):
@@ -1003,7 +1020,10 @@ def main():
     ap.add_argument("--c3-utts", type=int, default=C3_UTTS)
     ap.add_argument("--c4-utts", type=int, default=C4_UTTS)
     ap.add_argument("--c5-models", type=int, default=C5_MODELS)
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write what the last timed EM iteration computed to DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be at least 1 and --warmup at least 0")
     if args.impl == "reference":
         run_reference(args)
     else:

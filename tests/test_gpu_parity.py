@@ -13,6 +13,7 @@ import pytest
 from oracle import oracle as o
 from oracle import ref as r
 from speech_recognition_hmm_continuous_b200 import api, synth
+from cli_lists import write_list
 
 pytestmark = pytest.mark.gpu
 RTOL = 1e-4  # north_star tolerance for floating-point results
@@ -286,9 +287,10 @@ def test_viterbi_paths_bit_exact_and_scores(ctx):
 
 
 # ---------------------------------------------------------------------- drop-in programs ----
-def test_cli_train_then_test_matches_reference_outputs(golden_dir, tmp_path):
+def test_cli_train_then_test_matches_reference_outputs(golden_dir, tmp_path, monkeypatch):
     """bin/hmm_continuous_fs and bin/recognition_continuous_fs with the reference's argv on the
     synth_c1 case: reports agree with the reference's (iterations, mean probability to 1e-4, labels)."""
+    monkeypatch.chdir(tmp_path)
     g = np.load(os.path.join(golden_dir, "synth_c1.npz"))
     V, N, M, D = int(g["V"]), int(g["N"]), int(g["M"]), int(g["D"])
     cen, s = synth.make_centres(V, N, M, D, seed=1234)
@@ -303,9 +305,9 @@ def test_cli_train_then_test_matches_reference_outputs(golden_dir, tmp_path):
             api.write_features(f, x[off[u]:off[u + 1]])
             files.append(f)
         lst = str(tmp_path / ("list%d.txt" % v))
-        open(lst, "w").write("\n".join(files) + "\n")
+        write_list(lst, files)
         hmm = str(tmp_path / ("w%d.hmm" % v))
-        subprocess.run([os.path.join(bindir, "hmm_continuous_fs"), "word%d" % v, str(N), "1", str(M), lst, hmm],
+        subprocess.run([os.path.join(bindir, "hmm_continuous_fs"), "word%d" % v, str(N), "1", str(M), lst, os.path.basename(hmm)],
                        check=True, stdout=subprocess.DEVNULL)
         mean, its = r.parse_train_report(hmm[:-4] + ".txt")
         assert its == g["iterations"][v] and abs(mean - g["mean_logp"][v]) <= RTOL * abs(g["mean_logp"][v])
@@ -315,8 +317,8 @@ def test_cli_train_then_test_matches_reference_outputs(golden_dir, tmp_path):
         f = str(tmp_path / ("te%d.bin" % u))
         api.write_features(f, xt[offt[u]:offt[u + 1]])
         tf.append(f)
-    open(str(tmp_path / "models.txt"), "w").write("\n".join(models) + "\n")
-    open(str(tmp_path / "feat.txt"), "w").write("\n".join(tf) + "\n")
+    write_list(tmp_path / "models.txt", models)
+    write_list(tmp_path / "feat.txt", tf)
     open(str(tmp_path / "words.txt"), "w").write("\n".join("word%d" % v for v in g["test_labels"]) + "\n")
     res = str(tmp_path / "res.txt")
     subprocess.run([os.path.join(bindir, "recognition_continuous_fs"), "1", str(tmp_path / "models.txt"), "1",
@@ -332,10 +334,11 @@ def test_cli_train_then_test_matches_reference_outputs(golden_dir, tmp_path):
         assert strip(txt) == strip(open(ref_res).read())
 
 
-def test_cli_two_model_sets_weighted_sum(tmp_path):
+def test_cli_two_model_sets_weighted_sum(tmp_path, monkeypatch):
     """recognition_continuous_fs with models_number = 2 (R-FS:326-364): two model sets of different topology and
     feature width, each with its own feature list; the score of a word is sum_j coef_j * logP_j and the label its
     argmax.  Expected values from the oracle's forward scorer on every (utterance, word, set)."""
+    monkeypatch.chdir(tmp_path)
     V, labels = 4, [0, 1, 2, 3, 2, 0]
     sets = []
     for j, (N, M, D) in enumerate(((5, 3, 39), (3, 2, 13))):
@@ -348,8 +351,8 @@ def test_cli_two_model_sets_weighted_sum(tmp_path):
         for u in range(len(labels)):
             fp.append(str(tmp_path / ("s%du%d.bin" % (j, u))))
             api.write_features(fp[-1], x[off[u]:off[u + 1]])
-        open(str(tmp_path / ("models%d.txt" % j)), "w").write("\n".join(mp) + "\n")
-        open(str(tmp_path / ("feat%d.txt" % j)), "w").write("\n".join(fp) + "\n")
+        write_list(tmp_path / ("models%d.txt" % j), mp)
+        write_list(tmp_path / ("feat%d.txt" % j), fp)
         sets.append((ms, x, off))
     open(str(tmp_path / "words.txt"), "w").write("\n".join("word%d" % v for v in labels) + "\n")
     coef = (0.75, 0.25)
@@ -452,9 +455,10 @@ def test_two_stream_model_matches_reference(golden_dir):
         c.close()
 
 
-def test_cli_two_streams_match_reference_outputs(golden_dir, tmp_path):
+def test_cli_two_streams_match_reference_outputs(golden_dir, tmp_path, monkeypatch):
     """The drop-in programs with param_number = 2 on the case the reference itself was run on (synth_p2.npz): training
     report (iterations, mean probability), the two-stream .hmm files, and the recogniser's result file line by line."""
+    monkeypatch.chdir(tmp_path)
     g = np.load(os.path.join(golden_dir, "synth_p2.npz"))
     V, N, off, offt = int(g["V"]), int(g["N"]), g["off"], g["offt"]
     bindir = os.path.join(os.path.dirname(api.LIB_PATH), "bin")
@@ -467,9 +471,9 @@ def test_cli_two_streams_match_reference_outputs(golden_dir, tmp_path):
                 files.append(str(tmp_path / ("tr_s%d_%d.bin" % (p, u))))
                 api.write_features(files[-1], g["x%d" % p][off[u]:off[u + 1]])
             lists.append(str(tmp_path / ("list_s%d_w%d.txt" % (p, v))))
-            open(lists[-1], "w").write("\n".join(files) + "\n")
+            write_list(lists[-1], files)
         hmms.append(str(tmp_path / ("w%d.hmm" % v)))
-        subprocess.run([os.path.join(bindir, "hmm_continuous_fs"), "word%d" % v, str(N), "2", str(g["M"][0]), str(g["M"][1]), lists[0], lists[1], hmms[-1]],
+        subprocess.run([os.path.join(bindir, "hmm_continuous_fs"), "word%d" % v, str(N), "2", str(g["M"][0]), str(g["M"][1]), lists[0], lists[1], os.path.basename(hmms[-1])],
                        check=True, stdout=subprocess.DEVNULL)
         mean, its = r.parse_train_report(hmms[-1][:-4] + ".txt")
         assert its == g["iterations"][v] and abs(mean - g["mean_logp"][v]) <= RTOL * abs(g["mean_logp"][v])
@@ -487,8 +491,8 @@ def test_cli_two_streams_match_reference_outputs(golden_dir, tmp_path):
             files.append(str(tmp_path / ("te_s%d_%d.bin" % (p, u))))
             api.write_features(files[-1], g["xt%d" % p][offt[u]:offt[u + 1]])
         feats.append(str(tmp_path / ("feat_s%d.txt" % p)))
-        open(feats[-1], "w").write("\n".join(files) + "\n")
-    open(str(tmp_path / "models.txt"), "w").write("\n".join(hmms) + "\n")
+        write_list(feats[-1], files)
+    write_list(tmp_path / "models.txt", hmms)
     open(str(tmp_path / "words.txt"), "w").write("\n".join("word%d" % v for v in g["test_labels"]) + "\n")
     res = str(tmp_path / "res.txt")
     out = subprocess.run([os.path.join(bindir, "recognition_continuous_fs"), "1", str(tmp_path / "models.txt"), "1", feats[0], feats[1],
@@ -1015,12 +1019,13 @@ def test_resident_forward_backward_other_state_counts(ctx, N):
 
 
 # ------------------------------------------------- resume from a model file (optional last argument) ----
-def test_cli_resumes_from_an_initial_model(tmp_path):
+def test_cli_resumes_from_an_initial_model(tmp_path, monkeypatch):
     """hmm_continuous_fs ... out.hmm initial.hmm (T-FS:216-222; the reference reads argv[argc] there and would crash,
     SURVEY section 5 'checkpoint / resume'): training continues from the model in the file.  The first model is trained
     on two utterances, the resumed run on all eight, so that it has several iterations of real work.  Expected values:
     the oracle's EM loop started from the same file -- equal iteration count, mean log-probability and parameters
     within 1e-4 (the test first checks that no stopping decision of that loop is within 5 % of the threshold)."""
+    monkeypatch.chdir(tmp_path)
     N, M = 4, 2
     cen, sc = synth.make_centres(1, N, M, 39, seed=341)
     x, off = synth.make_utterances(cen, sc, [0] * 8, seed=342, tmin=50, tmax=80)
@@ -1029,12 +1034,12 @@ def test_cli_resumes_from_an_initial_model(tmp_path):
         files.append(str(tmp_path / ("u%d.bin" % u)))
         api.write_features(files[-1], x[off[u]:off[u + 1]])
     lst2, lst = str(tmp_path / "list2.txt"), str(tmp_path / "list.txt")
-    open(lst2, "w").write("\n".join(files[:2]) + "\n")
-    open(lst, "w").write("\n".join(files) + "\n")
+    write_list(lst2, files[:2])
+    write_list(lst, files)
     exe = os.path.join(os.path.dirname(api.LIB_PATH), "bin", "hmm_continuous_fs")
     first, second = str(tmp_path / "first.hmm"), str(tmp_path / "second.hmm")
-    subprocess.run([exe, "word", str(N), "1", str(M), lst2, first], check=True, stdout=subprocess.DEVNULL)
-    subprocess.run([exe, "word", str(N), "1", str(M), lst, second, first], check=True, stdout=subprocess.DEVNULL)
+    subprocess.run([exe, "word", str(N), "1", str(M), lst2, "first.hmm"], check=True, stdout=subprocess.DEVNULL)
+    subprocess.run([exe, "word", str(N), "1", str(M), lst, "second.hmm", "first.hmm"], check=True, stdout=subprocess.DEVNULL)
     mean2, its2 = r.parse_train_report(second[:-4] + ".txt")
     # the oracle's loop from the same start (T-FS:238-358), keeping the stopping rule's variations
     mo = r.read_model(first)
@@ -1219,9 +1224,10 @@ def test_viterbi_tiny_cases_against_brute_force():
     c.close()
 
 
-def test_cli_job_file_runs_every_line_in_one_process(tmp_path):
+def test_cli_job_file_runs_every_line_in_one_process(tmp_path, monkeypatch):
     """`hmm_continuous_fs @jobs.txt` (one ordinary argument list per line, one CUDA context for all of them) writes the same
     models and reports as one invocation per word."""
+    monkeypatch.chdir(tmp_path)
     N, M, V = 5, 3, 3
     cen, sc = synth.make_centres(V, N, M, 39, seed=901)
     labels = np.repeat(np.arange(V), 5)
@@ -1234,9 +1240,9 @@ def test_cli_job_file_runs_every_line_in_one_process(tmp_path):
             files.append(str(tmp_path / ("w%d_u%d.bin" % (v, u))))
             api.write_features(files[-1], x[off[u]:off[u + 1]])
         lst = str(tmp_path / ("list%d.txt" % v))
-        open(lst, "w").write("\n".join(files) + "\n")
-        subprocess.run([exe, "word%d" % v, str(N), "1", str(M), lst, str(tmp_path / ("single%d.hmm" % v))], check=True, stdout=subprocess.DEVNULL)
-        jobs.append("word%d %d 1 %d %s %s" % (v, N, M, lst, str(tmp_path / ("batch%d.hmm" % v))))
+        write_list(lst, files)
+        subprocess.run([exe, "word%d" % v, str(N), "1", str(M), lst, "single%d.hmm" % v], check=True, stdout=subprocess.DEVNULL)
+        jobs.append("word%d %d 1 %d %s batch%d.hmm" % (v, N, M, lst, v))
     jf = str(tmp_path / "jobs.txt")
     open(jf, "w").write("\n".join(jobs) + "\n\n")
     subprocess.run([exe, "@" + jf], check=True, stdout=subprocess.DEVNULL)

@@ -11,6 +11,7 @@ import pytest
 from oracle import oracle as o
 from oracle import ref as r
 from speech_recognition_hmm_continuous_b200 import api, synth
+from cli_lists import write_list
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 
@@ -93,7 +94,8 @@ def test_model_file_format(tmp_path):
 
 
 @pytest.mark.skipif(not r.available("d39m16"), reason="oracle/_ref not built")
-def test_reads_model_written_by_reference(tmp_path):
+def test_reads_model_written_by_reference(tmp_path, monkeypatch):
+    monkeypatch.chdir(tmp_path)
     x, off = _case(3, 78)
     files = []
     for u in range(len(off) - 1):
@@ -101,8 +103,8 @@ def test_reads_model_written_by_reference(tmp_path):
         api.write_features(f, x[off[u]:off[u + 1]])
         files.append(f)
     lst = str(tmp_path / "l.txt")
-    open(lst, "w").write("\n".join(files) + "\n")
-    r.run_train_cli("d39m16", "abc", 5, 3, lst, str(tmp_path / "m.hmm"))
+    write_list(lst, files)
+    r.run_train_cli("d39m16", "abc", 5, 3, "l.txt", "m.hmm")
     a = api.read_model(str(tmp_path / "m.hmm"))
     b = r.read_model(str(tmp_path / "m.hmm"))
     assert a.words == ["abc"]
@@ -239,10 +241,11 @@ def test_model_set_reader_takes_32_bit_headers_and_reports_bad_files(tmp_path):
         api.read_model_set([str(tmp_path / "missing.hmm")])
 
 
-def test_model_set_reader_reads_reference_written_files(tmp_path):
+def test_model_set_reader_reads_reference_written_files(tmp_path, monkeypatch):
     """Models written by the compiled reference trainer come back identical through the bulk reader."""
     if not r.available("d39m16"):
         pytest.skip("compiled reference not present")
+    monkeypatch.chdir(tmp_path)
     paths = []
     for w in range(2):
         x, off = _case(3, 78 + w)
@@ -252,9 +255,9 @@ def test_model_set_reader_reads_reference_written_files(tmp_path):
             api.write_features(f, x[off[u]:off[u + 1]])
             files.append(f)
         lst = str(tmp_path / ("l%d.txt" % w))
-        open(lst, "w").write("\n".join(files) + "\n")
+        write_list(lst, files)
         paths.append(str(tmp_path / ("m%d.hmm" % w)))
-        r.run_train_cli("d39m16", "word%d" % w, 5, 3, lst, paths[-1])
+        r.run_train_cli("d39m16", "word%d" % w, 5, 3, os.path.basename(lst), os.path.basename(paths[-1]))
     back = api.read_model_set(paths)
     assert back.words == ["word0", "word1"]
     for w in range(2):
@@ -286,11 +289,12 @@ def test_multi_stream_model_file_round_trip_and_reference_layout(tmp_path, golde
     assert open(one, "rb").read() == open(one_s, "rb").read()
 
 
-def test_multi_stream_model_file_written_by_reference(tmp_path, golden_dir):
+def test_multi_stream_model_file_written_by_reference(tmp_path, golden_dir, monkeypatch):
     """The reference trainer run with two streams writes a file our reader takes (and vice versa: byte-identical rewrite)."""
     if not r.available("p2"):
         pytest.skip("compiled two-stream reference not present")
     import subprocess
+    monkeypatch.chdir(tmp_path)
     g = np.load(os.path.join(golden_dir, "synth_p2.npz"))
     off, lists = g["off"], []
     for p in range(2):
@@ -299,9 +303,9 @@ def test_multi_stream_model_file_written_by_reference(tmp_path, golden_dir):
             files.append(str(tmp_path / ("s%d_%d.bin" % (p, u))))
             api.write_features(files[-1], g["x%d" % p][off[u]:off[u + 1]])
         lists.append(str(tmp_path / ("l%d.txt" % p)))
-        open(lists[-1], "w").write("\n".join(files) + "\n")
+        write_list(lists[-1], files)
     hmm = str(tmp_path / "ref.hmm")
-    subprocess.run([os.path.join(r.REF_DIR, "hmm_fs_p2"), "word0", str(int(g["N"])), "2", str(g["M"][0]), str(g["M"][1]), lists[0], lists[1], hmm],
+    subprocess.run([os.path.join(r.REF_DIR, "hmm_fs_p2"), "word0", str(int(g["N"])), "2", str(g["M"][0]), str(g["M"][1]), "l0.txt", "l1.txt", "ref.hmm"],
                    stdout=subprocess.DEVNULL, check=True)
     back = api.read_model_streams(hmm)
     for p in range(2):
@@ -332,7 +336,7 @@ def test_cli_usage_and_file_errors():
     assert p.returncode == 1 and "does not match the argument list" in p.stdout.decode()
 
 
-def test_cli_refuses_models_beyond_the_state_limit_up_front(tmp_path):
+def test_cli_refuses_models_beyond_the_state_limit_up_front(tmp_path, monkeypatch):
     """The kernels are built for HMMCU_MAX_STATES = 8 states per model (the reference allows 20 / 15, T-FS:41, R-FS:37).
     Both programs say so before reading any feature file or touching the device; .hmm files with more states are still
     read and written by the host-side file code (HMMH_MAX_FILE_STATES)."""
@@ -354,7 +358,8 @@ def test_cli_refuses_models_beyond_the_state_limit_up_front(tmp_path):
     back = api.read_model(hmm)
     assert back.N == N and np.array_equal(back.mu, ms.mu)
     ml = str(tmp_path / "models.txt")
-    open(ml, "w").write(hmm + "\n")
+    monkeypatch.chdir(tmp_path)
+    write_list(ml, [hmm])
     fl, wl = str(tmp_path / "f.txt"), str(tmp_path / "w.txt")   # empty test set: the model check comes before any device work
     open(fl, "w").close()
     open(wl, "w").close()
