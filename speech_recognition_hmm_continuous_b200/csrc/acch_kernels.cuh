@@ -118,6 +118,7 @@ __global__ void k_pack_wT_h(const double *__restrict__ mu, const double *__restr
                             unsigned short *__restrict__ images, float *__restrict__ kcT) {
   const int img = blockIdx.y, v = img / nRB, rb = img - v * nRB;
   const int KP = 2 * DP;
+  pdl_wait();
   unsigned short *im = images + (size_t)img * (ah_image_bytes(KP) / 2);
   for (int idx = blockIdx.x * blockDim.x + threadIdx.x; idx < 128 * KP; idx += gridDim.x * blockDim.x) {
     const int r = idx / KP, k = idx - r * KP;
@@ -192,6 +193,10 @@ k_accum_h(const TcTile *__restrict__ units, int nunits, const int32_t *__restric
   __syncthreads();
   tc_fence_after();
   const uint32_t tmem0 = (uint32_t)lds_i32(tmem_slot);
+  // Above: only the unit table (uploaded with the training map) and this CTA's own shared and tensor memory.  Below:
+  // gamma (k_fb_res), logb (k_emis_ws) and x16 (k_pack_x16) of this launch sequence, and the statistics.
+  pdl_wait();
+  pdl_trigger();  // this CTA's work is a fixed unit range: nothing is left to claim
 
   auto img_at = [&](int ui) -> int {
     if (ui < u_begin || ui >= u_end) return -1;

@@ -32,6 +32,7 @@
 // stages them, runs the chains (two lanes per utterance), then forms gamma and the transition sums with all 128
 // threads over frames, and writes gamma out through a small staging buffer.  Per-utterance sums go to a row of
 // `ustats`; k_fb_reduce adds the rows of every model in a fixed order (bit-reproducible statistics).
+// The batch counter is zeroed once when it is allocated; the last team to leave each launch zeroes it again.
 #pragma once
 #include "fb_kernels.cuh"
 
@@ -226,12 +227,19 @@ k_fb_res(const float *__restrict__ logb, const int64_t *__restrict__ off, const 
     }
   };
   for (int i = tt; i < 32 * RS; i += kResTeamThreads) S.dummy[i] = 0x3fe00000u;  // 0.5
+  pdl_wait();  // logb comes from the emission kernel just before
   if (tt == 0) S.next = atomicAdd(counter, 1);
   for (;;) {
     stamp();
     team_sync();
     const int b = S.next;
-    if (b >= nbatches) break;
+    if (b >= nbatches) {
+      // Every team makes exactly one claim past the end, so the claim nbatches + teams - 1 is the last access to the
+      // counter in this launch: that team leaves it at 0 for the next one.
+      if (tt == 0 && b == nbatches + (int)gridDim.x * kResTeams - 1) atomicExch(counter, 0);
+      pdl_trigger();
+      break;
+    }
     const ResBatch bd = batches[b];
     if (role == 0) {  // the batch's utterances: one lane each; word offsets by a prefix sum over the lanes
       int T = 0;

@@ -10,6 +10,7 @@
 #include <atomic>
 #include <map>
 #include <string>
+#include <utility>
 #include <vector>
 
 #include "hmm_cuda.h"
@@ -223,6 +224,25 @@ static int fail(hmmcu_ctx *c, int code, const char *fmt, ...) {
     if (e_ != cudaSuccess)                                                                          \
       return fail(ctx, HMMCU_ECUDA, "kernel launch failed: %s (%s:%d)", cudaGetErrorString(e_), __FILE__, __LINE__); \
   } while (0)
+
+// A launch with programmatic dependent launch: the kernel may be scheduled as soon as every CTA of the previous kernel
+// of the stream has called pdl_trigger() or exited, and its CTAs run up to pdl_wait() (kernels.cuh) meanwhile.  Only
+// for kernels that call pdl_wait() in every CTA before they touch what an earlier kernel wrote.  Under stream capture
+// the edge from the previous kernel node becomes a programmatic edge of the graph.
+template <typename... KArgs, typename... Args>
+static cudaError_t launch_pdl(void (*kernel)(KArgs...), dim3 grid, dim3 block, size_t smem, cudaStream_t st, Args &&...args) {
+  cudaLaunchAttribute attr;
+  attr.id = cudaLaunchAttributeProgrammaticStreamSerialization;
+  attr.val.programmaticStreamSerializationAllowed = 1;
+  cudaLaunchConfig_t cfg = {};
+  cfg.gridDim = grid;
+  cfg.blockDim = block;
+  cfg.dynamicSmemBytes = smem;
+  cfg.stream = st;
+  cfg.attrs = &attr;
+  cfg.numAttrs = 1;
+  return cudaLaunchKernelEx(&cfg, kernel, std::forward<Args>(args)...);
+}
 
 static void t_begin(hmmcu_ctx *ctx, const char *name) {
   if (!ctx->timing) return;
@@ -1014,8 +1034,8 @@ static int ensure_simt_pack(hmmcu_ctx *ctx) {
 // additive constants of all Gaussians (log2 units), shared by the tensor-core W packers
 static int launch_pack_kc(hmmcu_ctx *ctx) {
   const int64_t VG = (int64_t)ctx->V * ctx->G;
-  k_pack_kc<<<(unsigned)((VG * 32 + 255) / 256), 256, 0, ctx->st>>>(ctx->mu.as<double>(), ctx->iv.as<double>(), ctx->det.as<double>(),
-                                                                    ctx->c.as<double>(), ctx->ctr.as<double>(), VG, ctx->D, ctx->kc2.as<float>());
+  CK(launch_pdl(k_pack_kc, (unsigned)((VG * 32 + 255) / 256), 256, 0, ctx->st, ctx->mu.as<double>(), ctx->iv.as<double>(),
+                ctx->det.as<double>(), ctx->c.as<double>(), ctx->ctr.as<double>(), VG, ctx->D, ctx->kc2.as<float>()));
   LAUNCH_CHECK();
   return HMMCU_OK;
 }
@@ -1049,9 +1069,9 @@ static bool h_acc_on(const hmmcu_ctx *ctx) {
 static int launch_pack_acc(hmmcu_ctx *ctx) {
   const int KP = 2 * ctx->DP, nRB = (ctx->G + 127) / 128, nimg = ctx->V * nRB;
   if (h_acc_on(ctx)) {
-    k_pack_wT_h<<<dim3((128 * KP + 255) / 256, nimg), 256, 0, ctx->st>>>(ctx->mu.as<double>(), ctx->iv.as<double>(), ctx->kc2.as<float>(),
-                                                                         ctx->ctr.as<double>(), ctx->acc_sc.as<float>(), ctx->G, nRB, ctx->D, ctx->DP,
-                                                                         ctx->acc_images16.as<unsigned short>(), ctx->acc_kc.as<float>());
+    CK(launch_pdl(k_pack_wT_h, dim3((128 * KP + 255) / 256, nimg), 256, 0, ctx->st, ctx->mu.as<double>(), ctx->iv.as<double>(),
+                  ctx->kc2.as<float>(), ctx->ctr.as<double>(), ctx->acc_sc.as<float>(), ctx->G, nRB, ctx->D, ctx->DP,
+                  ctx->acc_images16.as<unsigned short>(), ctx->acc_kc.as<float>()));
     LAUNCH_CHECK();
     return HMMCU_OK;
   }
@@ -1147,9 +1167,9 @@ static bool train16_wanted(const hmmcu_ctx *) { return false; }
 
 static int launch_pack_ws(hmmcu_ctx *ctx, hmmcu_ctx::TcSet &ts) {
   const int KP = 2 * ctx->DP;
-  k_pack_w_ws<<<dim3((ts.TN * KP + 255) / 256, ts.nimg), 256, 0, ctx->st>>>(ctx->mu.as<double>(), ctx->iv.as<double>(), ctx->kc2.as<float>(),
-                                                                            ctx->ctr.as<double>(), ctx->M, ws_pad_m(ctx->M), ctx->D, ctx->DP, ts.TN,
-                                                                            ts.s0.as<int32_t>(), ts.ns.as<int32_t>(), ts.images.as<float>());
+  CK(launch_pdl(k_pack_w_ws, dim3((ts.TN * KP + 255) / 256, ts.nimg), 256, 0, ctx->st, ctx->mu.as<double>(), ctx->iv.as<double>(),
+                ctx->kc2.as<float>(), ctx->ctr.as<double>(), ctx->M, ws_pad_m(ctx->M), ctx->D, ctx->DP, ts.TN, ts.s0.as<int32_t>(),
+                ts.ns.as<int32_t>(), ts.images.as<float>()));
   LAUNCH_CHECK();
   return HMMCU_OK;
 }
@@ -1807,10 +1827,14 @@ static int set_train_map(hmmcu_ctx *ctx, const int32_t *utt2model) {
   CK(cudaMemcpyAsync(ctx->mus_d.p, start.data(), sizeof(int32_t) * (V + 1), cudaMemcpyHostToDevice, ctx->st));
   CK(cudaMemcpyAsync(ctx->mu_d.p, utts.data(), sizeof(int32_t) * U, cudaMemcpyHostToDevice, ctx->st));
   CK(cudaMemcpyAsync(ctx->tiles_d.p, tiles.data(), sizeof(EmisTile) * tiles.size(), cudaMemcpyHostToDevice, ctx->st));
-  {  // k_fb_res: the live utterances longest first, cut into batches that fit one team's shared memory; the row of
-     // every utterance in the per-utterance statistics (= its position in the model-grouped list)
+  {  // k_fb_res: the live utterances longest first, cut into batches that fit one team's shared memory and hold at most
+     // ceil(live / teams) utterances, so that a small corpus still reaches every team of the grid (a batch's time is its
+     // longest chain plus staging and the gamma phase over all its frames); the row of every utterance in the
+     // per-utterance statistics (= its position in the model-grouped list)
     const int nlive = start[V];
     ctx->n_live = nlive;
+    const int teams = kResTeams * std::max(ctx->sm_count, 1);
+    const int per_batch = std::max(1, std::min(kResMaxUtts, (nlive + teams - 1) / teams));
     std::vector<int32_t> order(utts.begin(), utts.begin() + nlive), upos(std::max(U, 1), 0);
     for (int k = 0; k < nlive; k++) upos[utts[k]] = k;
     std::stable_sort(order.begin(), order.end(), [&](int32_t a, int32_t b) { return ctx->off[a + 1] - ctx->off[a] > ctx->off[b + 1] - ctx->off[b]; });
@@ -1820,7 +1844,7 @@ static int set_train_map(hmmcu_ctx *ctx, const int32_t *utt2model) {
     for (int k = 0; k < nlive && ctx->res_fits;) {
       int64_t used = 0;
       int n = 0;
-      while (k + n < nlive && n < kResMaxUtts) {
+      while (k + n < nlive && n < per_batch) {
         const int64_t w = res_utt_words(ctx->N, ctx->off[order[k + n] + 1] - ctx->off[order[k + n]]);
         if (used + w > cap) break;
         used += w;
@@ -1834,7 +1858,10 @@ static int set_train_map(hmmcu_ctx *ctx, const int32_t *utt2model) {
     CK(ctx->res_order.ensure(sizeof(int32_t) * std::max(nlive, 1)));
     CK(ctx->res_upos.ensure(sizeof(int32_t) * std::max(U, 1)));
     CK(ctx->res_batches.ensure(sizeof(ResBatch) * std::max<size_t>(rb.size(), 1)));
-    CK(ctx->res_counter.ensure(sizeof(int)));
+    if (!ctx->res_counter.p) {  // k_fb_res leaves it at 0 after every launch
+      CK(ctx->res_counter.ensure(sizeof(int)));
+      CK(cudaMemsetAsync(ctx->res_counter.p, 0, sizeof(int), ctx->st));
+    }
     CK(ctx->ustats.ensure(sizeof(double) * (size_t)std::max(nlive, 1) * res_stats_row(std::min(ctx->N, 8))));
     CK(cudaMemcpyAsync(ctx->res_order.p, order.data(), sizeof(int32_t) * nlive, cudaMemcpyHostToDevice, ctx->st));
     CK(cudaMemcpyAsync(ctx->res_upos.p, upos.data(), sizeof(int32_t) * U, cudaMemcpyHostToDevice, ctx->st));
@@ -1923,9 +1950,13 @@ static int estep_core(hmmcu_ctx *ctx, const int32_t *utt2model, int phases, cons
   // ---- the launch sequence: statistics cleared, emissions, forward-backward, accumulators ----
   const float *lb_fb = fb_logb ? fb_logb : ctx->logb.as<float>();
   const float *gm_acc = acc_gamma ? acc_gamma : ctx->gamma.as<float>();
+  const bool res_fb = ctx->use_res_fb && ctx->banded && ctx->res_fits && ctx->n_res_batches > 0;
   auto enqueue = [&]() -> int {
     if (phases & 1) CK(cudaMemsetAsync(ctx->stats.p, 0, sizeof(double) * ctx->stats_n, ctx->st));
     if (U == 0) return HMMCU_OK;
+    // masked utterances report 0 (k_fb_res writes the live ones only); cleared here, so that no memset node sits between the
+    // emission kernel and k_fb_res
+    if ((phases & 2) && res_fb && ctx->n_live < U) CK(cudaMemsetAsync(ctx->logp_utt_d.p, 0, sizeof(double) * U, ctx->st));
     int rc2;
     bool fb_forked = false;
     const bool pack_forked = pack16 && !ctx->timing && (phases & 3) && ctx->mstep_fork;
@@ -1948,18 +1979,16 @@ static int estep_core(hmmcu_ctx *ctx, const int32_t *utt2model, int phases, cons
     if (phases & 2) {
     t_begin(ctx, "fwdbwd");
     {
-        if (ctx->use_res_fb && ctx->banded && ctx->res_fits && ctx->n_res_batches > 0) {
+        if (res_fb) {
         // every utterance resident in shared memory: log-emissions read once, gamma written once (fbres_kernels.cuh)
-        CK(cudaMemsetAsync(ctx->res_counter.p, 0, sizeof(int), ctx->st));
         if (ctx->debug_acc & 8) CK(cudaMemsetAsync(ctx->acc_dbg.p, 0, sizeof(float) * 3 * 16384, ctx->st));
-        if (ctx->n_live < U) CK(cudaMemsetAsync(ctx->logp_utt_d.p, 0, sizeof(double) * U, ctx->st));  // masked utterances report 0
         const int grid = (int)std::min<int64_t>(ctx->n_res_batches, ctx->sm_count);
-        DISPATCH_N(N, (cudaFuncSetAttribute(k_fb_res<NS>, cudaFuncAttributeMaxDynamicSharedMemorySize, kResSmemBytes),
-                       k_fb_res<NS><<<grid, kResThreads, kResSmemBytes, ctx->st>>>(
-                           lb_fb, ctx->off_d.as<int64_t>(), ctx->u2m_d.as<int32_t>(), ctx->A.as<double>(), ctx->res_order.as<int32_t>(),
-                           ctx->res_upos.as<int32_t>(), ctx->res_batches.as<ResBatch>(), (int)ctx->n_res_batches, ctx->res_counter.as<int>(),
-                           ctx->gamma.as<float>(), ctx->ustats.as<double>(), ctx->logp_utt_d.as<double>(),
-                           (ctx->debug_acc & 8) ? (long long *)ctx->acc_dbg.p : nullptr)));
+        DISPATCH_N(N, CK(cudaFuncSetAttribute(k_fb_res<NS>, cudaFuncAttributeMaxDynamicSharedMemorySize, kResSmemBytes));
+                   CK(launch_pdl(k_fb_res<NS>, grid, kResThreads, kResSmemBytes, ctx->st, lb_fb, ctx->off_d.as<int64_t>(),
+                                 ctx->u2m_d.as<int32_t>(), ctx->A.as<double>(), ctx->res_order.as<int32_t>(), ctx->res_upos.as<int32_t>(),
+                                 ctx->res_batches.as<ResBatch>(), (int)ctx->n_res_batches, ctx->res_counter.as<int>(),
+                                 ctx->gamma.as<float>(), ctx->ustats.as<double>(), ctx->logp_utt_d.as<double>(),
+                                 (ctx->debug_acc & 8) ? (long long *)ctx->acc_dbg.p : nullptr)));
         LAUNCH_CHECK();
         // the per-model sums of the transition statistics feed nothing before the M-step: beside the accumulate kernel
         fb_forked = !ctx->timing && (phases & 4) && ctx->mstep_fork;
@@ -2008,15 +2037,15 @@ static int estep_core(hmmcu_ctx *ctx, const int32_t *utt2model, int phases, cons
       const float *dsc = ctx->acc_sc.as<float>() + 5 * DP;
       if (grid > 0) {
         CK(cudaFuncSetAttribute(k_accum_h, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-        k_accum_h<<<grid, kAhThreads, smem, ctx->st>>>(ctx->acc_unitsH.as<TcTile>(), (int)ctx->n_acc_unitsH, ctx->frame_ids_d.as<int32_t>(),
-                                                      ctx->x16.as<unsigned char>(), ctx->acc_images16.as<uint32_t>(), ctx->acc_kc.as<float>(),
-                                                      ctx->logb.as<float>(), gm_acc, N, M, G, D, DP, ctx->stats.as<double>(), ss, off_S0, off_S1,
-                                                      off_S2, ctx->acc_scratch.as<float>(), dsc);
+        CK(launch_pdl(k_accum_h, grid, kAhThreads, smem, ctx->st, ctx->acc_unitsH.as<TcTile>(), (int)ctx->n_acc_unitsH,
+                      ctx->frame_ids_d.as<int32_t>(), ctx->x16.as<unsigned char>(), ctx->acc_images16.as<uint32_t>(), ctx->acc_kc.as<float>(),
+                      ctx->logb.as<float>(), gm_acc, N, M, G, D, DP, ctx->stats.as<double>(), ss, off_S0, off_S1, off_S2,
+                      ctx->acc_scratch.as<float>(), dsc));
         LAUNCH_CHECK();
       }
-      k_finalize_slots<<<dim3(G, V), 64 * kFinParts, 0, ctx->st>>>(ctx->stats.as<double>(), ss, G, D, DP, 2 * DP, (G + 127) / 128, off_S0, off_S1,
-                                                                  off_S2, ctx->ctr.as<double>(), ctx->mu.as<double>(), ctx->acc_scratch.as<float>(),
-                                                                  ctx->acc_slot_start_h.as<int32_t>(), ctx->acc_slot_ids_h.as<int32_t>(), dsc);
+      CK(launch_pdl(k_finalize_slots, dim3(G, V), 64 * kFinParts, 0, ctx->st, ctx->stats.as<double>(), ss, G, D, DP, 2 * DP, (G + 127) / 128,
+                    off_S0, off_S1, off_S2, ctx->ctr.as<double>(), ctx->mu.as<double>(), ctx->acc_scratch.as<float>(),
+                    ctx->acc_slot_start_h.as<int32_t>(), ctx->acc_slot_ids_h.as<int32_t>(), dsc));
       LAUNCH_CHECK();
     } else if (ws_acc) {
       const size_t smem = ws_acc_smem_bytes(2 * DP);
@@ -2167,10 +2196,9 @@ int hmmcu_mstep(hmmcu_ctx *ctx, double threshold, double *sum_logp, double *n_ut
     k_mstep_ctl<<<(V + 127) / 128, 128, 0, ctx->st>>>(ctx->stats.as<double>(), ssz, V, threshold, ctx->em_old.as<double>(),
                                                       ctx->em_active.as<int>(), ctx->ctl_d.as<double>(), ctx->upd_d.as<int>());
     LAUNCH_CHECK();
-    k_mstep_apply<<<dim3(1 + (ctx->G + 7) / 8, V), 256, 0, ctx->st>>>(ctx->stats.as<double>(), ssz, ctx->N, ctx->M, ctx->Dm,
-                                                                       1.0e-5 /* FINITE_PROBAB, T-FS:39 */, ctx->upd_d.as<int>(),
-                                                                       ctx->A.as<double>(), ctx->c.as<double>(), ctx->mu.as<double>(),
-                                                                       ctx->iv.as<double>(), ctx->det.as<double>());
+    CK(launch_pdl(k_mstep_apply, dim3(1 + (ctx->G + 7) / 8, V), 256, 0, ctx->st, ctx->stats.as<double>(), ssz, ctx->N, ctx->M, ctx->Dm,
+                  1.0e-5 /* FINITE_PROBAB, T-FS:39 */, ctx->upd_d.as<int>(), ctx->A.as<double>(), ctx->c.as<double>(),
+                  ctx->mu.as<double>(), ctx->iv.as<double>(), ctx->det.as<double>()));
     LAUNCH_CHECK();
     int rc2;
     // The accuracy-guard scan and the second W packer do not feed the main chain (new parameters -> kc -> emission

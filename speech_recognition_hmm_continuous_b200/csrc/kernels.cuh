@@ -23,6 +23,14 @@ constexpr double kLogTrueMin = -744.4400719213812;
 
 __host__ __device__ inline int round_up(int a, int b) { return (a + b - 1) / b * b; }
 
+// Programmatic dependent launch (launch_pdl in hmmcu.cu).  pdl_wait() returns once the kernels this one depends on
+// have completed and their writes are visible (at once after a plain launch); a kernel launched with launch_pdl calls
+// it in every CTA before it reads anything an earlier kernel of its launch sequence wrote and before its first global
+// write.  pdl_trigger() lets the next kernel of the stream be scheduled once every CTA of this one has called it or
+// exited, so that its launch and prologue overlap this kernel's drain.
+__device__ __forceinline__ void pdl_wait() { asm volatile("griddepcontrol.wait;" ::: "memory"); }
+__device__ __forceinline__ void pdl_trigger() { asm volatile("griddepcontrol.launch_dependents;" ::: "memory"); }
+
 // ------------------------------------------------------------------------------------------------
 // centre: per-dimension mean of up to 4096 evenly strided frames (deterministic, one block).
 // ------------------------------------------------------------------------------------------------
@@ -450,6 +458,7 @@ __global__ void k_rank(const double *__restrict__ logp, int U, int V, double wei
 __global__ void k_mstep_ctl(const double *__restrict__ stats, int64_t ss, int V, double threshold, double *__restrict__ em_old,
                             int *__restrict__ em_active, double *__restrict__ ctl, int *__restrict__ upd) {
   const int v = blockIdx.x * blockDim.x + threadIdx.x;
+  pdl_trigger();
   if (v >= V) return;
   const double *st = stats + (int64_t)v * ss;
   const double probab = st[ss - 2], nutt = st[ss - 1];
@@ -473,6 +482,8 @@ k_mstep_apply(const double *__restrict__ stats, int64_t ss, int N, int M, int D,
               double *__restrict__ Aall, double *__restrict__ call, double *__restrict__ muall, double *__restrict__ ivall,
               double *__restrict__ detall) {
   const int v = blockIdx.y, tid = threadIdx.x, G = N * M;
+  pdl_wait();
+  pdl_trigger();
   if (!upd[v]) return;
   const double *st = stats + (int64_t)v * ss;
   const double *num = st, *den = num + (int64_t)N * N, *denmix = den + N, *S0 = denmix + N;

@@ -441,6 +441,8 @@ __global__ void k_pack_kc(const double *__restrict__ mu, const double *__restric
   // one warp per Gaussian, lanes over the dimensions (coalesced reads of mu / iv, shuffle reduction)
   const int64_t g = ((int64_t)blockIdx.x * blockDim.x + threadIdx.x) >> 5;
   const int lane = threadIdx.x & 31;
+  pdl_wait();
+  pdl_trigger();
   if (g >= VG) return;
   double q = 0.0;
   for (int d = lane; d < D; d += 32) {

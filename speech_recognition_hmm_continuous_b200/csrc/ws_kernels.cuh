@@ -163,6 +163,7 @@ __global__ void k_pack_w_ws(const double *__restrict__ mu, const double *__restr
                             float *__restrict__ images) {
   const int img = blockIdx.y;
   const int KP = 2 * DP;
+  pdl_wait();
   const uint32_t P = (uint32_t)(KP / 4) * 128;
   const size_t img_floats = ws_image_bytes(TN, KP) / 4;
   float *hi = images + (size_t)img * img_floats;
@@ -345,6 +346,7 @@ k_emis_ws(const TcTile *__restrict__ units, int nunits, int ntiles_dec, int nfra
   __syncthreads();
   tc_fence_after();
   const uint32_t tmem0 = (uint32_t)lds_i32(tmem_slot);
+  pdl_trigger();  // this CTA's work is a fixed unit range: nothing is left to claim
   // TMEM columns: AST operand stages of 160 [x_hi | x2_hi | x_lo | x2_lo], then two accumulator stages of ACS.
   // Images wider than 96 columns (one state of up to 176 mixtures) leave room for a single operand stage.
   const int AST = TN > 96 ? 1 : 2;
@@ -1185,7 +1187,8 @@ k_finalize_slots(double *__restrict__ stats, int64_t stats_stride, int G, int D,
   double *st = stats + (int64_t)v * stats_stride;
   __shared__ double sp[kFinParts][3][64];
   const int img = v * nRB + (g >> 7), row = g & 127;
-  const int k0 = slot_start[img], nk = slot_start[img + 1] - k0;
+  const int k0 = slot_start[img], nk = slot_start[img + 1] - k0;  // (slot tables: uploaded with the training map)
+  pdl_wait();
   double s0 = 0.0, s1 = 0.0, s2 = 0.0;
   for (int k = part; k < nk; k += kFinParts) {
     const float *sl = scratch + ((size_t)slot_ids[k0 + k] * 128 + row) * KP2;
