@@ -217,8 +217,16 @@ int hmmcu_viterbi_scores(hmmcu_ctx *ctx, double *score);
 int64_t hmmcu_launch_count(const hmmcu_ctx *ctx);
 /* Device time in ms of the most recent call's kernels, by name (CUDA events on the context's
  * stream).  names: "emis", "fwdbwd", "accum", "mstep", "score", "viterbi", "logb64", "pack", "init".  -1 if unknown.
- * Two pseudo-names report state instead of time: "kappa" (accuracy-guard value) and "tc_active"
- * (1 if the last emission launch ran on tensor cores). */
+ * Pseudo-names report state instead of time:
+ *   "kappa"           accuracy-guard value of the current model pack
+ *   "tc_active"       1 if the last emission launch ran on tensor cores
+ *   "dec_f16_active"  1 if the last decode emission launch used half-precision operands
+ *   "acc_h_active"    1 if the last mixture-accumulate launch was the half-precision kernel
+ *   "dec_grid"        CTAs of the decode emission kernel's launch configuration (0 = not chosen yet, -1 = unusable)
+ *   "res_batches"     batches of the resident forward-backward kernel for the current training map
+ *                     (0 when the windowed kernel takes the E-step)
+ *   "res_batch_max"   the most utterances in one of those batches (0 likewise)
+ *   "res_teams"       teams that claim those batches: 4 per CTA of its launch, min(res_batches, SMs) CTAs (0 likewise) */
 double hmmcu_last_kernel_ms(const hmmcu_ctx *ctx, const char *name);
 void hmmcu_enable_timing(hmmcu_ctx *ctx, int on);
 

@@ -19,7 +19,7 @@
 // the NEXT window of kFbWin frames of every utterance of the CTA into shared memory as b~ (double) while
 // the chains consume the current one (two buffers) -- forward window from the start of the utterance,
 // backward window from its end -- so a chain step is NS LDS.64, the banded matvec, the power-of-two
-// scaling and two 16-byte stores of the scaled vector in single precision (rows of 8 floats).
+// scaling and two 16-byte stores of the scaled vector as the high words of its doubles (rows of 8 words, d32_pack).
 // A second phase (one warp per utterance, lanes over frames) forms gamma, the transition sums and sum m_t.
 #pragma once
 #include "kernels.cuh"
@@ -82,33 +82,30 @@ __device__ __forceinline__ double pow2_scale_max(const double (&v)[NS], int &e) 
   return __hiloint2double(ok ? (2046 - be) << 20 : 0x3ff00000, 0);
 }
 
-template <int NS>
-__device__ __forceinline__ void store_row(float *__restrict__ p, const double (&z)[NS]) {
-  float f[kFbRow];
-#pragma unroll
-  for (int i = 0; i < kFbRow; i++) f[i] = (i < NS) ? (float)z[i] : 0.f;
-  *reinterpret_cast<float4 *>(p) = make_float4(f[0], f[1], f[2], f[3]);
-  if (NS > 4) *reinterpret_cast<float4 *>(p + 4) = make_float4(f[4], f[5], f[6], f[7]);
+// high word of a non-negative double, rounded to nearest: the full double range at 4 bytes per value (a float row
+// would flush a state whose mass is below 2^-126 of the frame's largest, and the other chain can lift it back to
+// order one: alpha^ beta^ of such a state is not small)
+__device__ __forceinline__ uint32_t d32_pack(double v) {
+  return (uint32_t)__double2hiint(v) + ((uint32_t)__double2loint(v) >> 31);
 }
+__device__ __forceinline__ double d32_unpack(uint32_t w) { return __hiloint2double((int)w, 0); }
+
 template <int NS>
-__device__ __forceinline__ void load_row(const float *__restrict__ p, double (&z)[NS]) {
-  const float4 a = *reinterpret_cast<const float4 *>(p);
-  float f[kFbRow] = {a.x, a.y, a.z, a.w, 0.f, 0.f, 0.f, 0.f};
-  if (NS > 4) {
-    const float4 b = *reinterpret_cast<const float4 *>(p + 4);
-    f[4] = b.x; f[5] = b.y; f[6] = b.z; f[7] = b.w;
-  }
+__device__ __forceinline__ void store_row(uint32_t *__restrict__ p, const double (&z)[NS]) {
+  uint32_t f[kFbRow];
 #pragma unroll
-  for (int i = 0; i < NS; i++) z[i] = (double)f[i];
+  for (int i = 0; i < kFbRow; i++) f[i] = (i < NS) ? d32_pack(z[i]) : 0u;
+  *reinterpret_cast<uint4 *>(p) = make_uint4(f[0], f[1], f[2], f[3]);
+  if (NS > 4) *reinterpret_cast<uint4 *>(p + 4) = make_uint4(f[4], f[5], f[6], f[7]);
 }
 
 // Outputs: gamma32[F][N] (the reference's alpha^ beta^ / c, T-FS:1709); per-model statistics head
 // (num_trans, den_trans, den_mix, sum_logp, n_utt) by double atomics, one set per utterance;
-// logp_utt[U] (0 for masked utterances).  alpha_ws / beta_ws: float [F][kFbRow] workspaces.
+// logp_utt[U] (0 for masked utterances).  alpha_ws / beta_ws: [F][kFbRow] workspaces of d32 words.
 template <int NS, bool BANDED>
 __global__ void __launch_bounds__(kFbThreads)
 k_fb(const float *__restrict__ logb, const int64_t *__restrict__ off, const int32_t *__restrict__ u2m,
-     const double *__restrict__ Aall, int U, float *__restrict__ alpha_ws, float *__restrict__ beta_ws,
+     const double *__restrict__ Aall, int U, uint32_t *__restrict__ alpha_ws, uint32_t *__restrict__ beta_ws,
      float *__restrict__ gamma, double *__restrict__ stats, int64_t stats_stride, int64_t off_sumlogp,
      double *__restrict__ logp_utt) {
   extern __shared__ __align__(16) uint8_t fb_smem[];
@@ -195,7 +192,7 @@ k_fb(const float *__restrict__ logb, const int64_t *__restrict__ off, const int3
     } else if (chain && warp == 0) {  // forward: frames w0 .. w0+kFbWin-1
       const double *bw = bcur + (size_t)lane * US;
       const int kend = min(kFbWin, myT - w0);
-      float *ap = alpha_ws + (mybase + w0) * kFbRow;
+      uint32_t *ap = alpha_ws + (mybase + w0) * kFbRow;
       for (int k = 0; k < kend; k++) {
         double b[NS], raw[NS];
 #pragma unroll
@@ -279,29 +276,29 @@ k_fb(const float *__restrict__ logb, const int64_t *__restrict__ off, const int3
 #pragma unroll
     for (int i = 0; i < NS; i++) { acc_num[i][0] = acc_num[i][1] = 0.0; acc_dt[i] = 0.0; acc_dm[i] = 0.0; }
     // the rows of frame t + 32 are fetched while frame t is being worked on (the loop is latency bound otherwise)
-    struct Raw { float4 a0, a1, b0, b1, c0, c1; float l0[NS], l1[NS]; };
+    struct Raw { uint4 a0, a1, b0, b1, c0, c1; float l0[NS], l1[NS]; };
     auto fetch = [&](int t, Raw &r) {
-      const float4 z4 = make_float4(0.f, 0.f, 0.f, 0.f);
+      const uint4 z4 = make_uint4(0u, 0u, 0u, 0u);
       r.a0 = r.a1 = r.b0 = r.b1 = r.c0 = r.c1 = z4;
 #pragma unroll
       for (int i = 0; i < NS; i++) r.l0[i] = r.l1[i] = 0.f;
       if (t < T) {
-        const float4 *pa = reinterpret_cast<const float4 *>(alpha_ws + (base + t) * kFbRow);
-        const float4 *pb = reinterpret_cast<const float4 *>(beta_ws + (base + t) * kFbRow);
+        const uint4 *pa = reinterpret_cast<const uint4 *>(alpha_ws + (base + t) * kFbRow);
+        const uint4 *pb = reinterpret_cast<const uint4 *>(beta_ws + (base + t) * kFbRow);
         r.a0 = pa[0]; r.b0 = pb[0];
         if (NS > 4) { r.a1 = pa[1]; r.b1 = pb[1]; }
         load_lb<NS>(logb + (base + t) * NS, r.l0);
         if (t < T - 1) {
-          r.c0 = pb[2];  // beta row of frame t + 1 (rows are kFbRow = 8 floats)
+          r.c0 = pb[2];  // beta row of frame t + 1 (rows are kFbRow = 8 words)
           if (NS > 4) r.c1 = pb[3];
           load_lb<NS>(logb + (base + t + 1) * NS, r.l1);
         }
       }
     };
-    auto unpack = [](const float4 &x0, const float4 &x1, double (&o)[NS]) {
-      const float f[8] = {x0.x, x0.y, x0.z, x0.w, x1.x, x1.y, x1.z, x1.w};
+    auto unpack = [](const uint4 &x0, const uint4 &x1, double (&o)[NS]) {
+      const uint32_t f[8] = {x0.x, x0.y, x0.z, x0.w, x1.x, x1.y, x1.z, x1.w};
 #pragma unroll
-      for (int i = 0; i < NS; i++) o[i] = (double)f[i];
+      for (int i = 0; i < NS; i++) o[i] = d32_unpack(f[i]);
     };
     Raw cur, nxt;
     fetch(lane, cur);

@@ -83,12 +83,6 @@ __host__ __device__ constexpr int res_row_stride(int NS) { return NS | 1; }
 __host__ __device__ inline int64_t res_utt_words(int NS, int64_t T) { return 2 * (int64_t)res_row_stride(NS) * T; }
 __host__ __device__ inline int res_stats_row(int NS) { return 4 * NS + 1; }  // [num a_ii | num a_i,i+1 | den_trans | den_mix | logP]
 
-// high word of a non-negative double, rounded to nearest
-__device__ __forceinline__ uint32_t d32_pack(double v) {
-  return (uint32_t)__double2hiint(v) + ((uint32_t)__double2loint(v) >> 31);
-}
-__device__ __forceinline__ double d32_unpack(uint32_t w) { return __hiloint2double((int)w, 0); }
-
 // One chain step.  The state y is carried UNSCALED by its own step's factor: the power of two r that normalises y is
 // folded into the b~ of the step that consumes it, so the exponent arithmetic (integer pipe) runs beside the matrix-vector
 // product instead of in front of it:      y' = (A-part of y) o (b~ r),   r = 2^-e,  e = largest exponent field of y.

@@ -190,6 +190,7 @@ struct hmmcu_ctx {
   int peer_fused = 1;                   // hmmcu_peer_allreduce as one launch (k_peer_allreduce1) instead of push + reduce
   int64_t peer_n = 0;                   // doubles per slot the area was sized for
   int64_t n_res_batches = 0;
+  int res_batch_max = 0;  // the most utterances in one of those batches
   int n_live = 0;         // utterances of the training map that belong to a model (the others are masked)
   bool res_fits = false;  // every utterance of the training map fits one team's shared memory
   int debug_acc = 0;
@@ -200,6 +201,11 @@ struct hmmcu_ctx {
   DevBuf logb, logb64, post, gamma, alpha_ws, beta_ws, stats, logp_utt_d, score_d, psi_ws, path_d, tiles_dec, rank_in, rank_out;
   int64_t stats_n = 0;
 };
+
+// k_fb_res takes the forward-backward of the current training map (otherwise k_fb does)
+static bool res_fb_on(const hmmcu_ctx *ctx) { return ctx->use_res_fb && ctx->banded && ctx->res_fits && ctx->n_res_batches > 0; }
+// CTAs of its launch: one per SM at most, none without a batch
+static int res_grid(const hmmcu_ctx *ctx) { return (int)std::min<int64_t>(ctx->n_res_batches, ctx->sm_count); }
 
 static int fail(hmmcu_ctx *c, int code, const char *fmt, ...) {
   va_list ap;
@@ -456,6 +462,10 @@ double hmmcu_last_kernel_ms(const hmmcu_ctx *ctx, const char *name) {
   if (strcmp(name, "dec_f16_active") == 0) return ctx->last_dec16 ? 1.0 : 0.0;
   if (strcmp(name, "acc_h_active") == 0) return ctx->last_acc_h ? 1.0 : 0.0;
   if (strcmp(name, "dec_grid") == 0) return (double)ctx->dec_grid;                // CTAs of the last k_emis_dec launch configuration
+  // the k_fb_res batches of the current training map: how many, the most utterances in one, the teams that claim them
+  if (strcmp(name, "res_batches") == 0) return res_fb_on(ctx) ? (double)ctx->n_res_batches : 0.0;
+  if (strcmp(name, "res_batch_max") == 0) return res_fb_on(ctx) ? (double)ctx->res_batch_max : 0.0;
+  if (strcmp(name, "res_teams") == 0) return res_fb_on(ctx) ? (double)(kResTeams * res_grid(ctx)) : 0.0;
   {  // "<name>_total": the sum over the batches of the last hmmcu_forward_scores / hmmcu_viterbi_scores call
     const size_t ln = strlen(name);
     if (ln > 6 && strcmp(name + ln - 6, "_total") == 0) {
@@ -1841,6 +1851,7 @@ static int set_train_map(hmmcu_ctx *ctx, const int32_t *utt2model) {
     const int64_t cap = res_slot_words_rt(ctx->N);
     std::vector<ResBatch> rb;
     ctx->res_fits = cap > 0;
+    ctx->res_batch_max = 0;
     for (int k = 0; k < nlive && ctx->res_fits;) {
       int64_t used = 0;
       int n = 0;
@@ -1852,6 +1863,7 @@ static int set_train_map(hmmcu_ctx *ctx, const int32_t *utt2model) {
       }
       if (n == 0) { ctx->res_fits = false; break; }  // an utterance longer than a team's shared memory: k_fb takes the E-step
       rb.push_back({k, n});
+      ctx->res_batch_max = std::max(ctx->res_batch_max, n);
       k += n;
     }
     ctx->n_res_batches = ctx->res_fits ? (int64_t)rb.size() : 0;
@@ -1927,9 +1939,9 @@ static int estep_core(hmmcu_ctx *ctx, const int32_t *utt2model, int phases, cons
     CK(ctx->logb.ensure(sizeof(float) * F * N));
     if (!use_tc) CK(ctx->post.ensure(sizeof(float) * F * G));
     CK(ctx->gamma.ensure(sizeof(float) * F * N));
-    if (!(ctx->use_res_fb && ctx->banded && ctx->res_fits && ctx->n_res_batches > 0)) {  // k_fb_res keeps alpha / beta on the SM
-      CK(ctx->alpha_ws.ensure(sizeof(float) * F * kFbRow));
-      CK(ctx->beta_ws.ensure(sizeof(float) * F * kFbRow));
+    if (!res_fb_on(ctx)) {  // k_fb_res keeps alpha / beta on the SM
+      CK(ctx->alpha_ws.ensure(sizeof(uint32_t) * F * kFbRow));
+      CK(ctx->beta_ws.ensure(sizeof(uint32_t) * F * kFbRow));
     }
     CK(ctx->logp_utt_d.ensure(sizeof(double) * U));
     if (ws_emis) {
@@ -1950,7 +1962,7 @@ static int estep_core(hmmcu_ctx *ctx, const int32_t *utt2model, int phases, cons
   // ---- the launch sequence: statistics cleared, emissions, forward-backward, accumulators ----
   const float *lb_fb = fb_logb ? fb_logb : ctx->logb.as<float>();
   const float *gm_acc = acc_gamma ? acc_gamma : ctx->gamma.as<float>();
-  const bool res_fb = ctx->use_res_fb && ctx->banded && ctx->res_fits && ctx->n_res_batches > 0;
+  const bool res_fb = res_fb_on(ctx);
   auto enqueue = [&]() -> int {
     if (phases & 1) CK(cudaMemsetAsync(ctx->stats.p, 0, sizeof(double) * ctx->stats_n, ctx->st));
     if (U == 0) return HMMCU_OK;
@@ -1982,7 +1994,7 @@ static int estep_core(hmmcu_ctx *ctx, const int32_t *utt2model, int phases, cons
         if (res_fb) {
         // every utterance resident in shared memory: log-emissions read once, gamma written once (fbres_kernels.cuh)
         if (ctx->debug_acc & 8) CK(cudaMemsetAsync(ctx->acc_dbg.p, 0, sizeof(float) * 3 * 16384, ctx->st));
-        const int grid = (int)std::min<int64_t>(ctx->n_res_batches, ctx->sm_count);
+        const int grid = res_grid(ctx);
         DISPATCH_N(N, CK(cudaFuncSetAttribute(k_fb_res<NS>, cudaFuncAttributeMaxDynamicSharedMemorySize, kResSmemBytes));
                    CK(launch_pdl(k_fb_res<NS>, grid, kResThreads, kResSmemBytes, ctx->st, lb_fb, ctx->off_d.as<int64_t>(),
                                  ctx->u2m_d.as<int32_t>(), ctx->A.as<double>(), ctx->res_order.as<int32_t>(), ctx->res_upos.as<int32_t>(),
@@ -2006,12 +2018,12 @@ static int estep_core(hmmcu_ctx *ctx, const int32_t *utt2model, int phases, cons
       if (ctx->banded) {
         DISPATCH_N(N, (cudaFuncSetAttribute(k_fb<NS, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)fsm), k_fb<NS, true><<<blocks, kFbThreads, fsm, ctx->st>>>(
                           lb_fb, ctx->off_d.as<int64_t>(), ctx->u2m_d.as<int32_t>(), ctx->A.as<double>(), U,
-                          ctx->alpha_ws.as<float>(), ctx->beta_ws.as<float>(), ctx->gamma.as<float>(), ctx->stats.as<double>(),
+                          ctx->alpha_ws.as<uint32_t>(), ctx->beta_ws.as<uint32_t>(), ctx->gamma.as<float>(), ctx->stats.as<double>(),
                           ss, off_lp, ctx->logp_utt_d.as<double>())));
       } else {
         DISPATCH_N(N, (cudaFuncSetAttribute(k_fb<NS, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)fsm), k_fb<NS, false><<<blocks, kFbThreads, fsm, ctx->st>>>(
                           lb_fb, ctx->off_d.as<int64_t>(), ctx->u2m_d.as<int32_t>(), ctx->A.as<double>(), U,
-                          ctx->alpha_ws.as<float>(), ctx->beta_ws.as<float>(), ctx->gamma.as<float>(), ctx->stats.as<double>(),
+                          ctx->alpha_ws.as<uint32_t>(), ctx->beta_ws.as<uint32_t>(), ctx->gamma.as<float>(), ctx->stats.as<double>(),
                           ss, off_lp, ctx->logp_utt_d.as<double>())));
       }
       LAUNCH_CHECK();

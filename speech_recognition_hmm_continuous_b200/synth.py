@@ -24,12 +24,13 @@ def make_centres(V, N, M, D=39, seed=1234):
     return s * rng.standard_normal((V, N, M, D)), s
 
 
-def make_utterances(centres, s, labels, seed=1234, tmin=250, tmax=350):
-    """-> x float64 [F][D], off int64 [U+1].  labels[u] = word of utterance u."""
+def make_utterances(centres, s, labels, seed=1234, tmin=250, tmax=350, lengths=None):
+    """-> x float64 [F][D], off int64 [U+1].  labels[u] = word of utterance u; its length is lengths[u] when given,
+    otherwise drawn from U{tmin..tmax}."""
     rng = np.random.default_rng(seed + 1)
     V, N, M, D = centres.shape
     U = len(labels)
-    T = rng.integers(tmin, tmax + 1, size=U)
+    T = rng.integers(tmin, tmax + 1, size=U) if lengths is None else np.asarray(lengths, dtype=np.int64)
     off = np.zeros(U + 1, dtype=np.int64)
     np.cumsum(T, out=off[1:])
     F = int(off[-1])

@@ -1137,9 +1137,10 @@ def test_c5_shape_forward_and_viterbi_scores_match_oracle(ctx):
 
 
 def test_large_estep_default_dispatch_matches_oracle(ctx):
-    """A 1,600-utterance E-step through the default dispatch (many batches per team of the resident forward-backward
-    kernel, several CTAs' partial sums per accumulate image): the statistics of three of the 16 words against the
-    oracle's E-step on those words' utterances (T-FS:244-321)."""
+    """A 1,600-utterance E-step through the default dispatch (534 batches of at most 3 utterances for the 592 teams of
+    the resident forward-backward kernel on 148 SMs, several CTAs' partial sums per accumulate image): the statistics of
+    three of the 16 words against the oracle's E-step on those words' utterances (T-FS:244-321).  Full batches and
+    several batches per team: tests/test_fb_res_batches.py."""
     V, N, M, U = 16, 5, 4, 1600
     cen, s = synth.make_centres(V, N, M, 39, seed=6000)
     labels = np.arange(U) % V
