@@ -64,15 +64,13 @@ void hmmcu_host_free(void *p);
  * "upload_chunks": chunks hmmcu_set_features splits the host-to-device copy into (packing overlaps the copy);
  * "mstep_fork": 1 (default) = the accuracy-guard scan and one of the two model packers of hmmcu_mstep run on side streams;
  * "dec_emis": 1 (default) = decode emissions of models with M <= 16 through k_emis_dec (frame tile resident in tensor memory, W
- * images multicast over a cluster, interleaved log-emission layout), 0 = k_emis_ws; "dec_cluster": 2 (default) or 4 CTAs per
- * cluster; "dec_f16": 1 (default) = k_emis_dec with half-precision operands (per-dimension power-of-two scaling, as accurate as
- * the 3xTF32 split; used while the accuracy guard holds and the padded feature row is a multiple of 8), 0 = 3xTF32; "fwd_f64": 1 = the forward cell scorer with a double-precision linear chain instead of the single-precision
- * log-domain one; "dec_budget_kb": log-emission budget of one decode batch in KiB (0 = 6 GiB or a third of the free memory);
+ * images multicast over a cluster of two CTAs, interleaved log-emission layout), 0 = k_emis_ws;
+ * "dec_f16": 1 (default) = k_emis_dec with half-precision operands (per-dimension power-of-two scaling, as accurate as
+ * the 3xTF32 split; used while the accuracy guard holds and the padded feature row is a multiple of 8), 0 = 3xTF32;
+ * "dec_budget_kb": log-emission budget of one decode batch in KiB (0 = 6 GiB or a third of the free memory);
  * "h_acc": 1 (default) = the mixture accumulators through k_accum_h (half-precision hi / lo operands, frame tiles packed once per
  * feature set and fetched by bulk copies; taken while the padded feature row is a multiple of 8 and at most 40), 0 = k_accum_ws
- * (3xTF32, loader warps); "peer_ll": 1 (default) = hmmcu_peer_allreduce with tagged 8-byte words (k_peer_allreduce_ll: no system fence, no
- * flags), 0 = k_peer_allreduce1 (slice-wise push, fence, flags) or, with "peer_fused": 0, hmmcu_peer_push + hmmcu_peer_reduce;
- * "dec_dbg": experiment switches of k_emis_dec (results are garbage: 1 no epilogue arithmetic, 2 no MMAs, 4 no W copies). */
+ * (3xTF32, loader warps).  Any other key fails with HMMCU_EINVAL. */
 int hmmcu_set_option(hmmcu_ctx *ctx, const char *key, int value);
 
 /* ---------------------------------------------------------------- inputs ----------------- */
@@ -162,31 +160,27 @@ double *hmmcu_stats_device(hmmcu_ctx *ctx, int64_t *n_doubles);
 int hmmcu_stats_download(hmmcu_ctx *ctx, double *stats);
 
 /* The sum of the statistics over the ranks of one NVLink / NVSwitch domain WITHOUT a library collective: every rank
- * stores its statistics straight into a receive slot of every peer (peer memory mapped through CUDA IPC), raises a flag
- * there, waits for its own flags and adds the slots in rank order -- one short kernel pair on the context's stream, the
- * same bytes on every rank (the M-step that follows is bit-identical everywhere).  Set-up, once per model-set geometry:
+ * stores its statistics straight into a receive slot of every peer (peer memory mapped through CUDA IPC), waits for the
+ * peers' copies in its own area and adds them in rank order -- one short kernel on the context's stream, the same bytes
+ * on every rank (the M-step that follows is bit-identical everywhere).  Set-up, once per model-set geometry:
  *   hmmcu_peer_export   (after hmmcu_set_models) allocates this rank's receive area and returns its 64-byte IPC handle
  *   [the caller exchanges the handles of all ranks, e.g. with the all-gather of its process group]
  *   hmmcu_peer_import   maps the areas of all ranks (handles[world][64]; the entry of `rank` itself is ignored)
  *   hmmcu_peer_import_pointers   the same for areas that are already addressable in this process (several contexts in
  *                       one process, tests): areas[world] device pointers from hmmcu_peer_area
  * Per EM iteration, between hmmcu_estep and hmmcu_mstep (replaces the all-reduce of hmmh_allreduce_fn):
- *   hmmcu_peer_push     my statistics -> every peer's slot for me, then my flag there
- *   hmmcu_peer_reduce   wait for every peer's flag, statistics = sum over the ranks in rank order
- *   hmmcu_peer_allreduce  the same sum in ONE launch; by default every double travels as two 8-byte words tagged with the
- *                       iteration number (an aligned 8-byte store lands atomically), so the kernel needs neither a system
- *                       fence nor flags: a thread pushes its elements to every peer and adds the peers' copies in rank order
- *                       as they land (options "peer_ll", "peer_fused" select the older forms)
+ *   hmmcu_peer_allreduce  statistics = sum over the ranks in rank order, in ONE launch: every double travels as two 8-byte
+ *                       words tagged with the iteration number (an aligned 8-byte store lands atomically), so the kernel
+ *                       needs neither a system fence nor flags: a thread pushes its elements to every peer and adds the
+ *                       peers' copies in rank order as they land
  * Two slot sets alternate, so a rank that runs ahead never overwrites what a slower rank still reads. */
 #define HMMCU_IPC_HANDLE_BYTES 64
 int hmmcu_peer_export(hmmcu_ctx *ctx, int world, void *handle_out);
 int hmmcu_peer_import(hmmcu_ctx *ctx, int rank, int world, const void *handles);
 void *hmmcu_peer_area(hmmcu_ctx *ctx);
 int hmmcu_peer_import_pointers(hmmcu_ctx *ctx, int rank, int world, void *const *areas);
-int hmmcu_peer_push(hmmcu_ctx *ctx);
-int hmmcu_peer_reduce(hmmcu_ctx *ctx);
 int hmmcu_peer_allreduce(hmmcu_ctx *ctx);
-/* 1 when a hmmcu_peer_reduce gave up waiting for a peer (20 s); synchronises the context's stream */
+/* 1 when a hmmcu_peer_allreduce gave up waiting for a peer (20 s); synchronises the context's stream */
 int hmmcu_peer_error(hmmcu_ctx *ctx);
 
 /* Device-resident EM iteration.  The M-step of the trainer's main() (T-FS:326-352:

@@ -27,8 +27,8 @@ EXPORTS = [
     "hmmcu_features_begin", "hmmcu_features_append", "hmmcu_features_wait", "hmmcu_features_end", "hmmcu_staging", "hmmcu_link_streams", "hmmh_read_model_streams", "hmmh_write_model_streams", "hmmh_train_streams",
     "hmmh_model_set_alloc", "hmmh_model_set_free", "hmmh_read_model_set", "hmmh_write_model_set", "hmmh_upload_model_set",
     "hmmh_read_list", "hmmh_free_list", "hmmh_scan_features", "hmmh_ingest_to", "hmmh_ingest",
-    "hmmcu_peer_export", "hmmcu_peer_import", "hmmcu_peer_area", "hmmcu_peer_import_pointers", "hmmcu_peer_push", "hmmcu_peer_reduce",
-    "hmmcu_peer_allreduce", "hmmcu_peer_error",
+    "hmmcu_peer_export", "hmmcu_peer_import", "hmmcu_peer_area", "hmmcu_peer_import_pointers", "hmmcu_peer_allreduce",
+    "hmmcu_peer_error",
 ]
 
 
@@ -144,7 +144,7 @@ def load():
     lib.hmmcu_peer_area.restype = C.c_void_p
     lib.hmmcu_peer_area.argtypes = [C.c_void_p]
     lib.hmmcu_peer_import_pointers.argtypes = [C.c_void_p, C.c_int, C.c_int, C.POINTER(C.c_void_p)]
-    for f in ("hmmcu_peer_push", "hmmcu_peer_reduce", "hmmcu_peer_allreduce", "hmmcu_peer_error"):
+    for f in ("hmmcu_peer_allreduce", "hmmcu_peer_error"):
         getattr(lib, f).argtypes = [C.c_void_p]
     _lib = lib
     return lib
@@ -411,12 +411,6 @@ class Context:
     def peer_import_pointers(self, rank, world, areas):
         arr = (C.c_void_p * world)(*[C.c_void_p(a) for a in areas])
         self._ck(self.lib.hmmcu_peer_import_pointers(self.h, int(rank), int(world), arr), "hmmcu_peer_import_pointers")
-
-    def peer_push(self):
-        self._ck(self.lib.hmmcu_peer_push(self.h), "hmmcu_peer_push")
-
-    def peer_reduce(self):
-        self._ck(self.lib.hmmcu_peer_reduce(self.h), "hmmcu_peer_reduce")
 
     def peer_allreduce(self):
         self._ck(self.lib.hmmcu_peer_allreduce(self.h), "hmmcu_peer_allreduce")

@@ -277,8 +277,7 @@ k_accum_h(const TcTile *__restrict__ units, int nunits, const int32_t *__restric
         const uint32_t Xh = sm0 + (uint32_t)s * stage_bytes;
         const uint64_t bh = make_smem_desc2(Xh, 128, PX), bl = make_smem_desc2(Xh + x_bytes, 128, PX);
         const uint32_t d = tb + (uint32_t)s * SUB, wh = tb + kAhTmW, wl = wh + DP;
-        if (g_acc_dbg & 2) {
-        } else if (NK1 == 5) {  // D = 39: fully unrolled, addresses are immediates
+        if (NK1 == 5) {  // D = 39: fully unrolled, addresses are immediates
 #pragma unroll
           for (int j = 0; j < 5; j++) tc_mma_f16_ts(d, wh + j * 8, bh + (uint64_t)(j * 16), idesc1, j > 0);  // Wh*Xh
 #pragma unroll
@@ -319,15 +318,13 @@ k_accum_h(const TcTile *__restrict__ units, int nunits, const int32_t *__restric
         const uint32_t Xh = sm0 + (uint32_t)sj * stage_bytes;
         const uint64_t bh = make_smem_desc2(Xh + g2_off, PX, 128), bl = make_smem_desc2(Xh + x_bytes + g2_off, PX, 128);
         const uint32_t w0 = tb + (uint32_t)sj * SUB, d = tb + kAhTmS;
-        if (!(g_acc_dbg & 2)) {
 #pragma unroll
-          for (int k = 0; k < SUB / 16; k++)
-            tc_mma_f16_ts(d, w0 + 32 * (k >> 1) + 8 * (k & 1), bh + kstep * k, idesc2, (cnt > 1 || k > 0) ? 1u : 0u);  // wh*Xh
+        for (int k = 0; k < SUB / 16; k++)
+          tc_mma_f16_ts(d, w0 + 32 * (k >> 1) + 8 * (k & 1), bh + kstep * k, idesc2, (cnt > 1 || k > 0) ? 1u : 0u);  // wh*Xh
 #pragma unroll
-          for (int k = 0; k < SUB / 16; k++) tc_mma_f16_ts(d, w0 + 32 * (k >> 1) + 8 * (k & 1) + 16, bh + kstep * k, idesc2, 1);  // wl*Xh
+        for (int k = 0; k < SUB / 16; k++) tc_mma_f16_ts(d, w0 + 32 * (k >> 1) + 8 * (k & 1) + 16, bh + kstep * k, idesc2, 1);  // wl*Xh
 #pragma unroll
-          for (int k = 0; k < SUB / 16; k++) tc_mma_f16_ts(d, w0 + 32 * (k >> 1) + 8 * (k & 1), bl + kstep * k, idesc2, 1);       // wh*Xl
-        }
+        for (int k = 0; k < SUB / 16; k++) tc_mma_f16_ts(d, w0 + 32 * (k >> 1) + 8 * (k & 1), bl + kstep * k, idesc2, 1);       // wh*Xl
         tc_commit_a(x_free + 8 * sj);
         if (drain) tc_commit_a(s_full);
       }
@@ -368,7 +365,7 @@ k_accum_h(const TcTile *__restrict__ units, int nunits, const int32_t *__restric
         dead = cur_rb * 128 + 32 * q >= G;
       }
       mbar_wait_a(d1_full + 8 * s, (i / NST) & 1);
-      if (!dead && !(g_acc_dbg & 1)) {  // my 32 frames: accumulator columns [32 hb, 32 hb + 32) of stage s
+      if (!dead) {  // my 32 frames: accumulator columns [32 hb, 32 hb + 32) of stage s
         tc_fence_after();
         const uint32_t tl = tmem0 + (uint32_t)s * SUB + trow + 32 * hb;
         uint32_t v0[16], v1[16], wh[16], wl[16];

@@ -7,17 +7,18 @@
 // expansions of the same frames, a quarter of all instructions of a kernel that is bound by instruction issue.  Here the
 // loops are swapped: a CTA expands a frame tile ONCE into tensor memory and keeps it there while ALL W images stream
 // past it.  A W image is 60 KB; one per 1,440 tensor-pipe cycles and SM would be ~12 TB/s of L2 reads, so the CTAs work
-// in CLUSTERS of four: every CTA fetches a quarter of the image with a bulk-tensor-engine copy that is MULTICAST into the
-// shared memory of all four (cp.async.bulk ... .multicast::cluster), each CTA's `full` barrier counting the bytes of all
-// four quarters.  A stage is refilled only when the MMAs of all four CTAs have released it (tcgen05.commit multicast to the
-// `empty` barriers of the cluster).
+// in CLUSTERS of two: every CTA fetches half of the image with a bulk-tensor-engine copy that is MULTICAST into the
+// shared memory of both (cp.async.bulk ... .multicast::cluster), each CTA's `full` barrier counting the bytes of both
+// halves.  A stage is refilled only when the MMAs of both CTAs have released it (tcgen05.commit multicast to the
+// `empty` barriers of the cluster).  Pairs, not clusters of four: pairs fill all 148 SMs of a B200, while 37 clusters of
+// four do not all fit its GPCs at once (DESIGN.md, "Measured and dropped").
 //
 // Warps (18): 0-11 epilogue (TMEM lane quarter w & 3, 16-column groups g with g % 3 == w >> 2: log-sum-exp over the
 // mixtures of every state, additive constants from shared memory, stores log b), 12-15 frame expanders (one frame row per
 // thread, once per round), 16 MMA issuer (also copies the image's constants out of the W stage before it is released),
 // 17 producer (one lane issues the multicast copies).
 // Rounds: round r of CTA b is frame tile r * gridDim + b; every CTA of a cluster runs the same number of rounds and every
-// round runs all images (a CTA without a tile in the last round still fetches and releases its quarters).
+// round runs all images (a CTA without a tile in the last round still fetches and releases its half).
 // TMEM columns: [0, 160) the frame tile [x_hi | x2_hi | x_lo | x2_lo] (DP <= 40), then THREE accumulator stages of 96
 // columns (TN <= 96): the log-sum-exp epilogue of a unit takes longer than its MMAs, and with two stages the tensor pipe
 // waited for it (period = (MMA + epilogue) / 2; measured 54 % pipe activity, the same as k_emis_ws).  W image layout and
@@ -27,7 +28,7 @@
 
 namespace hmmk {
 
-constexpr int kDecClusterMax = 4;  // CTAs per cluster: 4 (a quarter of every image per CTA) or 2, template parameter CL
+constexpr int kDecCluster = 2;     // CTAs per cluster (half of every image per CTA)
 constexpr int kDecEpiWarps = 12;
 constexpr int kDecThreads = (kDecEpiWarps + 6) * 32;  // + 4 expanders, MMA issuer, producer
 constexpr int kDecStages = 3;                         // W images in flight per CTA
@@ -73,12 +74,12 @@ __device__ __forceinline__ void tc_commit_multicast(uint32_t mbar, uint16_t mask
   asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.multicast::cluster.b64 [%0], %1;" ::"r"(mbar), "h"(mask) : "memory");
 }
 
-// MP: padded mixtures per state (1, 2, 3, 4, 5, 8, 16); MR: real mixtures of a state (0 = all MP); CL: CTAs per cluster;
+// MP: padded mixtures per state (1, 2, 3, 4, 5, 8, 16); MR: real mixtures of a state (0 = all MP);
 // H16: half-precision operands (images of k_pack_w_dec16, `scales` of k_dec16_scales)
-template <int MP, int MR, int CL, bool H16>
+template <int MP, int MR, bool H16>
 __global__ void __launch_bounds__(kDecThreads, 1)
 k_emis_dec(int ntiles, int nframes, int nimg, const float *__restrict__ x32, const float *__restrict__ images, int DP, int TN,
-           float *__restrict__ logb, int64_t fbase, int64_t ldb, int S_total, int SCt, int dbg, const float *__restrict__ scales) {
+           float *__restrict__ logb, int64_t fbase, int64_t ldb, int S_total, int SCt, const float *__restrict__ scales) {
   extern __shared__ __align__(1024) uint8_t smem_raw[];
   constexpr int NST = H16 ? kDecStages16 : kDecStages;
   const int KP = 2 * DP;
@@ -96,13 +97,12 @@ k_emis_dec(int ntiles, int nframes, int nimg, const float *__restrict__ x32, con
   }
   const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
   const uint32_t crank = cluster_ctarank();
-  constexpr int kDecCluster = CL;
   constexpr uint16_t kMask = (1u << kDecCluster) - 1;
 
   if (tid == 0) {
     auto init = [](uint32_t addr, uint32_t count) { asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" ::"r"(addr), "r"(count) : "memory"); };
     for (int s = 0; s < NST; s++) {
-      init(full + 8 * s, 1);             // this CTA's producer (arrive.expect_tx); the bytes come from all four CTAs
+      init(full + 8 * s, 1);             // this CTA's producer (arrive.expect_tx); the bytes come from both CTAs
       init(empty + 8 * s, kDecCluster);  // tcgen05.commit of every CTA of the cluster
     }
     for (int a = 0; a < NA; a++) {
@@ -138,8 +138,7 @@ k_emis_dec(int ntiles, int nframes, int nimg, const float *__restrict__ x32, con
       for (int r = 0; r < nrounds; r++) {
         for (int j = 0; j < nimg; j++, n++) {
           const int s = n % NST;
-          mbar_wait_a(empty + 8 * s, ((n / NST) & 1) ^ 1);  // all four CTAs have multiplied what the stage held
-          if ((dbg & 4) && n >= NST) { mbar_arrive_a(full + 8 * s); continue; }  // experiment: no W traffic
+          mbar_wait_a(empty + 8 * s, ((n / NST) & 1) ^ 1);  // both CTAs have multiplied what the stage held
           mbar_expect_tx_a(full + 8 * s, img_bytes);
           bulk_copy_multicast(Ws + (uint32_t)s * img_bytes + crank * qbytes,
                               reinterpret_cast<const char *>(images) + (size_t)j * img_bytes + (size_t)crank * qbytes, qbytes, full + 8 * s, kMask);
@@ -160,7 +159,7 @@ k_emis_dec(int ntiles, int nframes, int nimg, const float *__restrict__ x32, con
       }
       for (int j = 0; j < nimg; j++, n++) {
         const int s = n % NST;
-        mbar_wait_a(full + 8 * s, (n / NST) & 1);  // the image (all four quarters) has landed
+        mbar_wait_a(full + 8 * s, (n / NST) & 1);  // the image (both halves) has landed
         if (have) {
           const int a = nu % NA;
           mbar_wait_a(dempty + 8 * a, ((nu / NA) & 1) ^ 1);  // accumulator stage (and its constants) drained by the epilogue
@@ -175,7 +174,7 @@ k_emis_dec(int ntiles, int nframes, int nimg, const float *__restrict__ x32, con
             const uint64_t wh = make_smem_desc2(wbase, 128, P), wl = make_smem_desc2(wbase + (uint32_t)(TN / 8) * P, 128, P);
             const uint32_t d = tb + acc0 + (uint32_t)a * ACS;
             uint32_t acc = 0;
-            for (int p = 0; p < ((dbg & 2) ? 0 : 3); p++) {  // Xh*Wh, Xl*Wh, Xh*Wl
+            for (int p = 0; p < 3; p++) {  // Xh*Wh, Xl*Wh, Xh*Wl
               const uint32_t a0 = (p == 1) ? xl : xh;
               const uint64_t b0 = (p == 2) ? wl : wh;
 #pragma unroll 10
@@ -185,7 +184,7 @@ k_emis_dec(int ntiles, int nframes, int nimg, const float *__restrict__ x32, con
                 acc = 1;
               }
             }
-            tc_commit_multicast(empty + 8 * s, kMask);  // stage s may be refilled once all four CTAs say so
+            tc_commit_multicast(empty + 8 * s, kMask);  // stage s may be refilled once both CTAs say so
             tc_commit_a(dfull + 8 * a);
             if (j == nimg - 1) tc_commit_a(xempty);  // the frame tile may be replaced
           }
@@ -297,7 +296,7 @@ k_emis_dec(int ntiles, int nframes, int nimg, const float *__restrict__ x32, con
 #pragma unroll
         for (int k = 0; k < kMaxG; k++) {
           const int c = h + EH * k;
-          if (c < ngroups && !(dbg & 1)) {
+          if (c < ngroups) {
             const float4 k0 = kc4[c * 4], k1 = kc4[c * 4 + 1], k2 = kc4[c * 4 + 2], k3 = kc4[c * 4 + 3];
             const float kc[16] = {k0.x, k0.y, k0.z, k0.w, k1.x, k1.y, k1.z, k1.w, k2.x, k2.y, k2.z, k2.w, k3.x, k3.y, k3.z, k3.w};
             float val[16];  // log2(c_g N_g(x)); -inf for a Gaussian of density 0 and for the pad columns

@@ -51,15 +51,6 @@ __device__ __forceinline__ double exp_scaled(float y) {
   return (y < -700.f) ? 0.0 : __hiloint2double(hi, lo);
 }
 
-// r = 2^-e with e the unbiased exponent of s (so that s*r is in [1,2)); e returned.  s == 0, denormal,
-// inf or NaN: r = 1, e = 0.
-__device__ __forceinline__ double pow2_scale(double s, int &e) {
-  const int be = (__double2hiint(s) >> 20) & 0x7ff;
-  if (be == 0 || be == 0x7ff) { e = 0; return 1.0; }
-  e = be - 1023;
-  return __hiloint2double((2046 - be) << 20, 0);
-}
-
 template <int NS>
 __device__ __forceinline__ void load_lb(const float *__restrict__ p, float (&l)[NS]) {
 #pragma unroll

@@ -197,7 +197,7 @@ __global__ void __launch_bounds__(kResThreads, 1)
 k_fb_res(const float *__restrict__ logb, const int64_t *__restrict__ off, const int32_t *__restrict__ u2m,
          const double *__restrict__ Aall, const int32_t *__restrict__ order, const int32_t *__restrict__ upos,
          const ResBatch *__restrict__ batches, int nbatches, int *__restrict__ counter, float *__restrict__ gamma,
-         double *__restrict__ ustats, double *__restrict__ logp_utt, long long *__restrict__ dbg) {
+         double *__restrict__ ustats, double *__restrict__ logp_utt) {
   extern __shared__ __align__(16) uint8_t res_smem[];
   const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
   const int team = warp >> 2, role = warp & 3, tt = role * 32 + lane;  // tt: thread index within the team
@@ -209,22 +209,10 @@ k_fb_res(const float *__restrict__ logb, const int64_t *__restrict__ off, const 
   ResTeamShared<NS> &S = *reinterpret_cast<ResTeamShared<NS> *>(res_smem + (size_t)team * FX);
   uint32_t *slot = reinterpret_cast<uint32_t *>(res_smem + kResTeams * FX) + (size_t)team * SW;
   auto team_sync = [&]() { asm volatile("bar.sync %0, %1;" ::"r"(team + 1), "n"(kResTeamThreads) : "memory"); };
-  // diagnostic time stamps of the phases of this team's first batches: dbg[(block * 4 + team) * 32 + k]
-  int nstamp = 0;
-  auto stamp = [&]() {
-    if (dbg != nullptr && tt == 0 && nstamp < 16) {  // [0..16) globaltimer ns, [16..32) clock64 of the same instants
-      long long t;
-      asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(t));
-      dbg[((size_t)blockIdx.x * kResTeams + team) * 32 + nstamp] = t;
-      dbg[((size_t)blockIdx.x * kResTeams + team) * 32 + 16 + nstamp] = clock64();
-      nstamp++;
-    }
-  };
   for (int i = tt; i < 32 * RS; i += kResTeamThreads) S.dummy[i] = 0x3fe00000u;  // 0.5
   pdl_wait();  // logb comes from the emission kernel just before
   if (tt == 0) S.next = atomicAdd(counter, 1);
   for (;;) {
-    stamp();
     team_sync();
     const int b = S.next;
     if (b >= nbatches) {
@@ -269,7 +257,6 @@ k_fb_res(const float *__restrict__ logb, const int64_t *__restrict__ off, const 
     }
     asm volatile("cp.async.wait_all;" ::: "memory");
     __syncwarp();
-    stamp();
     for (int j = role; j < bd.count; j += 4) {
       const int T = S.T[j];
       uint32_t *F = slot + S.woff[j];
@@ -296,7 +283,6 @@ k_fb_res(const float *__restrict__ logb, const int64_t *__restrict__ off, const 
       if (lane == 0) S.msum[j] = macc;
     }
     team_sync();
-    stamp();
     // ---------------- the chains; meanwhile the idle warps claim the team's next batch and pull it into L2 ----------------
     if (!chain_warp) {
       if (role == ((team + 1) & 3)) {
@@ -317,7 +303,6 @@ k_fb_res(const float *__restrict__ logb, const int64_t *__restrict__ off, const 
       res_chain<NS>(lane, bd.count, S.T, S.woff, S.model, Aall, slot, S.dummy, S.phi, S.lp);
     }
     team_sync();
-    stamp();
     // ---------------- gamma, transition and den sums: one warp per utterance, lanes over frames; gamma replaces alpha~
     // in its row of F and the rows leave as they lie ([frame][state], coalesced) ----------------
     for (int j = role; j < bd.count; j += 4) {

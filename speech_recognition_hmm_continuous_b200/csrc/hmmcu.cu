@@ -159,7 +159,7 @@ struct hmmcu_ctx {
   DevBuf tc_tiles_train, frame_ids_d, tc_tiles_dec, ws_tiles_train;
   int64_t n_tc_tiles_train = 0, n_ws_tiles_train = 0;
   // tensor-core accumulate kernel: W images per (model, block of 128 Gaussians) and its work units
-  DevBuf acc_images, acc_kc, acc_units, acc_dbg, acc_units64, acc_scratch, acc_slot_start, acc_slot_ids;
+  DevBuf acc_images, acc_kc, acc_units, acc_units64, acc_scratch, acc_slot_start, acc_slot_ids;
   int64_t n_acc_units64 = 0;
   int use_ws_acc = 1;  // warp-specialised accumulate kernel (0 = k_accum_tc)
   // k_accum_h (acch_kernels.cuh): half-precision operands, the expanded frame tiles of all units packed once per feature set
@@ -168,32 +168,24 @@ struct hmmcu_ctx {
   int64_t n_acc_unitsH = 0, n_x16_tiles = 0;
   uint64_t x_version = 1, map_version = 1, x16_x = 0, x16_map = 0;  // what x16 was packed from
   int use_dec_emis = 1;  // decode emissions with the frames resident in tensor memory and the W images multicast over a cluster (k_emis_dec)
-  int dec_cluster = 2;   // CTAs per cluster of k_emis_dec (2 or 4)
-  int fwd_f64 = 0;       // forward cell scorer with the chain in double (k_fwd_cells) instead of k_fwd_cells32
   int dec_f16 = 1;       // decode emission kernels with half-precision operands (kind::f16 MMAs at twice the TF32 rate)
   int dec_budget_kb = 0; // log-emission budget of a decode batch in KiB (0 = 6 GiB or a third of the free memory); tests
-  int dec_dbg = 0;       // experiments on k_emis_dec: 1 = no epilogue arithmetic, 2 = no MMAs, 4 = no W copies (results are garbage)
   bool last_acc_h = false;  // the last accumulate launch was k_accum_h
   bool last_dec16 = false;  // the last decode emission launch (k_emis_dec / k_emis_ws<false>) used half-precision operands
   int dec_grid = 0;      // CTAs of k_emis_dec (whole clusters that fit the device at once), 0 = not asked yet
   int use_res_fb = 1;  // shared-memory-resident forward-backward (k_fb_res) whenever the utterances fit and A is banded
   DevBuf res_order, res_upos, res_batches, res_counter, ustats;
-  // peer all-reduce over NVLink (hmmcu_peer_*): my receive area [2 slot sets][world][stats_n] doubles, then
-  // [2][world] 64-bit flags; the areas of all ranks as mapped here; the iteration counter lives on the device
+  // peer all-reduce over NVLink (hmmcu_peer_*): my receive area of tagged words [2 slot sets][world][stats_n] x 16 B;
+  // the areas of all ranks as mapped here; the iteration counter lives on the device
   DevBuf peer_area, peer_ptrs_d, peer_seq_d;
   std::vector<void *> peer_ptrs;        // [world], entry `rank` = my own area
   std::vector<void *> peer_opened;      // IPC mappings to close
   int peer_rank = -1, peer_world = 0;
-  int peer_ll = 1;                      // hmmcu_peer_allreduce with tagged 8-byte words (k_peer_allreduce_ll): no fence, no flags
-  int peer_dbg = 0;                     // k_peer_allreduce1 writes phase stamps (experiments)
-  DevBuf peer_stamps;
-  int peer_fused = 1;                   // hmmcu_peer_allreduce as one launch (k_peer_allreduce1) instead of push + reduce
   int64_t peer_n = 0;                   // doubles per slot the area was sized for
   int64_t n_res_batches = 0;
   int res_batch_max = 0;  // the most utterances in one of those batches
   int n_live = 0;         // utterances of the training map that belong to a model (the others are masked)
   bool res_fits = false;  // every utterance of the training map fits one team's shared memory
-  int debug_acc = 0;
   bool acc_dirty = true;
   int64_t n_acc_units = 0;
 
@@ -405,14 +397,14 @@ void hmmcu_destroy(hmmcu_ctx *ctx) {
   cudaStreamSynchronize(ctx->st);
   unlink_streams(ctx);
   for (void *p : ctx->peer_opened) cudaIpcCloseMemHandle(p);
-  ctx->peer_area.release(); ctx->peer_ptrs_d.release(); ctx->peer_seq_d.release(); ctx->peer_stamps.release();
+  ctx->peer_area.release(); ctx->peer_ptrs_d.release(); ctx->peer_seq_d.release();
   ctx->logb_joint.release();
   DevBuf *bufs[] = {&ctx->x64_own, &ctx->x32, &ctx->ctr, &ctx->off_d, &ctx->A, &ctx->c, &ctx->mu, &ctx->iv, &ctx->det,
                     &ctx->mu32, &ctx->iv32, &ctx->k32, &ctx->kc2, &ctx->u2m_d, &ctx->mus_d, &ctx->mu_d, &ctx->tiles_d, &ctx->logb,
                     &ctx->post, &ctx->gamma, &ctx->alpha_ws, &ctx->stats, &ctx->logp_utt_d, &ctx->score_d,
                     &ctx->psi_ws, &ctx->path_d, &ctx->tiles_dec, &ctx->rank_in, &ctx->rank_out, &ctx->tc_train.images, &ctx->tc_train.kc, &ctx->tc_train.s0,
                     &ctx->tc_train.ns, &ctx->xabs_d, &ctx->tc_dec.images, &ctx->tc_dec.kc, &ctx->tc_dec.s0, &ctx->tc_dec.ns, &ctx->tc_tiles_train,
-                    &ctx->frame_ids_d, &ctx->tc_tiles_dec, &ctx->acc_images, &ctx->acc_kc, &ctx->acc_units, &ctx->beta_ws, &ctx->acc_dbg, &ctx->em_old, &ctx->em_active, &ctx->ctl_d, &ctx->ext_d, &ctx->upd_d, &ctx->ws_train.images, &ctx->ws_train.s0, &ctx->ws_train.ns,
+                    &ctx->frame_ids_d, &ctx->tc_tiles_dec, &ctx->acc_images, &ctx->acc_kc, &ctx->acc_units, &ctx->beta_ws, &ctx->em_old, &ctx->em_active, &ctx->ctl_d, &ctx->ext_d, &ctx->upd_d, &ctx->ws_train.images, &ctx->ws_train.s0, &ctx->ws_train.ns,
                     &ctx->ws_dec.images, &ctx->ws_dec.images16, &ctx->ws_dec.scales16, &ctx->ws_dec.s0, &ctx->ws_dec.ns, &ctx->ws_tiles_train, &ctx->acc_units64, &ctx->logb64, &ctx->acc_scratch, &ctx->acc_slot_start, &ctx->acc_slot_ids, &ctx->in_lst, &ctx->in_off, &ctx->in_vk, &ctx->in_cent,
                     &ctx->in_sum, &ctx->in_dist, &ctx->in_cnt, &ctx->in_idx, &ctx->in_dd, &ctx->in_ord, &ctx->vit_map, &ctx->vit_tiles,
                     &ctx->res_order, &ctx->res_upos, &ctx->res_batches, &ctx->res_counter, &ctx->ustats,
@@ -511,33 +503,13 @@ int hmmcu_set_option(hmmcu_ctx *ctx, const char *key, int value) {
   if (strcmp(key, "mstep_fork") == 0) { ctx->mstep_fork = value != 0; return HMMCU_OK; }
   if (strcmp(key, "upload_chunks") == 0) { ctx->up_chunks = std::max(1, std::min(value, hmmcu_ctx::kUpChunks)); return HMMCU_OK; }
   if (strcmp(key, "tc_emis") == 0) { ctx->use_tc = value; return HMMCU_OK; }
-  if (strcmp(key, "debug_acc") == 0) { ctx->debug_acc = value; return HMMCU_OK; }
   if (strcmp(key, "ws_emis") == 0) { ctx->use_ws = value; return HMMCU_OK; }
   if (strcmp(key, "ws_acc") == 0) { ctx->use_ws_acc = value; ctx->acc_dirty = true; return HMMCU_OK; }
-  if (strcmp(key, "peer_fused") == 0) { ctx->peer_fused = value; return HMMCU_OK; }
-  if (strcmp(key, "peer_ll") == 0) { ctx->peer_ll = value; return HMMCU_OK; }
-  if (strcmp(key, "peer_dbg") == 0) {
-    ctx->peer_dbg = value;
-    if (value) {
-      CK(cudaSetDevice(ctx->dev));
-      CK(ctx->peer_stamps.ensure(sizeof(long long) * 128 * 8));
-      CK(cudaMemsetAsync(ctx->peer_stamps.p, 0, sizeof(long long) * 128 * 8, ctx->st));
-    }
-    return HMMCU_OK;
-  }
   if (strcmp(key, "h_acc") == 0) { ctx->use_h_acc = value; ctx->acc_dirty = true; return HMMCU_OK; }
   if (strcmp(key, "res_fb") == 0) { ctx->use_res_fb = value; return HMMCU_OK; }
-  if (strcmp(key, "fwd_f64") == 0) { ctx->fwd_f64 = value; return HMMCU_OK; }
   if (strcmp(key, "dec_f16") == 0) { ctx->dec_f16 = value; ctx->ws_dec.dirty = true; return HMMCU_OK; }
   if (strcmp(key, "dec_budget_kb") == 0) { ctx->dec_budget_kb = value; return HMMCU_OK; }
-  if (strcmp(key, "acc_dbg") == 0) {
-    CK(cudaSetDevice(ctx->dev));
-    CK(cudaMemcpyToSymbol(g_acc_dbg, &value, sizeof(int)));
-    return HMMCU_OK;
-  }
-  if (strcmp(key, "dec_dbg") == 0) { ctx->dec_dbg = value; return HMMCU_OK; }
   if (strcmp(key, "dec_emis") == 0) { ctx->use_dec_emis = value; return HMMCU_OK; }
-  if (strcmp(key, "dec_cluster") == 0) { ctx->dec_cluster = value == 4 ? 4 : 2; ctx->dec_grid = 0; return HMMCU_OK; }
   return fail(ctx, HMMCU_EINVAL, "unknown option %s", key);
 }
 int64_t hmmcu_stats_size(int N, int M, int D) {
@@ -1249,27 +1221,21 @@ static int launch_emis_ws(hmmcu_ctx *ctx, const TcTile *units_dev, int64_t nunit
   const size_t smem = ws_emis_smem_bytes(ts.TN, 2 * ctx->DP);
   const int grid = (int)std::min<int64_t>(nunits, ctx->sm_count);
   const int MPd = ws_pad_m(ctx->M);
-  if (ctx->debug_acc & 2) {
-    CK(ctx->acc_dbg.ensure(sizeof(float) * 3 * 16384));
-    CK(cudaMemsetAsync(ctx->acc_dbg.p, 0, sizeof(float) * 3 * 16384, ctx->st));
-  }
-  const bool h16 = (TRAIN ? train16_wanted(ctx) : dec16_wanted(ctx)) && ts.images16.p != nullptr && !(ctx->debug_acc & 2);
+  const bool h16 = (TRAIN ? train16_wanted(ctx) : dec16_wanted(ctx)) && ts.images16.p != nullptr;
   if (!TRAIN) ctx->last_dec16 = h16;
-#define WS_LAUNCH4(MPT, DBGT, MRT, HT)                                                                                             \
-  do {                                                                                                                             \
-    CK(cudaFuncSetAttribute(k_emis_ws<TRAIN, MPT, DBGT, MRT, HT>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));        \
-    k_emis_ws<TRAIN, MPT, DBGT, MRT, HT><<<grid, kWsThreads, smem, ctx->st>>>(units_dev, (int)nunits, ntiles_dec, nframes_dec,     \
-                                                                     ctx->frame_ids_d.as<int32_t>(), ctx->x32.as<float>(),         \
-                                                                     HT ? ts.images16.as<float>() : ts.images.as<float>(), ctx->N, \
-                                                                     MPd, ctx->DP, ts.TN, logb, fbase, ldb, ctx->V * ctx->N,       \
-                                                                     ts.SCt, DBGT ? (long long *)ctx->acc_dbg.p : nullptr,         \
-                                                                     ts.scales16.as<float>());                                     \
+#define WS_LAUNCH4(MPT, MRT, HT)                                                                                             \
+  do {                                                                                                                       \
+    CK(cudaFuncSetAttribute(k_emis_ws<TRAIN, MPT, MRT, HT>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));        \
+    k_emis_ws<TRAIN, MPT, MRT, HT><<<grid, kWsThreads, smem, ctx->st>>>(units_dev, (int)nunits, ntiles_dec, nframes_dec,     \
+                                                               ctx->frame_ids_d.as<int32_t>(), ctx->x32.as<float>(),         \
+                                                               HT ? ts.images16.as<float>() : ts.images.as<float>(), ctx->N, \
+                                                               MPd, ctx->DP, ts.TN, logb, fbase, ldb, ctx->V * ctx->N,       \
+                                                               ts.SCt, ts.scales16.as<float>());                             \
   } while (0)
-#define WS_LAUNCH(MPT)                                         \
-  do {                                                         \
-    if (ctx->debug_acc & 2) WS_LAUNCH4(MPT, true, 0, false);   \
-    else if (h16) WS_LAUNCH4(MPT, false, 0, true);             \
-    else WS_LAUNCH4(MPT, false, 0, false);                     \
+#define WS_LAUNCH(MPT)                              \
+  do {                                              \
+    if (h16) WS_LAUNCH4(MPT, 0, true);              \
+    else WS_LAUNCH4(MPT, 0, false);                 \
   } while (0)
   switch (MPd) {
     case 1: WS_LAUNCH(1); break;
@@ -1303,13 +1269,12 @@ static int launch_emis_tc(hmmcu_ctx *ctx, const TcTile *tiles_dev, int ntiles, f
 }
 
 
-// decode emissions, frames resident in tensor memory, W images multicast over clusters of four CTAs (dec_kernels.cuh)
-template <int MP, int MR, int CL, bool H16>
+// decode emissions, frames resident in tensor memory, W images multicast over clusters of two CTAs (dec_kernels.cuh)
+template <int MP, int MR, bool H16>
 static int launch_emis_dec_c(hmmcu_ctx *ctx, int ntiles, int nframes, float *logb, int64_t fbase, int64_t ldb) {
-  constexpr int kDecCluster = CL;
   hmmcu_ctx::TcSet &ts = ctx->ws_dec;
   const size_t smem = dec_emis_smem_bytes(ts.TN, 2 * ctx->DP, H16);
-  auto kern = k_emis_dec<MP, MR, CL, H16>;
+  auto kern = k_emis_dec<MP, MR, H16>;
   CK(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
   cudaLaunchConfig_t cfg = {};
   cudaLaunchAttribute attr[1];
@@ -1322,7 +1287,7 @@ static int launch_emis_dec_c(hmmcu_ctx *ctx, int ntiles, int nframes, float *log
   cfg.stream = ctx->st;
   cfg.attrs = attr;
   cfg.numAttrs = 1;
-  if (ctx->dec_grid == 0) {  // whole clusters that are resident together: one CTA per SM, four SMs of one GPC per cluster
+  if (ctx->dec_grid == 0) {  // whole clusters that are resident together: one CTA per SM, two SMs of one GPC per cluster
     cfg.gridDim = dim3((ctx->sm_count / kDecCluster) * kDecCluster);
     int ncl = 0;
     if (cudaOccupancyMaxActiveClusters(&ncl, kern, &cfg) != cudaSuccess || ncl < 1) {
@@ -1337,8 +1302,7 @@ static int launch_emis_dec_c(hmmcu_ctx *ctx, int ntiles, int nframes, float *log
   cfg.gridDim = dim3(std::min(ctx->dec_grid, want));
   const float *x32 = ctx->x32.as<float>(), *img = H16 ? ts.images16.as<float>() : ts.images.as<float>(), *scales = ts.scales16.as<float>();
   int nimg = ts.nimg, DP = ctx->DP, TN = ts.TN, S_total = ctx->V * ctx->N, SCt = ts.SCt;
-  int dbg = ctx->dec_dbg;
-  CK(cudaLaunchKernelEx(&cfg, kern, ntiles, nframes, nimg, x32, img, DP, TN, logb, fbase, ldb, S_total, SCt, dbg, scales));
+  CK(cudaLaunchKernelEx(&cfg, kern, ntiles, nframes, nimg, x32, img, DP, TN, logb, fbase, ldb, S_total, SCt, scales));
   ctx->last_dec16 = H16;
   ctx->launches++;
   ctx->last_tc = true;
@@ -1347,10 +1311,8 @@ static int launch_emis_dec_c(hmmcu_ctx *ctx, int ntiles, int nframes, float *log
 template <int MP, int MR>
 static int launch_emis_dec_t(hmmcu_ctx *ctx, int ntiles, int nframes, float *logb, int64_t fbase, int64_t ldb) {
   if (dec16_wanted(ctx) && ws_pad_m(ctx->M) <= 16 && ctx->ws_dec.images16.p)
-    return ctx->dec_cluster == 2 ? launch_emis_dec_c<MP, MR, 2, true>(ctx, ntiles, nframes, logb, fbase, ldb)
-                                 : launch_emis_dec_c<MP, MR, 4, true>(ctx, ntiles, nframes, logb, fbase, ldb);
-  return ctx->dec_cluster == 2 ? launch_emis_dec_c<MP, MR, 2, false>(ctx, ntiles, nframes, logb, fbase, ldb)
-                               : launch_emis_dec_c<MP, MR, 4, false>(ctx, ntiles, nframes, logb, fbase, ldb);
+    return launch_emis_dec_c<MP, MR, true>(ctx, ntiles, nframes, logb, fbase, ldb);
+  return launch_emis_dec_c<MP, MR, false>(ctx, ntiles, nframes, logb, fbase, ldb);
 }
 static int launch_emis_dec(hmmcu_ctx *ctx, int ntiles, int nframes, float *logb, int64_t fbase, int64_t ldb) {
   switch (ws_pad_m(ctx->M)) {
@@ -1365,7 +1327,7 @@ static int launch_emis_dec(hmmcu_ctx *ctx, int ntiles, int nframes, float *logb,
   }
 }
 static bool dec_supported(const hmmcu_ctx *ctx) {
-  return ctx->use_dec_emis && ws_pad_m(ctx->M) <= 16 && ctx->DP <= 40 && ctx->dec_grid >= 0 && ctx->sm_count >= kDecClusterMax;
+  return ctx->use_dec_emis && ws_pad_m(ctx->M) <= 16 && ctx->DP <= 40 && ctx->dec_grid >= 0 && ctx->sm_count >= kDecCluster;
 }
 
 // --------------------------------------------------------------------------------- emissions ----
@@ -1451,19 +1413,11 @@ template <int NS> struct ScoreLaunch {
       return;
     }
     const unsigned grid = (unsigned)(((int64_t)nu * ctx->V + kCellThreads - 1) / kCellThreads);
-    if (!ctx->fwd_f64) {  // default: the single-precision log-domain chain (sum of the frame maxima in double)
+    // the single-precision log-domain chain (sum of the frame maxima in double)
 #define FWD32(B, L) k_fwd_cells32<NS, B, L><<<grid, kCellThreads, 0, ctx->st>>>(logb, fbase, ldb, ctx->off_d.as<int64_t>(), u0, nu, ctx->V, ctx->A.as<double>(), out)
-      if (ctx->banded) { if (lay8) FWD32(true, true); else FWD32(true, false); }
-      else { if (lay8) FWD32(false, true); else FWD32(false, false); }
+    if (ctx->banded) { if (lay8) FWD32(true, true); else FWD32(true, false); }
+    else { if (lay8) FWD32(false, true); else FWD32(false, false); }
 #undef FWD32
-      return;
-    }
-    if (ctx->banded)
-      k_fwd_cells<NS, true><<<grid, kCellThreads, 0, ctx->st>>>(logb, fbase, ldb, ctx->off_d.as<int64_t>(), u0, nu, ctx->V,
-                                                                ctx->A.as<double>(), out);
-    else
-      k_fwd_cells<NS, false><<<grid, kCellThreads, 0, ctx->st>>>(logb, fbase, ldb, ctx->off_d.as<int64_t>(), u0, nu, ctx->V,
-                                                                 ctx->A.as<double>(), out);
   }
   static void vit(hmmcu_ctx *ctx, const float *logb, int64_t fbase, int64_t ldb, int u0, int nu, double *out, bool lay8) {
     const unsigned grid = (unsigned)(((int64_t)nu * ctx->V + kCellThreads - 1) / kCellThreads);
@@ -1610,7 +1564,7 @@ static int score_all(hmmcu_ctx *ctx, double *out_host, int mode, int emulate) {
     // the interleaved layout of k_emis_dec is read by k_fwd_cells32, k_vit_cells8 and k_fwd_score; with several feature
     // streams every stream has to write it (their log-emissions are added element by element)
     auto can8 = [](const hmmcu_ctx *c) { return tc_supported(c) && ws_supported(c) && dec_supported(c); };
-    bool all8 = !(mode == 0 && !emulate && ctx->fwd_f64) && can8(ctx);
+    bool all8 = can8(ctx);
     for (hmmcu_ctx *q : ctx->linked) all8 = all8 && can8(q);
     bool lay8 = all8;
     if ((rc = decode_emissions(ctx, fb0, fb1, &lay8)) != HMMCU_OK) return rc;
@@ -1955,7 +1909,6 @@ static int estep_core(hmmcu_ctx *ctx, const int32_t *utt2model, int phases, cons
     } else {
       if ((rc = ensure_simt_pack(ctx)) != HMMCU_OK) return rc;
     }
-    if (ctx->debug_acc & 13) CK(ctx->acc_dbg.ensure(sizeof(float) * 3 * 16384));
   }
   ctx->train_path = ws_emis ? 2 : use_tc ? 1 : 0;
   t_single(ctx, "emis");
@@ -1993,14 +1946,12 @@ static int estep_core(hmmcu_ctx *ctx, const int32_t *utt2model, int phases, cons
     {
         if (res_fb) {
         // every utterance resident in shared memory: log-emissions read once, gamma written once (fbres_kernels.cuh)
-        if (ctx->debug_acc & 8) CK(cudaMemsetAsync(ctx->acc_dbg.p, 0, sizeof(float) * 3 * 16384, ctx->st));
         const int grid = res_grid(ctx);
         DISPATCH_N(N, CK(cudaFuncSetAttribute(k_fb_res<NS>, cudaFuncAttributeMaxDynamicSharedMemorySize, kResSmemBytes));
                    CK(launch_pdl(k_fb_res<NS>, grid, kResThreads, kResSmemBytes, ctx->st, lb_fb, ctx->off_d.as<int64_t>(),
                                  ctx->u2m_d.as<int32_t>(), ctx->A.as<double>(), ctx->res_order.as<int32_t>(), ctx->res_upos.as<int32_t>(),
                                  ctx->res_batches.as<ResBatch>(), (int)ctx->n_res_batches, ctx->res_counter.as<int>(),
-                                 ctx->gamma.as<float>(), ctx->ustats.as<double>(), ctx->logp_utt_d.as<double>(),
-                                 (ctx->debug_acc & 8) ? (long long *)ctx->acc_dbg.p : nullptr)));
+                                 ctx->gamma.as<float>(), ctx->ustats.as<double>(), ctx->logp_utt_d.as<double>())));
         LAUNCH_CHECK();
         // the per-model sums of the transition statistics feed nothing before the M-step: beside the accumulate kernel
         fb_forked = !ctx->timing && (phases & 4) && ctx->mstep_fork;
@@ -2061,24 +2012,13 @@ static int estep_core(hmmcu_ctx *ctx, const int32_t *utt2model, int phases, cons
       LAUNCH_CHECK();
     } else if (ws_acc) {
       const size_t smem = ws_acc_smem_bytes(2 * DP);
-      if (ctx->debug_acc & 4) CK(cudaMemsetAsync(ctx->acc_dbg.p, 0, sizeof(float) * 3 * 16384, ctx->st));
       const int grid = (int)std::min<int64_t>(ctx->n_acc_units64, ctx->sm_count);
       if (grid > 0) {
-        if (ctx->debug_acc & 4) {
-          CK(cudaFuncSetAttribute(k_accum_ws<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-          k_accum_ws<true><<<grid, kAccWsThreads, smem, ctx->st>>>(ctx->acc_units64.as<TcTile>(), (int)ctx->n_acc_units64, ctx->frame_ids_d.as<int32_t>(),
-                                                                 ctx->x32.as<float>(), ctx->acc_images.as<float>(), ctx->acc_kc.as<float>(),
-                                                                 ctx->logb.as<float>(), gm_acc, N, M, G, D, DP,
-                                                                 ctx->stats.as<double>(), ss, off_S0, off_S1, off_S2, ctx->acc_scratch.as<float>(),
-                                                                 (long long *)ctx->acc_dbg.p);
-        } else {
-          CK(cudaFuncSetAttribute(k_accum_ws<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-          k_accum_ws<false><<<grid, kAccWsThreads, smem, ctx->st>>>(ctx->acc_units64.as<TcTile>(), (int)ctx->n_acc_units64, ctx->frame_ids_d.as<int32_t>(),
-                                                                  ctx->x32.as<float>(), ctx->acc_images.as<float>(), ctx->acc_kc.as<float>(),
-                                                                  ctx->logb.as<float>(), gm_acc, N, M, G, D, DP,
-                                                                  ctx->stats.as<double>(), ss, off_S0, off_S1, off_S2, ctx->acc_scratch.as<float>(),
-                                                                  nullptr);
-        }
+        CK(cudaFuncSetAttribute(k_accum_ws, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+        k_accum_ws<<<grid, kAccWsThreads, smem, ctx->st>>>(ctx->acc_units64.as<TcTile>(), (int)ctx->n_acc_units64, ctx->frame_ids_d.as<int32_t>(),
+                                                           ctx->x32.as<float>(), ctx->acc_images.as<float>(), ctx->acc_kc.as<float>(),
+                                                           ctx->logb.as<float>(), gm_acc, N, M, G, D, DP,
+                                                           ctx->stats.as<double>(), ss, off_S0, off_S1, off_S2, ctx->acc_scratch.as<float>());
         LAUNCH_CHECK();
       }
       k_finalize_slots<<<dim3(G, V), 64 * kFinParts, 0, ctx->st>>>(ctx->stats.as<double>(), ss, G, D, DP, tc_kp2(2 * DP), (G + 127) / 128, off_S0,
@@ -2090,13 +2030,11 @@ static int estep_core(hmmcu_ctx *ctx, const int32_t *utt2model, int phases, cons
       const size_t smem = tc_acc_smem_bytes(2 * DP);
       CK(cudaFuncSetAttribute(k_accum_tc, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
       const int grid = (int)std::min<int64_t>(ctx->n_acc_units, ctx->sm_count);
-      if (ctx->debug_acc & 1) CK(cudaMemsetAsync(ctx->acc_dbg.p, 0, sizeof(float) * 3 * 16384, ctx->st));
       if (grid > 0) {
         k_accum_tc<<<grid, kTcThreads, smem, ctx->st>>>(ctx->acc_units.as<TcTile>(), (int)ctx->n_acc_units, ctx->frame_ids_d.as<int32_t>(),
                                                         ctx->x32.as<float>(), ctx->acc_images.as<float>(), ctx->acc_kc.as<float>(),
                                                         ctx->logb.as<float>(), gm_acc, N, M, G, D, DP,
-                                                        ctx->stats.as<double>(), ss, off_S0, off_S1, off_S2,
-                                                        (ctx->debug_acc & 1) ? ctx->acc_dbg.as<float>() : nullptr);
+                                                        ctx->stats.as<double>(), ss, off_S0, off_S1, off_S2);
         LAUNCH_CHECK();
       }
       const int64_t total = (int64_t)V * G * D;
@@ -2124,7 +2062,7 @@ static int estep_core(hmmcu_ctx *ctx, const int32_t *utt2model, int phases, cons
     if (fb_forked) CK(cudaStreamWaitEvent(ctx->st, ctx->ev_join[0], 0));
     return HMMCU_OK;
   };
-  const uint64_t key = 1u | ((ctx->use_res_fb && ctx->banded && ctx->res_fits) ? (1u << 8) : 0u) | (use_tc ? 2u : 0u) | (ws_emis ? 4u : 0u) | (ws_acc ? 8u : 0u) | (h_acc ? 32u : 0u) | (pack16 ? 64u : 0u) | (ctx->banded ? 16u : 0u) | ((uint64_t)(ctx->debug_acc & 15) << 9);
+  const uint64_t key = 1u | ((ctx->use_res_fb && ctx->banded && ctx->res_fits) ? (1u << 8) : 0u) | (use_tc ? 2u : 0u) | (ws_emis ? 4u : 0u) | (ws_acc ? 8u : 0u) | (h_acc ? 32u : 0u) | (pack16 ? 64u : 0u) | (ctx->banded ? 16u : 0u);
   ctx->last_tc = use_tc;
   if (phases & 4) ctx->last_acc_h = h_acc;
   // (pieces of a multi-stream E-step: plain launches)
@@ -2292,15 +2230,6 @@ double *hmmcu_stats_device(hmmcu_ctx *ctx, int64_t *n_doubles) {
   return ctx->stats.as<double>();
 }
 
-// diagnostic: first unit's GEMM1 output (log2 c N), weights and GEMM2 output of the accumulate kernel
-extern "C" int hmmcu_debug_acc_read(hmmcu_ctx *ctx, float *out) {
-  if (!ctx || !out || !ctx->acc_dbg.p) return HMMCU_EINVAL;
-  CK(cudaSetDevice(ctx->dev));
-  CK(cudaMemcpyAsync(out, ctx->acc_dbg.p, sizeof(float) * 3 * 16384, cudaMemcpyDeviceToHost, ctx->st));
-  CK(cudaStreamSynchronize(ctx->st));
-  return HMMCU_OK;
-}
-
 int hmmcu_stats_download(hmmcu_ctx *ctx, double *stats) {
   if (!ctx || !stats) return HMMCU_EINVAL;
   CK(cudaSetDevice(ctx->dev));
@@ -2311,159 +2240,15 @@ int hmmcu_stats_download(hmmcu_ctx *ctx, double *stats) {
 
 
 // ------------------------------------------------------- peer all-reduce over NVLink (no library) ----
-// Area of a rank: slots double[2][world][n] | flags u64[2][world].  Iteration `seq` (1, 2, ..) uses slot set seq & 1;
-// flags only ever grow (the latest iteration whose data of that parity has landed), so nothing is reset.
-__device__ __forceinline__ unsigned long long ld_acquire_sys(const unsigned long long *p) {
-  unsigned long long v;
-  asm volatile("ld.acquire.sys.global.u64 %0, [%1];" : "=l"(v) : "l"(p) : "memory");
-  return v;
-}
-__device__ __forceinline__ void st_release_sys(unsigned long long *p, unsigned long long v) {
-  asm volatile("st.release.sys.global.u64 [%0], %1;" ::"l"(p), "l"(v) : "memory");
-}
-
-// grid (blocks per peer, world): block (b, q) copies its share of my statistics into peer q's slot for me; the last block
-// to finish for a peer (fence + counter) raises my flag there.
-__global__ void __launch_bounds__(256)
-k_peer_push(const double *__restrict__ stats, int64_t n, void *const *__restrict__ areas, int rank, int world,
-            const unsigned long long *__restrict__ seq_p, unsigned int *__restrict__ done) {
-  const int q = blockIdx.y;
-  if (q == rank) return;
-  const unsigned long long seq = *seq_p + 1;
-  const int set = (int)(seq & 1);
-  double *dst = reinterpret_cast<double *>(areas[q]) + ((int64_t)set * world + rank) * n;
-  const int64_t n2 = n >> 1;
-  const double2 *s2 = reinterpret_cast<const double2 *>(stats);
-  double2 *d2 = reinterpret_cast<double2 *>(dst);
-  if ((reinterpret_cast<uintptr_t>(dst) & 15) == 0 && (reinterpret_cast<uintptr_t>(stats) & 15) == 0) {
-    for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < n2; i += (int64_t)gridDim.x * blockDim.x) d2[i] = s2[i];
-    if ((n & 1) && blockIdx.x == 0 && threadIdx.x == 0) dst[n - 1] = stats[n - 1];
-  } else {
-    for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (int64_t)gridDim.x * blockDim.x) dst[i] = stats[i];
-  }
-  __threadfence_system();
-  __syncthreads();
-  if (threadIdx.x == 0) {
-    const unsigned int prev = atomicAdd(&done[q], 1u);
-    if (prev == gridDim.x - 1) {
-      done[q] = 0;
-      __threadfence_system();
-      unsigned long long *flags = reinterpret_cast<unsigned long long *>(reinterpret_cast<double *>(areas[q]) + 2 * (int64_t)world * n);
-      st_release_sys(flags + set * world + rank, seq);
-    }
-  }
-}
-
-// every block waits for the flags of all peers (bounded: ~20 s, then *err = 1), then statistics = sum over the ranks in rank
-// order; the last block to finish advances the iteration counter
-__global__ void __launch_bounds__(256)
-k_peer_reduce(double *__restrict__ stats, int64_t n, const double *__restrict__ area, int rank, int world,
-              unsigned long long *__restrict__ seq_p, unsigned int *__restrict__ done, int *__restrict__ err) {
-  const unsigned long long seq = *seq_p + 1;
-  const int set = (int)(seq & 1);
-  const unsigned long long *flags = reinterpret_cast<const unsigned long long *>(area + 2 * (int64_t)world * n);
-  if (threadIdx.x < world && threadIdx.x != rank) {
-    long long t0, t1;
-    asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(t0));
-    while (ld_acquire_sys(flags + set * world + threadIdx.x) < seq) {
-      asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(t1));
-      if (t1 - t0 > 20000000000ll) { *err = 1; break; }
-    }
-  }
-  __syncthreads();
-  const double *slots = area + (int64_t)set * world * n;
-  for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (int64_t)gridDim.x * blockDim.x) {
-    double sacc = 0.0;
-    for (int q = 0; q < world; q++) sacc += (q == rank) ? stats[i] : slots[(int64_t)q * n + i];
-    stats[i] = sacc;
-  }
-  __threadfence();
-  __syncthreads();
-  if (threadIdx.x == 0) {
-    const unsigned int prev = atomicAdd(&done[world], 1u);
-    if (prev == gridDim.x - 1) {
-      done[world] = 0;
-      *seq_p = seq;
-    }
-  }
-}
-
-// One launch for the whole sum: block b pushes ITS slice of my statistics into every peer's slot for me, fences, raises the
-// slice's flag there, waits for the same slice's flags of all peers in my own area and adds the slices in rank order.  The
-// ranks synchronise slice by slice (no grid-wide hand-off, no second launch).  Blocks depend on remote blocks only, and a
-// block pushes before it waits, so any grid that is resident at once (<= kPeerBlocks <= SM count) cannot dead-lock.
+// Area of a rank: tagged words [2 slot sets][world][n] x 16 B.  Iteration `seq` (1, 2, ..) uses slot set seq & 1.
+// Every double travels as two 8-byte words {low half, seq} {high half, seq} written with one 16-byte volatile store ("LL"
+// stores, the scheme of the collective libraries' low-latency protocol); an aligned 8-byte word is written atomically, so a
+// word whose tag equals this iteration's seq carries this iteration's data, and the receiver simply polls the words it is
+// about to add: no fence, no flags, nothing to reset (the area starts zeroed and seq starts at 1).  A thread pushes its
+// elements to every peer and then adds the peers' elements in rank order as they land.  Twice the NVLink bytes of plain
+// doubles (1 MB per peer at C2), but no block depends on another block, and no fence: faster than the fenced forms with
+// flags at 2, 4 and 8 GPUs (DESIGN.md section 6).
 constexpr int kPeerBlocks = 128;
-__global__ void __launch_bounds__(256)
-k_peer_allreduce1(double *__restrict__ stats, int64_t n, void *const *__restrict__ areas, const double *__restrict__ area, int rank, int world,
-                  unsigned long long *__restrict__ seq_p, unsigned int *__restrict__ done, int *__restrict__ err,
-                  long long *__restrict__ stamps) {
-  const unsigned long long seq = *seq_p + 1;
-  const int set = (int)(seq & 1), b = blockIdx.x, nb = gridDim.x;
-  // experiment switch "peer_dbg": %globaltimer of block b at start | stores issued | fenced | peers' flags seen | summed
-  auto stamp = [&](int k) {
-    if (stamps && threadIdx.x == 0) {
-      long long t;
-      asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(t));
-      stamps[b * 8 + k] = t;
-    }
-  };
-  stamp(0);
-  const int64_t chunk = ((n + nb - 1) / nb + 1) & ~(int64_t)1;  // even: double2 copies stay aligned
-  const int64_t i0 = min(n, (int64_t)b * chunk), i1 = min(n, i0 + chunk);
-  const size_t flag_off = sizeof(double) * (size_t)(2 * (int64_t)world * n) + sizeof(unsigned long long) * 2 * (size_t)world;
-  for (int q = 0; q < world; q++) {
-    if (q == rank) continue;
-    double *dst = reinterpret_cast<double *>(areas[q]) + ((int64_t)set * world + rank) * n;
-    if ((reinterpret_cast<uintptr_t>(dst) & 15) == 0 && (reinterpret_cast<uintptr_t>(stats) & 15) == 0) {
-      const double2 *s2 = reinterpret_cast<const double2 *>(stats + i0);
-      double2 *d2 = reinterpret_cast<double2 *>(dst + i0);
-      const int64_t m2 = (i1 - i0) >> 1;
-      for (int64_t i = threadIdx.x; i < m2; i += blockDim.x) d2[i] = s2[i];
-      if (((i1 - i0) & 1) && threadIdx.x == 0) dst[i1 - 1] = stats[i1 - 1];
-    } else {
-      for (int64_t i = i0 + threadIdx.x; i < i1; i += blockDim.x) dst[i] = stats[i];
-    }
-  }
-  stamp(1);
-  __threadfence_system();
-  __syncthreads();
-  stamp(2);
-  if (threadIdx.x < world && threadIdx.x != rank) {
-    unsigned long long *fq = reinterpret_cast<unsigned long long *>(reinterpret_cast<char *>(areas[threadIdx.x]) + flag_off);
-    st_release_sys(fq + ((int64_t)set * world + rank) * kPeerBlocks + b, seq);
-    const unsigned long long *fl = reinterpret_cast<const unsigned long long *>(reinterpret_cast<const char *>(area) + flag_off);
-    long long t0, t1;
-    asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(t0));
-    while (ld_acquire_sys(fl + ((int64_t)set * world + threadIdx.x) * kPeerBlocks + b) < seq) {
-      asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(t1));
-      if (t1 - t0 > 20000000000ll) { *err = 1; break; }
-    }
-  }
-  __syncthreads();
-  stamp(3);
-  const double *slots = area + (int64_t)set * world * n;
-  for (int64_t i = i0 + threadIdx.x; i < i1; i += blockDim.x) {
-    double sacc = 0.0;
-    for (int q = 0; q < world; q++) sacc += (q == rank) ? stats[i] : slots[(int64_t)q * n + i];
-    stats[i] = sacc;
-  }
-  __syncthreads();
-  stamp(4);
-  if (threadIdx.x == 0) {
-    const unsigned int prev = atomicAdd(&done[world], 1u);
-    if (prev == gridDim.x - 1) {  // every block has read the counter by now
-      done[world] = 0;
-      *seq_p = seq;
-    }
-  }
-}
-
-// The same sum with NO fence and NO separate flags ("LL" stores, the scheme of the collective libraries' low-latency protocol):
-// every double travels as two 8-byte words {low half, seq} {high half, seq} written with one 16-byte volatile store; an aligned
-// 8-byte word is written atomically, so a word whose tag equals this iteration's seq carries this iteration's data, and the
-// receiver simply polls the words it is about to add.  k_peer_allreduce1 spends 5-6 us in __threadfence_system and 6-12 us
-// waiting for the peers' slice flags (scripts/peer_stamps.py); here a thread pushes its elements to every peer and then adds the
-// peers' elements in rank order as they land.  Twice the NVLink bytes (1 MB per peer at C2), no block depends on another block.
 __device__ __forceinline__ void st_ll(void *p, uint32_t lo, uint32_t hi, uint32_t tag) {
   asm volatile("st.volatile.global.v4.u32 [%0], {%1, %2, %3, %4};" ::"l"(p), "r"(lo), "r"(tag), "r"(hi), "r"(tag) : "memory");
 }
@@ -2474,31 +2259,21 @@ __device__ __forceinline__ bool ld_ll(const void *p, uint32_t tag, double &v) {
   return t0 == tag && t1 == tag;
 }
 __global__ void __launch_bounds__(256)
-k_peer_allreduce_ll(double *__restrict__ stats, int64_t n, void *const *__restrict__ areas, size_t ll_off, int rank, int world,
-                    unsigned long long *__restrict__ seq_p, unsigned int *__restrict__ done, int *__restrict__ err, long long *__restrict__ stamps) {
+k_peer_allreduce_ll(double *__restrict__ stats, int64_t n, void *const *__restrict__ areas, int rank, int world,
+                    unsigned long long *__restrict__ seq_p, unsigned int *__restrict__ done, int *__restrict__ err) {
   const unsigned long long seq = *seq_p + 1;
   const int set = (int)(seq & 1);
   const uint32_t tag = (uint32_t)seq;
   const int64_t tid = (int64_t)blockIdx.x * blockDim.x + threadIdx.x, nth = (int64_t)gridDim.x * blockDim.x;
-  auto stamp = [&](int k) {
-    if (stamps && threadIdx.x == 0) {
-      long long t;
-      asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(t));
-      stamps[blockIdx.x * 8 + k] = t;
-    }
-  };
-  stamp(0);
   for (int64_t i = tid; i < n; i += nth) {
     const double v = stats[i];
     const uint32_t lo = (uint32_t)__double2loint(v), hi = (uint32_t)__double2hiint(v);
     for (int q = 0; q < world; q++) {
       if (q == rank) continue;
-      st_ll(reinterpret_cast<char *>(areas[q]) + ll_off + (((int64_t)set * world + rank) * n + i) * 16, lo, hi, tag);
+      st_ll(reinterpret_cast<char *>(areas[q]) + (((int64_t)set * world + rank) * n + i) * 16, lo, hi, tag);
     }
   }
-  stamp(1);
-  stamp(2);
-  const char *mine = reinterpret_cast<const char *>(areas[rank]) + ll_off + (int64_t)set * world * n * 16;
+  const char *mine = reinterpret_cast<const char *>(areas[rank]) + (int64_t)set * world * n * 16;
   long long t0 = 0;
   for (int64_t i = tid; i < n; i += nth) {
     double sacc = 0.0;
@@ -2520,8 +2295,6 @@ k_peer_allreduce_ll(double *__restrict__ stats, int64_t n, void *const *__restri
     stats[i] = sacc;
   }
   __syncthreads();
-  stamp(3);
-  stamp(4);
   if (threadIdx.x == 0) {
     const unsigned int prev = atomicAdd(&done[world], 1u);
     if (prev == gridDim.x - 1) {  // every block has read the counter by now
@@ -2532,13 +2305,7 @@ k_peer_allreduce_ll(double *__restrict__ stats, int64_t n, void *const *__restri
 }
 
 static int64_t peer_slot_doubles(const hmmcu_ctx *ctx) { return hmmcu_stats_size(ctx->N, ctx->M, ctx->Dm) * ctx->V; }
-// slots [2][world][n] | flags of the two-kernel form [2][world] | per-slice flags of k_peer_allreduce1 [2][world][kPeerBlocks] |
-// (16-byte aligned) tagged words of k_peer_allreduce_ll [2][world][n][2]
-static size_t peer_ll_offset(int64_t n, int world) {
-  const size_t b = sizeof(double) * (size_t)(2 * (int64_t)world * n) + sizeof(unsigned long long) * 2 * (size_t)world * (1 + kPeerBlocks);
-  return (b + 15) & ~(size_t)15;
-}
-static size_t peer_area_bytes(int64_t n, int world) { return peer_ll_offset(n, world) + (size_t)16 * 2 * (size_t)world * (size_t)n; }
+static size_t peer_area_bytes(int64_t n, int world) { return (size_t)16 * 2 * (size_t)world * (size_t)n; }
 
 static void peer_close(hmmcu_ctx *ctx) {
   for (void *p : ctx->peer_opened) cudaIpcCloseMemHandle(p);
@@ -2558,7 +2325,7 @@ int hmmcu_peer_export(hmmcu_ctx *ctx, int world, void *handle_out) {
   ctx->peer_area.release();  // a fresh allocation: the handle names the allocation, not a sub-range
   CK(ctx->peer_area.ensure(peer_area_bytes(n, world)));
   CK(cudaMemsetAsync(ctx->peer_area.p, 0, peer_area_bytes(n, world), ctx->st));
-  CK(ctx->peer_seq_d.ensure(sizeof(unsigned long long) + sizeof(unsigned int) * 80 + sizeof(int)));  // seq | done[world + 1] | err
+  CK(ctx->peer_seq_d.ensure(sizeof(unsigned long long) + sizeof(unsigned int) * 80 + sizeof(int)));  // seq | done[80] (done[world]: blocks finished) | err
   CK(cudaMemsetAsync(ctx->peer_seq_d.p, 0, sizeof(unsigned long long) + sizeof(unsigned int) * 80 + sizeof(int), ctx->st));
   CK(cudaStreamSynchronize(ctx->st));
   ctx->peer_n = n;
@@ -2617,74 +2384,20 @@ static int peer_ready(hmmcu_ctx *ctx, const char *what) {
   return HMMCU_OK;
 }
 
-int hmmcu_peer_push(hmmcu_ctx *ctx) {
-  int rc = peer_ready(ctx, "peer_push");
-  if (rc) return rc;
-  CK(cudaSetDevice(ctx->dev));
-  if (ctx->peer_world == 1) return HMMCU_OK;
-  unsigned long long *seq = ctx->peer_seq_d.as<unsigned long long>();
-  unsigned int *done = reinterpret_cast<unsigned int *>(seq + 1);
-  const int bpp = (int)std::max<int64_t>(1, std::min<int64_t>(16, ctx->peer_n / 4096));
-  t_begin(ctx, "allreduce");
-  k_peer_push<<<dim3(bpp, ctx->peer_world), 256, 0, ctx->st>>>(ctx->stats.as<double>(), ctx->peer_n, ctx->peer_ptrs_d.as<void *>(), ctx->peer_rank,
-                                                             ctx->peer_world, seq, done);
-  LAUNCH_CHECK();
-  return HMMCU_OK;
-}
-
-int hmmcu_peer_reduce(hmmcu_ctx *ctx) {
-  int rc = peer_ready(ctx, "peer_reduce");
-  if (rc) return rc;
-  CK(cudaSetDevice(ctx->dev));
-  if (ctx->peer_world == 1) return HMMCU_OK;
-  unsigned long long *seq = ctx->peer_seq_d.as<unsigned long long>();
-  unsigned int *done = reinterpret_cast<unsigned int *>(seq + 1);
-  int *err = reinterpret_cast<int *>(done + 80);
-  const int blocks = (int)std::max<int64_t>(1, std::min<int64_t>(ctx->sm_count, (ctx->peer_n + 1023) / 1024));
-  k_peer_reduce<<<blocks, 256, 0, ctx->st>>>(ctx->stats.as<double>(), ctx->peer_n, ctx->peer_area.as<double>(), ctx->peer_rank, ctx->peer_world, seq,
-                                             done, err);
-  LAUNCH_CHECK();
-  t_end(ctx, "allreduce");
-  return HMMCU_OK;
-}
-
 int hmmcu_peer_allreduce(hmmcu_ctx *ctx) {
   int rc = peer_ready(ctx, "peer_allreduce");
   if (rc) return rc;
   CK(cudaSetDevice(ctx->dev));
   if (ctx->peer_world == 1) return HMMCU_OK;
-  if (!ctx->peer_fused) {
-    rc = hmmcu_peer_push(ctx);
-    return rc ? rc : hmmcu_peer_reduce(ctx);
-  }
   unsigned long long *seq = ctx->peer_seq_d.as<unsigned long long>();
   unsigned int *done = reinterpret_cast<unsigned int *>(seq + 1);
   int *err = reinterpret_cast<int *>(done + 80);
-  if (ctx->peer_ll) {  // tagged 8-byte words, no fence, no flags
-    const int blocks = (int)std::max<int64_t>(1, std::min<int64_t>(std::min(kPeerBlocks, ctx->sm_count), (ctx->peer_n + 255) / 256));
-    t_begin(ctx, "allreduce");
-    k_peer_allreduce_ll<<<blocks, 256, 0, ctx->st>>>(ctx->stats.as<double>(), ctx->peer_n, ctx->peer_ptrs_d.as<void *>(), peer_ll_offset(ctx->peer_n, ctx->peer_world),
-                                                     ctx->peer_rank, ctx->peer_world, seq, done, err, ctx->peer_dbg ? ctx->peer_stamps.as<long long>() : nullptr);
-    LAUNCH_CHECK();
-    t_end(ctx, "allreduce");
-    return HMMCU_OK;
-  }
-  int blocks = (int)std::max<int64_t>(1, std::min<int64_t>(std::min(kPeerBlocks, ctx->sm_count), (ctx->peer_n + 2047) / 2048));
-  if (ctx->peer_fused > 1) blocks = std::min(std::min(kPeerBlocks, ctx->sm_count), ctx->peer_fused);  // experiments: the grid size
+  const int blocks = (int)std::max<int64_t>(1, std::min<int64_t>(std::min(kPeerBlocks, ctx->sm_count), (ctx->peer_n + 255) / 256));
   t_begin(ctx, "allreduce");
-  k_peer_allreduce1<<<blocks, 256, 0, ctx->st>>>(ctx->stats.as<double>(), ctx->peer_n, ctx->peer_ptrs_d.as<void *>(), ctx->peer_area.as<double>(),
-                                                 ctx->peer_rank, ctx->peer_world, seq, done, err, ctx->peer_dbg ? ctx->peer_stamps.as<long long>() : nullptr);
+  k_peer_allreduce_ll<<<blocks, 256, 0, ctx->st>>>(ctx->stats.as<double>(), ctx->peer_n, ctx->peer_ptrs_d.as<void *>(), ctx->peer_rank,
+                                                   ctx->peer_world, seq, done, err);
   LAUNCH_CHECK();
   t_end(ctx, "allreduce");
-  return HMMCU_OK;
-}
-
-// experiment read-out ("peer_dbg"): the stamps of the last k_peer_allreduce1, [kPeerBlocks][8] (scripts/peer_stamps.py)
-extern "C" int hmmcu_debug_peer_read(hmmcu_ctx *ctx, long long *out) {
-  if (!ctx || !out || !ctx->peer_stamps.p) return HMMCU_EINVAL;
-  CK(cudaSetDevice(ctx->dev));
-  CK(cudaMemcpyAsync(out, ctx->peer_stamps.p, sizeof(long long) * kPeerBlocks * 8, cudaMemcpyDeviceToHost, ctx->st));
-  CK(cudaStreamSynchronize(ctx->st));
   return HMMCU_OK;
 }
 

@@ -490,7 +490,7 @@ __global__ void __launch_bounds__(kTcThreads, 1)
 k_accum_tc(const TcTile *__restrict__ units, int nunits, const int32_t *__restrict__ frame_ids, const float *__restrict__ x32,
            const float *__restrict__ images, const float *__restrict__ kcT, const float *__restrict__ logb,
            const float *__restrict__ gamma, int N, int M, int G, int D, int DP, double *__restrict__ stats,
-           int64_t stats_stride, int64_t off_S0, int64_t off_S1, int64_t off_S2, float *__restrict__ dbg) {
+           int64_t stats_stride, int64_t off_S0, int64_t off_S1, int64_t off_S2) {
   extern __shared__ __align__(1024) uint8_t smem_raw[];
   __shared__ uint64_t mbar;
   __shared__ uint32_t tmem_base_s;
@@ -663,10 +663,6 @@ k_accum_tc(const TcTile *__restrict__ units, int nunits, const int32_t *__restri
       for (int c0 = chalf * 64; c0 < chalf * 64 + 64; c0 += 16) {
         uint32_t v[16], vl[16];
         tmem_ld16(tm_d1 + trow + c0, v);
-        if (dbg && ui == 0) {
-#pragma unroll
-          for (int j = 0; j < 16; j++) dbg[row * 128 + c0 + j] = fmaf(__uint_as_float(v[j]), 1.4426950408889634f, kcr);
-        }
 #pragma unroll
         for (int j = 0; j < 16; j++) {
           const float y = fmaf(__uint_as_float(v[j]), 1.4426950408889634f, kcr + cfs[(c0 + j) * 8 + s]);
@@ -677,7 +673,6 @@ k_accum_tc(const TcTile *__restrict__ units, int nunits, const int32_t *__restri
           split_tf32(w, h, l);
           v[j] = __float_as_uint(h);
           vl[j] = __float_as_uint(l);
-          if (dbg && ui == 0) dbg[16384 + row * 128 + c0 + j] = h + l;
         }
         tmem_st16(tm_d1 + trow + c0, v);
         tmem_st16(tm_wl + trow + c0, vl);
@@ -708,13 +703,6 @@ k_accum_tc(const TcTile *__restrict__ units, int nunits, const int32_t *__restri
     mbar_wait(&mbar, parity);
     parity ^= 1;
     tc_fence_after();
-    if (dbg && ui == 0) {
-      for (int c8 = c8_beg; c8 < c8_end; c8++) {
-        float v[8];
-        tmem_ld8(tm_d2 + trow + c8 * 8, v);
-        for (int j = 0; j < 8; j++) dbg[32768 + row * 128 + c8 * 8 + j] = v[j];
-      }
-    }
     if (++since_flush >= kAccFlushTiles) { drain_tmem(); since_flush = 0; }
     tc_fence_before();
     __syncthreads();  // X, XT, cfs and the weight columns are free again

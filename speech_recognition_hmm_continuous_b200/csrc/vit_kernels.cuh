@@ -245,84 +245,10 @@ __device__ __forceinline__ void cell_load(const float *__restrict__ p, float (&l
   for (int i = 0; i < NS; i++) l[i] = __ldg(p + i);
 }
 
-// forward score: log P(O, q_T = N-1 | model)   (calc_alpha + calc_probability, R-FS:739-836)
-template <int NS, bool BANDED>
-__global__ void __launch_bounds__(kCellThreads)
-k_fwd_cells(const float *__restrict__ logb, int64_t fbase, int64_t ldb, const int64_t *__restrict__ off, int u0, int nu,
-            int V, const double *__restrict__ Aall, double *__restrict__ out) {
-  const int64_t cell = (int64_t)blockIdx.x * kCellThreads + threadIdx.x;
-  if (cell >= (int64_t)nu * V) return;
-  const int u = u0 + (int)(cell / V), v = (int)(cell % V);
-  const int64_t base = off[u];
-  const int T = (int)(off[u + 1] - base);
-  double a[NS * NS];
-#pragma unroll
-  for (int k = 0; k < NS * NS; k++) a[k] = Aall[(int64_t)v * NS * NS + k];
-  double z[NS];
-#pragma unroll
-  for (int i = 0; i < NS; i++) z[i] = 0.0;
-  double msum = 0.0;
-  int esum = 0;
-  const float *p = logb + (base - fbase) * ldb + (int64_t)v * NS;
-  float nxt[kCellPF][NS];
-#pragma unroll
-  for (int k = 0; k < kCellPF; k++) cell_load<NS>(p + (int64_t)min(k, T - 1) * ldb, nxt[k]);
-  for (int t0 = 0; t0 < T; t0 += kCellPF) {
-    float cur[kCellPF][NS];
-#pragma unroll
-    for (int k = 0; k < kCellPF; k++) {
-#pragma unroll
-      for (int i = 0; i < NS; i++) cur[k][i] = nxt[k][i];
-    }
-#pragma unroll
-    for (int k = 0; k < kCellPF; k++) cell_load<NS>(p + (int64_t)min(t0 + kCellPF + k, T - 1) * ldb, nxt[k]);
-#pragma unroll
-    for (int k = 0; k < kCellPF; k++) {
-      if (t0 + k < T) {
-        float m = cur[k][0];
-#pragma unroll
-        for (int i = 1; i < NS; i++) m = fmaxf(m, cur[k][i]);
-        const float ms = (m > kNegInf) ? m : 0.f;
-        double raw[NS];
-        if (t0 + k == 0) {
-#pragma unroll
-          for (int i = 0; i < NS; i++) raw[i] = (i == 0) ? exp_scaled(cur[k][0] - ms) : 0.0;  // pi = [1,0,..,0]
-        } else {
-#pragma unroll
-          for (int i = 0; i < NS; i++) {
-            double aux;
-            if (BANDED) {
-              aux = z[i] * a[i * NS + i];
-              if (i > 0) aux = fma(z[i - 1], a[(i - 1) * NS + i], aux);
-            } else {
-              aux = 0.0;
-#pragma unroll
-              for (int j = 0; j < NS; j++) aux = fma(z[j], a[j * NS + i], aux);
-            }
-            raw[i] = aux * exp_scaled(cur[k][i] - ms);
-          }
-        }
-        double s = raw[0];
-#pragma unroll
-        for (int i = 1; i < NS; i++) s += raw[i];
-        int e;
-        const double r = pow2_scale(s, e);
-#pragma unroll
-        for (int i = 0; i < NS; i++) z[i] = raw[i] * r;
-        esum += e;
-        msum += (double)m;  // -inf when every state's density is 0: the score is -inf, as log(0) in the reference
-      }
-    }
-  }
-  // log P = sum m_t + ln2 sum e_t + log z_{T-1}(N-1); z is normalised to [1,2) by a power of two, so
-  // log(alpha^_{T-1}(N-1)) + sum log(1/c_t) of calc_probability (R-FS:820-836) telescopes to this.
-  out[(int64_t)u * V + v] = msum + 0.6931471805599453 * (double)esum + log(z[NS - 1]);
-}
-
-// The same score with the chain in SINGLE precision, in the LOG domain (default; k_fwd_cells stays behind the
-// "fwd_f64" option).  The double-precision chain above issues ~140 instructions per (cell, frame) -- five software
-// exponentials assembled into doubles, a scaling pass -- and is bound by instruction issue at half the HBM rate.  A
-// single-precision chain in the linear domain is not an option: against a mismatched model a state's mass falls by
+// forward score: log P(O, q_T = N-1 | model)   (calc_alpha + calc_probability, R-FS:739-836), with the chain in SINGLE
+// precision, in the LOG domain.  A double-precision linear chain issues ~140 instructions per (cell, frame) -- five
+// software exponentials assembled into doubles, a scaling pass -- and was bound by instruction issue at half the HBM
+// rate.  A single-precision chain in the linear domain is not an option: against a mismatched model a state's mass falls by
 // e^-100 per frame relative to its neighbour's, and a state that is 2^-126 below the frame's maximum today can carry the
 // best path tomorrow (measured: 2.5 % error in such a cell), where the reference's doubles still hold it.  So every state
 // keeps its own magnitude: with lz_i = log2 of the scaled alpha (max_i lz_i = 0 after every frame),

@@ -306,17 +306,13 @@ __device__ __forceinline__ void tc_mma_f16_ts(uint32_t tmem_d, uint32_t tmem_a, 
 // chunks 0-2 / 3-4 of the doubled row), 16 MMA issuer.
 // MR: mixtures of a state that are real (MR <= MP; the others are pad columns the log-sum-exp may skip), 0 = all MP
 // H16: half-precision operands (images of k_pack_w_dec16, `scales` of k_dec16_scales; DP a multiple of 8)
-template <bool TRAIN, int MP, bool DBG, int MR = 0, bool H16 = false>
+template <bool TRAIN, int MP, int MR = 0, bool H16 = false>
 __global__ void __launch_bounds__(kWsThreads, 1)
 k_emis_ws(const TcTile *__restrict__ units, int nunits, int ntiles_dec, int nframes_dec, const int32_t *__restrict__ frame_ids,
           const float *__restrict__ x32, const float *__restrict__ images, int N, int M, int DP, int TN, float *__restrict__ logb,
-          int64_t fbase, int64_t ldb, int S_total, int SCt, long long *__restrict__ tdbg, const float *__restrict__ scales = nullptr) {
+          int64_t fbase, int64_t ldb, int S_total, int SCt, const float *__restrict__ scales = nullptr) {
   extern __shared__ __align__(1024) uint8_t smem_raw[];
   const int KP = 2 * DP, NSLAB = H16 ? KP / 16 : KP / 8;  // K per MMA: 16 halves / 8 TF32 (8 tensor-memory columns, 256 bytes of a W row group)
-  // optional timeline of CTA 0 (diagnostic build): tdbg[unit][8] clock stamps
-  auto stamp = [&](int i, int slot) {
-    if (DBG && tdbg && blockIdx.x == 0 && (threadIdx.x & 31) == 0 && i < 64) tdbg[i * 8 + slot] = clock64();
-  };
   const uint32_t P = H16 ? (uint32_t)(KP / 8) * 128 : (uint32_t)(KP / 4) * 128;
   const uint32_t w_bytes = 2 * (uint32_t)(TN / 8) * P, img_bytes = w_bytes + (uint32_t)TN * 4;
   const uint32_t Ws = (smem_u32(smem_raw) + 1023u) & ~1023u;  // [hi | lo], shared-window address
@@ -399,9 +395,7 @@ k_emis_ws(const TcTile *__restrict__ units, int nunits, int ntiles_dec, int nfra
         for (int k = tid - kWsEpiWarps * 32; k < (int)(w_bytes / 16); k += 256) st_shared_v4(Ws + 16 * k, __ldg(wsrc + k));
         cur_img = unit.img;
       }
-      if (warp == kWsEpiWarps) stamp(i, 0);
       mbar_wait_a(empty + 8 * s, (ku & 1) ^ 1);  // operand stage s is free (unit i-AST has been multiplied)
-      if (warp == kWsEpiWarps) stamp(i, 1);
       tc_fence_after();
       // stage s: [x_hi (DP) | x2_hi (DP) | x_lo (DP) | x2_lo (DP)], 4 columns per store
       if (H16) {
@@ -447,7 +441,6 @@ k_emis_ws(const TcTile *__restrict__ units, int nunits, int ntiles_dec, int nfra
       tc_fence_before();
       fence_async_smem();  // the W image (generic-proxy writes) -> visible to the tensor core
       mbar_arrive_a(full + 8 * s);
-      if (warp == kWsEpiWarps) stamp(i, 2);
     };
     TcTile d0 = unit_at(u_begin), d1 = unit_at(u_begin + 1), d2 = unit_at(u_begin + 2);
     int64_t f1 = frame_of(d1);
@@ -474,9 +467,7 @@ k_emis_ws(const TcTile *__restrict__ units, int nunits, int ntiles_dec, int nfra
       const int s = i & 1, sa = i % AST;
       const uint32_t ph = (i >> 1) & 1;
       mbar_wait_a(full + 8 * sa, (i / AST) & 1);  // operands landed
-      stamp(i, 3);
       mbar_wait_a(dempty + 8 * s, ph ^ 1);    // accumulator stage drained by the epilogue (unit i-2)
-      stamp(i, 4);
       tc_fence_after();
       if (elect_one_sync()) {
         const uint32_t xh = tb + (uint32_t)sa * 160, xl = xh + (H16 ? (uint32_t)DP : 80u);
@@ -515,7 +506,6 @@ k_emis_ws(const TcTile *__restrict__ units, int nunits, int ntiles_dec, int nfra
         tc_commit_a(dfull + 8 * s);   // accumulator ready
       }
       __syncwarp();
-      stamp(i, 5);
     }
   } else {
     // =================================== EPILOGUE (warps 0 .. kWsEpiWarps-1) ===================================
@@ -554,7 +544,6 @@ k_emis_ws(const TcTile *__restrict__ units, int nunits, int ntiles_dec, int nfra
       const TcTile un2 = unit_at(ui + 2);
       const int s = i & 1;
       mbar_wait_a(dfull + 8 * s, (i >> 1) & 1);
-      if (warp == 0) stamp(i, 6);
       tc_fence_after();
       const int st_lim = TRAIN ? N : S_total;
       const int nst = max(0, min(SCt, st_lim - unit.state0));  // states present in this image
@@ -685,7 +674,6 @@ k_emis_ws(const TcTile *__restrict__ units, int nunits, int ntiles_dec, int nfra
       }
       tc_fence_before();
       mbar_arrive_a(dempty + 8 * s);
-      if (warp == 0) stamp(i, 7);
       un0 = un1; un1 = un2; fcur = fnext;
     }
   }
@@ -741,20 +729,12 @@ __host__ __device__ inline size_t ws_acc_smem_bytes(int KP) {
   return kAccStages * ws_acc_stage_bytes(KP) + 1024 + 256 + kAccImgCap * 4 + (size_t)tc_kp2(KP) * 128 * 4;
 }
 
-__device__ int g_acc_dbg = 0;  // experiments ("acc_dbg" option; results are garbage): 1 = no weight arithmetic in the epilogue, 2 = no MMAs
-
-template <bool DBG>
 __global__ void __launch_bounds__(kAccWsThreads, 1)
 k_accum_ws(const TcTile *__restrict__ units, int nunits, const int32_t *__restrict__ frame_ids, const float *__restrict__ x32,
            const float *__restrict__ images, const float *__restrict__ kcT, const float *__restrict__ logb,
            const float *__restrict__ gamma, int N, int M, int G, int D, int DP, double *__restrict__ stats,
-           int64_t stats_stride, int64_t off_S0, int64_t off_S1, int64_t off_S2, float *__restrict__ scratch,
-           long long *__restrict__ tdbg) {
+           int64_t stats_stride, int64_t off_S0, int64_t off_S1, int64_t off_S2, float *__restrict__ scratch) {
   extern __shared__ __align__(1024) uint8_t smem_raw[];
-  if (DBG && tdbg && blockIdx.x == 0 && threadIdx.x == 0) tdbg[1024] = clock64();
-  auto stamp = [&](int i, int slot) {  // latest arrival over the warps of a role (diagnostic build only)
-    if (DBG && tdbg && blockIdx.x == 0 && (threadIdx.x & 31) == 0 && i < 64) atomicMax((unsigned long long *)&tdbg[i * 16 + slot], (unsigned long long)clock64());
-  };
   constexpr int NST = kAccStages, SUB = kAccSub;
   const int KP = 2 * DP, KP2 = tc_kp2(KP), NSLAB = KP / 8, nq = DP / 4;
   const uint32_t PX = (uint32_t)(KP / 4) * 128;            // X: bytes per group of 8 frames
@@ -799,13 +779,11 @@ k_accum_ws(const TcTile *__restrict__ units, int nunits, const int32_t *__restri
   __syncthreads();
   tc_fence_after();
   const uint32_t tmem0 = (uint32_t)lds_i32(tmem_slot);
-  if (DBG && tdbg && blockIdx.x == 0 && threadIdx.x == 0) tdbg[1025] = clock64();
 
   auto img_at = [&](int ui) -> int {
     if (ui < u_begin || ui >= u_end) return -1;
     return (ui - u_begin < kAccImgCap) ? lds_i32(simg + 4 * (ui - u_begin)) : __ldg(&units[ui].img);
   };
-  auto unit_at = [&](int ui) -> TcTile { return ui < u_end ? units[ui] : TcTile{0, 0, -1, 0, 0, 0}; };
 
   if (warp >= 8 && warp < 8 + kAccLdWarps) {
     // =================================== X LOADERS ===================================
@@ -837,9 +815,7 @@ k_accum_ws(const TcTile *__restrict__ units, int nunits, const int32_t *__restri
     const uint32_t rbase = (uint32_t)(xr & 7) * 16 + (uint32_t)(xr >> 3) * PX;
     auto expand = [&](int i, const Pre &cur) {
       const int s = i % NST;
-      if (warp == 8) stamp(i, 0);
       mbar_wait_a(x_free + 8 * s, ((i / NST) & 1) ^ 1);  // stage s: GEMM2 of unit i-NST has retired
-      if (warp == 8) stamp(i, 1);
       const uint32_t Xh = sm0 + (uint32_t)s * stage_bytes, Xl = Xh + x_bytes;
 #pragma unroll
       for (int j = 0; j < kXQ; j++) {
@@ -857,7 +833,6 @@ k_accum_ws(const TcTile *__restrict__ units, int nunits, const int32_t *__restri
           st_shared_v4(Xl + o, l);
         }
       }
-      if (warp == 8) stamp(i, 10);
       // weight exponent of frame xr per state: log2(gamma) - logb log2(e); -inf = no weight.  cfs[state][frame]
       const uint32_t cfs = Xh + cfs_off + 4 * xr;
 #pragma unroll
@@ -869,10 +844,8 @@ k_accum_ws(const TcTile *__restrict__ units, int nunits, const int32_t *__restri
           sts_f32(cfs + st * SUB * 4, cf);
         }
       }
-      if (warp == 8) stamp(i, 11);
       fence_async_smem();
       mbar_arrive_a(x_full + 8 * s);
-      stamp(i, 2);
     };
     int2 d1 = desc_at(u_begin + 1), d2 = desc_at(u_begin + 2);
     int f1 = fid_of(d1);
@@ -915,9 +888,7 @@ k_accum_ws(const TcTile *__restrict__ units, int nunits, const int32_t *__restri
     };
     auto expand = [&](int i, const Pre &cur) {
       const int s = i % NST;
-      if (warp == 8 + kAccLdWarps) stamp(i, 14);
       mbar_wait_a(x_free + 8 * s, ((i / NST) & 1) ^ 1);
-      if (warp == 8 + kAccLdWarps) stamp(i, 12);
       const uint32_t XTh = sm0 + (uint32_t)s * stage_bytes + 2 * x_bytes, XTl = XTh + xt_bytes;
 #pragma unroll
       for (int k = 0; k < kTK; k++) {  // rows n (x) and n + DP (x^2), 16-byte chunk = frames 4fg..4fg+3
@@ -946,8 +917,6 @@ k_accum_ws(const TcTile *__restrict__ units, int nunits, const int32_t *__restri
       }
       fence_async_smem();
       mbar_arrive_a(x_full + 8 * s);
-      if (warp == 8 + kAccLdWarps) stamp(i, 13);
-      stamp(i, 2);
     };
     int2 d1 = desc_at(u_begin + 1), d2 = desc_at(u_begin + 2);
     Fids f1 = fids_of(d1);
@@ -979,14 +948,12 @@ k_accum_ws(const TcTile *__restrict__ units, int nunits, const int32_t *__restri
       const int img = img_at(u_begin + i);
       mbar_wait_a(x_full + 8 * s, (i / NST) & 1);
       if (img != img_prev) { mbar_wait_a(wimg_full, nimg & 1); nimg++; img_prev = img; }
-      stamp(i, 3);
       tc_fence_after();
       if (elect_one_sync()) {
         const uint32_t Xh = sm0 + (uint32_t)s * stage_bytes;
         const uint64_t bh = make_smem_desc2(Xh, 128, PX), bl = make_smem_desc2(Xh + x_bytes, 128, PX);
         const uint32_t d = tb + (uint32_t)s * SUB, wh = tb + kAccTmW, wl = wh + KP;
-        if (g_acc_dbg & 2) {
-        } else if (NSLAB == 10) {  // D = 39: fully unrolled, addresses are immediates
+        if (NSLAB == 10) {  // D = 39: fully unrolled, addresses are immediates
 #pragma unroll
           for (int j = 0; j < 10; j++) tc_mma_tf32_ts(d, wh + j * 8, bh + (uint64_t)(j * 16), idesc1, j > 0);  // Wh*Xh
 #pragma unroll
@@ -1007,7 +974,6 @@ k_accum_ws(const TcTile *__restrict__ units, int nunits, const int32_t *__restri
         tc_commit_a(d1_full + 8 * s);
       }
       __syncwarp();
-      stamp(i, 4);
     }
   } else if (warp == kAccG1Warp + 1) {
     // =================================== GEMM2 ISSUER ===================================
@@ -1021,7 +987,6 @@ k_accum_ws(const TcTile *__restrict__ units, int nunits, const int32_t *__restri
       const bool last_of_img = img_at(u_begin + j + 1) != img_at(u_begin + j);  // also true for this CTA's last unit
       mbar_wait_a(w_full + 8 * sj, (j / NST) & 1);
       if (need_s_free) { mbar_wait_a(s_free, (ndrain - 1) & 1); need_s_free = false; }
-      stamp(j, 8);
       tc_fence_after();
       cnt++;
       const bool drain = last_of_img || cnt == kAccDrain;
@@ -1029,21 +994,17 @@ k_accum_ws(const TcTile *__restrict__ units, int nunits, const int32_t *__restri
         const uint32_t XTh = sm0 + (uint32_t)sj * stage_bytes + 2 * x_bytes;
         const uint64_t bh = make_smem_desc2(XTh, 128, PT), bl = make_smem_desc2(XTh + xt_bytes, 128, PT);
         const uint32_t wh = tb + (uint32_t)sj * SUB, wl = wh + 128, d = tb + 256;
-        if (!(g_acc_dbg & 2)) {
 #pragma unroll
         for (int k = 0; k < SUB / 8; k++) tc_mma_tf32_ts(d, wh + k * 8, bh + (uint64_t)(k * 16), idesc2, (cnt > 1 || k > 0) ? 1u : 0u);  // wh*Xh
 #pragma unroll
         for (int k = 0; k < SUB / 8; k++) tc_mma_tf32_ts(d, wl + k * 8, bh + (uint64_t)(k * 16), idesc2, 1);                              // wl*Xh
 #pragma unroll
         for (int k = 0; k < SUB / 8; k++) tc_mma_tf32_ts(d, wh + k * 8, bl + (uint64_t)(k * 16), idesc2, 1);                              // wh*Xl
-        }
-        if (DBG && tdbg && blockIdx.x == 0 && j < 64) tdbg[j * 16 + 9] = clock64();
         tc_commit_a(x_free + 8 * sj);
         if (drain) tc_commit_a(s_full);
       }
       __syncwarp();
       if (drain) { ndrain++; need_s_free = true; cnt = 0; }
-      stamp(j, 5);
     }
   } else {
     // =================================== EPILOGUE (warps 0-7) ===================================
@@ -1085,8 +1046,7 @@ k_accum_ws(const TcTile *__restrict__ units, int nunits, const int32_t *__restri
         dead = cur_rb * 128 + 32 * q >= G;
       }
       mbar_wait_a(d1_full + 8 * s, (i / NST) & 1);
-      if (warp == 0) stamp(i, 6);
-      if (!dead && !(g_acc_dbg & 1)) {  // my FH frames: accumulator columns [FH hb, FH hb + FH) of stage s.  (The rows of a dead warp
+      if (!dead) {  // my FH frames: accumulator columns [FH hb, FH hb + FH) of stage s.  (The rows of a dead warp
                     // feed only pad rows of S, which are never read.)
         tc_fence_after();
         const int c0 = hb * FH;
@@ -1112,7 +1072,6 @@ k_accum_ws(const TcTile *__restrict__ units, int nunits, const int32_t *__restri
         tc_fence_before();
       }
       mbar_arrive_a(w_full + 8 * s);
-      stamp(i, 7);
       cnt++;
       if (last || cnt == kAccDrain) {  // S: TMEM (FP32, truncating) -> shared memory (round to nearest)
         mbar_wait_a(s_full, ndrain & 1);
@@ -1162,11 +1121,9 @@ k_accum_ws(const TcTile *__restrict__ units, int nunits, const int32_t *__restri
       img_prev = img; img = img_next; img_next = img_at(ui + 2);
     }
   }
-  if (DBG && tdbg && blockIdx.x == 0 && (threadIdx.x & 31) == 0) tdbg[1026 + warp] = clock64();
   tc_fence_before();
   __syncthreads();
   tc_fence_after();
-  if (DBG && tdbg && blockIdx.x == 0 && threadIdx.x == 0) tdbg[1050] = clock64();
   if (warp == kAccG1Warp) tmem_dealloc(tmem0, 512);
 }
 

@@ -913,31 +913,26 @@ def test_decode_in_many_batches_equals_one_batch(M):
 
 
 @pytest.mark.parametrize("dense", [False, True])
-def test_forward_cell_scorers_single_and_double_chain(dense):
-    """k_fwd_cells32 (log-domain single-precision chain, the default) and k_fwd_cells (double chain, option
-    "fwd_f64") against the oracle's calc_alpha + calc_probability (R-FS:739-836), for the reference's banded
-    topology and for a dense A, on mismatched models (a state's mass falls by e^-100 per frame there: a linear
-    single-precision chain loses the best path in such cells) and with an utterance shorter than the chain."""
+def test_forward_cell_scorer_against_the_oracle(dense):
+    """k_fwd_cells32 (log-domain single-precision chain) against the oracle's calc_alpha + calc_probability
+    (R-FS:739-836), for the reference's banded topology and for a dense A, on mismatched models (a state's mass falls
+    by e^-100 per frame there: a linear single-precision chain loses the best path in such cells) and with an
+    utterance shorter than the chain."""
     ms, x, off, labels = _synth(6, 5, 3, 12, seed=31, tmin=3, tmax=140)
     if dense:
         rng = np.random.default_rng(5)
         A = rng.random(ms.A.shape) + 0.05
         ms = api.ModelSet(A / A.sum(axis=2, keepdims=True), ms.c, ms.mu, ms.iv, ms.det)
     want = np.array([[o.forward_score(_oracle_model(ms, v), x[off[u]:off[u + 1]]) for v in range(ms.V)] for u in range(len(labels))])
-    got = {}
-    for f64 in (0, 1):
-        c = api.Context(0)
-        c.set_option("fwd_f64", f64)
-        c.set_features(x, off)
-        c.set_models(ms)
-        got[f64] = c.forward_scores()
-        c.close()
-        fin = np.isfinite(want)
-        assert (np.isfinite(got[f64]) == fin).all()
-        assert np.allclose(got[f64][fin], want[fin], rtol=RTOL, atol=0)
-        assert np.abs(got[f64][fin] / want[fin] - 1).max() < 2e-6
+    c = api.Context(0)
+    c.set_features(x, off)
+    c.set_models(ms)
+    got = c.forward_scores()
+    c.close()
     fin = np.isfinite(want)
-    assert np.abs(got[0][fin] / got[1][fin] - 1).max() < 1e-6
+    assert (np.isfinite(got) == fin).all()
+    assert np.allclose(got[fin], want[fin], rtol=RTOL, atol=0)
+    assert np.abs(got[fin] / want[fin] - 1).max() < 2e-6
 
 
 @pytest.mark.parametrize("N,M", [(5, 1), (5, 3), (5, 16), (3, 6), (6, 2)])
@@ -1255,12 +1250,13 @@ def test_cli_job_file_runs_every_line_in_one_process(tmp_path, monkeypatch):
         assert r.parse_train_report(str(tmp_path / ("single%d.txt" % v))) == r.parse_train_report(str(tmp_path / ("batch%d.txt" % v)))
 
 
-def test_peer_allreduce_sums_two_ranks_in_rank_order():
-    """hmmcu_peer_push / hmmcu_peer_reduce (the all-reduce of the sufficient statistics through peer memory, SURVEY 8e)
-    with two contexts of one process standing in for two ranks: both end with the same bytes, equal to rank 0's
-    statistics + rank 1's (double addition in rank order), over several iterations (the two slot sets alternate).  The
-    pushes of both ranks are enqueued before either reduce, so no kernel ever waits for one that has not been launched
-    (two spinning kernels must not share one GPU); on several GPUs the calls are simply push + reduce per rank."""
+def test_peer_allreduce_sums_two_co_resident_ranks_in_rank_order():
+    """hmmcu_peer_allreduce (the all-reduce of the sufficient statistics through peer memory, SURVEY 8e) with two
+    contexts of one process standing in for two ranks: both end with the same bytes, equal to rank 0's statistics +
+    rank 1's (double addition in rank order), over five iterations (the two slot sets alternate, so each is reused).
+    The two ranks' kernels spin on each other's tagged words; here they run on the two contexts' streams and are
+    co-resident on one GPU (each grid is at most 128 blocks of 256 threads, so both fit at once), so each one's words
+    land while the other waits."""
     ms, x, off, labels = _synth(3, 5, 4, 12, seed=1212)
     U = len(labels)
     halves = [(0, U // 2), (U // 2, U)]
@@ -1279,19 +1275,8 @@ def test_peer_allreduce_sums_two_ranks_in_rank_order():
         for r_, (c, (u0, u1)) in enumerate(zip(ctxs, halves)):
             st, _ = c.estep(labels[u0:u1])
             local.append(st)
-        if it in (1, 2, 3):
-            # the one-launch forms, both kernels spinning on each other on their own streams: 1, 3 = tagged 8-byte words
-            # (k_peer_allreduce_ll, the default; iteration 3 reuses the slot set of iteration 1), 2 = slice flags (k_peer_allreduce1)
-            for c in ctxs:
-                c.set_option("peer_ll", 0 if it == 2 else 1)
-                c.peer_allreduce()
-        else:
-            for c in ctxs:
-                c.peer_push()
-            for c in ctxs:
-                c.synchronize()
-            for c in ctxs:
-                c.peer_reduce()
+        for c in ctxs:
+            c.peer_allreduce()
         got = [c.stats_download() for c in ctxs]
         assert not ctxs[0].peer_error() and not ctxs[1].peer_error()
         want = local[0] + local[1]
