@@ -153,6 +153,21 @@ int64_t hmmcu_stats_size(int N, int M, int D);
  * below); logp_utt[U] the per-utterance log-probabilities (may be NULL). */
 int hmmcu_estep(hmmcu_ctx *ctx, const int32_t *utt2model, double *stats, double *logp_utt);
 
+/* The E-step of Viterbi (segmental k-means) training, as HTK's HInit re-segments: the same contract and the same
+ * statistics vector as hmmcu_estep, with the forward-backward pass replaced by the best state sequence of every utterance
+ * (single-precision emissions, delta in double; pi = [1,0,..], termination in the final state, lowest predecessor index
+ * on a tie, as hmmcu_viterbi).  Each frame belongs to its aligned state with weight 1, so
+ *   num_trans[i][j] = number of t < T-1 with (s_t, s_t+1) = (i, j)   (every pair of a full A, not only the band)
+ *   den_trans[i]    = number of t < T-1 with s_t = i,   den_mix[i] = number of t < T with s_t = i
+ *   S0 / S1 / S2c   the in-state mixture posteriors of the aligned state, accumulated as in hmmcu_estep
+ *   sum_logp, logp_utt   the Viterbi scores; n_utt as hmmcu_estep.
+ * An utterance with no path to the final state (T < N with a left-to-right A) scores -inf and adds no occupancy or
+ * counts, as it does in hmmcu_estep.  path[F] (may be NULL) receives the alignment, frame-aligned with the features
+ * (-1 on the frames of masked utterances): forced alignment as a by-product.  The statistics stay on the device
+ * (hmmcu_stats_device), so the all-reduce and hmmcu_mstep apply unchanged.  Linked (multi-stream) contexts are refused
+ * with HMMCU_EINVAL. */
+int hmmcu_estep_viterbi(hmmcu_ctx *ctx, const int32_t *utt2model, double *stats, double *logp_utt, int32_t *path);
+
 /* Device-side statistics for multi-GPU training: after hmmcu_estep(ctx, u2m, NULL, NULL) the
  * caller all-reduces the buffer in place on hmmcu_stream() (one ncclAllReduce(sum, double) per EM
  * iteration) and then downloads it. */
@@ -210,7 +225,7 @@ int hmmcu_viterbi_scores(hmmcu_ctx *ctx, double *score);
 /* Number of kernels this library has launched on ctx since creation (bench.py's gpu_launches). */
 int64_t hmmcu_launch_count(const hmmcu_ctx *ctx);
 /* Device time in ms of the most recent call's kernels, by name (CUDA events on the context's
- * stream).  names: "emis", "fwdbwd", "accum", "mstep", "score", "viterbi", "logb64", "pack", "init".  -1 if unknown.
+ * stream).  names: "emis", "fwdbwd", "align" (the alignment of hmmcu_estep_viterbi), "accum", "mstep", "score", "viterbi", "logb64", "pack", "init".  -1 if unknown.
  * Pseudo-names report state instead of time:
  *   "kappa"           accuracy-guard value of the current model pack
  *   "tc_active"       1 if the last emission launch ran on tensor cores
@@ -324,6 +339,12 @@ typedef int (*hmmh_allreduce_fn)(void *user, double *dev_buf, int64_t n_doubles,
 int hmmh_train(hmmcu_ctx *ctx, hmmh_model *models, int V, const int32_t *utt2model, int U,
                double *mean_logp, int *iterations, int max_iter, hmmh_allreduce_fn allreduce,
                void *user);
+
+/* The same loop with hmmcu_estep_viterbi as its E-step: Viterbi training, e.g. to refine initial models before
+ * hmmh_train (a few iterations with max_iter = k, then hmmh_train from the result).  One feature stream. */
+int hmmh_train_viterbi(hmmcu_ctx *ctx, hmmh_model *models, int V, const int32_t *utt2model, int U,
+                       double *mean_logp, int *iterations, int max_iter, hmmh_allreduce_fn allreduce,
+                       void *user);
 
 /* The same loop for models of P feature streams: ctxs[p] holds the features of stream p, models[p * V + v] is stream p
  * of word v; ctxs[1..P-1] are linked to ctxs[0] for the duration of the call (hmmcu_link_streams). */

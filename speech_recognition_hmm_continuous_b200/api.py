@@ -19,10 +19,10 @@ _lp = C.POINTER(C.c_int64)
 EXPORTS = [
     "hmmcu_create", "hmmcu_destroy", "hmmcu_last_error", "hmmcu_device_count", "hmmcu_stream", "hmmcu_synchronize",
     "hmmcu_host_alloc", "hmmcu_host_free", "hmmcu_set_option", "hmmcu_set_features", "hmmcu_set_features_device", "hmmcu_set_models",
-    "hmmcu_init_models", "hmmcu_emissions", "hmmcu_forward_scores", "hmmcu_rank", "hmmcu_stats_size", "hmmcu_estep", "hmmcu_stats_device",
+    "hmmcu_init_models", "hmmcu_emissions", "hmmcu_forward_scores", "hmmcu_rank", "hmmcu_stats_size", "hmmcu_estep", "hmmcu_estep_viterbi", "hmmcu_stats_device",
     "hmmcu_stats_download", "hmmcu_em_reset", "hmmcu_mstep", "hmmcu_get_models", "hmmcu_viterbi", "hmmcu_viterbi_scores", "hmmcu_launch_count", "hmmcu_last_kernel_ms",
     "hmmcu_enable_timing", "hmmh_model_alloc", "hmmh_model_free", "hmmh_read_features", "hmmh_write_features",
-    "hmmh_read_model", "hmmh_write_model", "hmmh_init_model", "hmmh_mstep", "hmmh_upload_models", "hmmh_train",
+    "hmmh_read_model", "hmmh_write_model", "hmmh_init_model", "hmmh_mstep", "hmmh_upload_models", "hmmh_train", "hmmh_train_viterbi",
     "hmmh_train_main", "hmmh_test_main",
     "hmmcu_features_begin", "hmmcu_features_append", "hmmcu_features_wait", "hmmcu_features_end", "hmmcu_staging", "hmmcu_link_streams", "hmmh_read_model_streams", "hmmh_write_model_streams", "hmmh_train_streams",
     "hmmh_model_set_alloc", "hmmh_model_set_free", "hmmh_read_model_set", "hmmh_write_model_set", "hmmh_upload_model_set",
@@ -107,6 +107,7 @@ def load():
     lib.hmmcu_viterbi_scores.argtypes = [C.c_void_p, _dp]
     lib.hmmcu_rank.argtypes = [C.c_void_p, _dp, C.c_int, C.c_int, C.c_double, _ip, _ip]
     lib.hmmcu_estep.argtypes = [C.c_void_p, _ip, _dp, _dp]
+    lib.hmmcu_estep_viterbi.argtypes = [C.c_void_p, _ip, _dp, _dp, _ip]
     lib.hmmcu_stats_download.argtypes = [C.c_void_p, _dp]
     lib.hmmcu_em_reset.argtypes = [C.c_void_p]
     lib.hmmcu_mstep.argtypes = [C.c_void_p, C.c_double, _dp, _dp, _ip]
@@ -137,8 +138,9 @@ def load():
                                 C.POINTER(IngestStats)]
     lib.hmmh_mstep.argtypes = [C.POINTER(_CModel), _dp]
     lib.hmmh_upload_models.argtypes = [C.c_void_p, C.POINTER(_CModel), C.c_int]
-    lib.hmmh_train.argtypes = [C.c_void_p, C.POINTER(_CModel), C.c_int, _ip, C.c_int, _dp, C.POINTER(C.c_int), C.c_int,
-                               C.c_void_p, C.c_void_p]
+    for f in ("hmmh_train", "hmmh_train_viterbi"):
+        getattr(lib, f).argtypes = [C.c_void_p, C.POINTER(_CModel), C.c_int, _ip, C.c_int, _dp, C.POINTER(C.c_int), C.c_int,
+                                    C.c_void_p, C.c_void_p]
     lib.hmmcu_peer_export.argtypes = [C.c_void_p, C.c_int, C.c_void_p]
     lib.hmmcu_peer_import.argtypes = [C.c_void_p, C.c_int, C.c_int, C.c_char_p]
     lib.hmmcu_peer_area.restype = C.c_void_p
@@ -340,6 +342,18 @@ class Context:
                                       _d(lpu) if want_logp else None), "hmmcu_estep")
         return stats, lpu
 
+    def estep_viterbi(self, utt2model, download=True, want_logp=True, want_path=False):
+        """hmmcu_estep_viterbi: the E-step of Viterbi training -> (stats, Viterbi score per utterance, path[F] or None)."""
+        u2m = np.ascontiguousarray(utt2model, dtype=np.int32)
+        ss = stats_size(self.N, self.M, self.D)
+        stats = np.zeros((self.V, ss)) if download else None
+        lpu = np.zeros(self.U) if want_logp else None
+        path = np.zeros(self.F, dtype=np.int32) if want_path else None
+        self._ck(self.lib.hmmcu_estep_viterbi(self.h, u2m.ctypes.data_as(_ip), _d(stats) if download else None,
+                                              _d(lpu) if want_logp else None,
+                                              path.ctypes.data_as(_ip) if want_path else None), "hmmcu_estep_viterbi")
+        return stats, lpu, path
+
     def stats_device(self):
         n = C.c_int64(0)
         p = self.lib.hmmcu_stats_device(self.h, C.byref(n))
@@ -377,6 +391,13 @@ class Context:
     def train(self, ms, utt2model, max_iter=0, allreduce=None):
         """hmmh_train: the reference's EM loop for all V words at once (in place on `ms`).
         allreduce(dev_ptr, n_doubles, stream_ptr) -> None sums the device buffer across ranks."""
+        return self._train(self.lib.hmmh_train, "hmmh_train", ms, utt2model, max_iter, allreduce)
+
+    def train_viterbi(self, ms, utt2model, max_iter=0, allreduce=None):
+        """hmmh_train_viterbi: the same loop with the Viterbi E-step (estep_viterbi), in place on `ms`."""
+        return self._train(self.lib.hmmh_train_viterbi, "hmmh_train_viterbi", ms, utt2model, max_iter, allreduce)
+
+    def _train(self, fn, what, ms, utt2model, max_iter, allreduce):
         u2m = np.ascontiguousarray(utt2model, dtype=np.int32)
         cm = ms._cmodels()
         mean = np.zeros(ms.V)
@@ -388,9 +409,8 @@ class Context:
                 return 0
             cb = ALLREDUCE_FN(_cb)
         self.V, self.N, self.M = ms.V, ms.N, ms.M
-        self._ck(self.lib.hmmh_train(self.h, cm, ms.V, u2m.ctypes.data_as(_ip), len(u2m), _d(mean),
-                                     its.ctypes.data_as(C.POINTER(C.c_int)), int(max_iter),
-                                     C.cast(cb, C.c_void_p) if cb else None, None), "hmmh_train")
+        self._ck(fn(self.h, cm, ms.V, u2m.ctypes.data_as(_ip), len(u2m), _d(mean), its.ctypes.data_as(C.POINTER(C.c_int)),
+                    int(max_iter), C.cast(cb, C.c_void_p) if cb else None, None), what)
         return its, mean
 
     # ---- statistics summed over the ranks through peer memory (NVLink), no library collective ----

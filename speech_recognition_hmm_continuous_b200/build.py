@@ -19,7 +19,7 @@ BIN = os.path.join(PKG, "bin")
 
 NVCC_FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo", "-O3", "-std=c++17",
               "-Xcompiler", "-fPIC", "-I", INC, "-I", CSRC]
-HOST_C = ["hmm_host.c", "ingest.c", "modelset.c", "train_main.c", "test_main.c"]
+HOST_C = ["hmm_host.c", "train_viterbi.c", "ingest.c", "modelset.c", "train_main.c", "test_main.c"]
 
 
 def _newer(target, sources):

@@ -22,6 +22,7 @@
 #include "dec_kernels.cuh"
 #include "acch_kernels.cuh"
 #include "vit_kernels.cuh"
+#include "vtrain_kernels.cuh"
 #include "init_kernels.cuh"
 
 using namespace hmmk;
@@ -106,7 +107,7 @@ struct hmmcu_ctx {
   bool timing = false;
   int use_graph = 1;          // replay the E-step / M-step launch sequences as CUDA graphs ("graphs" option)
   uint64_t cfg_epoch = 0;     // bumped by everything that changes what those sequences launch
-  GraphSlot g_estep, g_mstep;
+  GraphSlot g_estep, g_estep_vit, g_mstep;  // g_estep_vit: the E-step with the Viterbi alignment (hmmcu_estep_viterbi)
   int train_path = 0;         // emission / accumulate path of the last E-step: 0 CUDA cores, 1 k_emis_tc, 2 warp-specialised
   std::map<std::string, Timer> timers;
 
@@ -416,6 +417,7 @@ void hmmcu_destroy(hmmcu_ctx *ctx) {
     for (auto &pr : kv.second.pairs) { cudaEventDestroy(pr.first); cudaEventDestroy(pr.second); }
   }
   if (ctx->g_estep.exec) cudaGraphExecDestroy(ctx->g_estep.exec);
+  if (ctx->g_estep_vit.exec) cudaGraphExecDestroy(ctx->g_estep_vit.exec);
   if (ctx->g_mstep.exec) cudaGraphExecDestroy(ctx->g_mstep.exec);
   if (ctx->ctl_h) cudaFreeHost(ctx->ctl_h);
   if (ctx->ctr_h) cudaFreeHost(ctx->ctr_h);
@@ -1868,8 +1870,10 @@ static int launch_pack_x16(hmmcu_ctx *ctx, cudaStream_t st) {
 
 // phases: 1 = clear the statistics + emissions, 2 = forward-backward, 4 = mixture accumulators.  fb_logb / acc_gamma
 // replace the context's own log-emissions in the recursions / its own state posteriors in the accumulators
-// (multi-stream models); with all phases and no replacement this is the plain single-stream E-step.
-static int estep_core(hmmcu_ctx *ctx, const int32_t *utt2model, int phases, const float *fb_logb, const float *acc_gamma) {
+// (multi-stream models); with all phases and no replacement this is the plain single-stream E-step.  align: phase 2 is
+// the Viterbi alignment (k_vtrain) instead of forward-backward; it writes the same gamma and statistics, and its path.
+static int estep_core(hmmcu_ctx *ctx, const int32_t *utt2model, int phases, const float *fb_logb, const float *acc_gamma,
+                      bool align = false) {
   CK(cudaSetDevice(ctx->dev));
   int rc = ensure_packed(ctx);
   if (rc) return rc;
@@ -1893,7 +1897,10 @@ static int estep_core(hmmcu_ctx *ctx, const int32_t *utt2model, int phases, cons
     CK(ctx->logb.ensure(sizeof(float) * F * N));
     if (!use_tc) CK(ctx->post.ensure(sizeof(float) * F * G));
     CK(ctx->gamma.ensure(sizeof(float) * F * N));
-    if (!res_fb_on(ctx)) {  // k_fb_res keeps alpha / beta on the SM
+    if (align) {
+      CK(ctx->psi_ws.ensure(sizeof(unsigned long long) * F));
+      CK(ctx->path_d.ensure(sizeof(int32_t) * F));
+    } else if (!res_fb_on(ctx)) {  // k_fb_res keeps alpha / beta on the SM
       CK(ctx->alpha_ws.ensure(sizeof(uint32_t) * F * kFbRow));
       CK(ctx->beta_ws.ensure(sizeof(uint32_t) * F * kFbRow));
     }
@@ -1921,7 +1928,7 @@ static int estep_core(hmmcu_ctx *ctx, const int32_t *utt2model, int phases, cons
     if (U == 0) return HMMCU_OK;
     // masked utterances report 0 (k_fb_res writes the live ones only); cleared here, so that no memset node sits between the
     // emission kernel and k_fb_res
-    if ((phases & 2) && res_fb && ctx->n_live < U) CK(cudaMemsetAsync(ctx->logp_utt_d.p, 0, sizeof(double) * U, ctx->st));
+    if ((phases & 2) && res_fb && !align && ctx->n_live < U) CK(cudaMemsetAsync(ctx->logp_utt_d.p, 0, sizeof(double) * U, ctx->st));
     int rc2;
     bool fb_forked = false;
     const bool pack_forked = pack16 && !ctx->timing && (phases & 3) && ctx->mstep_fork;
@@ -1942,9 +1949,27 @@ static int estep_core(hmmcu_ctx *ctx, const int32_t *utt2model, int phases, cons
     }
     // 2. forward / backward, gamma, transition statistics, log-probabilities
     if (phases & 2) {
-    t_begin(ctx, "fwdbwd");
+    const char *tname = align ? "align" : "fwdbwd";
+    t_begin(ctx, tname);
     {
-        if (res_fb) {
+        if (align) {
+        // the Viterbi alignment: per-utterance rows for k_fb_reduce below, or atomics into the statistics (vtrain_kernels.cuh)
+        const int blocks = (U + kVtUtts - 1) / kVtUtts;
+        const size_t vsm = vtrain_smem_bytes(N);
+        double *rows = res_fb ? ctx->ustats.as<double>() : nullptr;
+        if (ctx->banded) {
+          DISPATCH_N(N, (k_vtrain<NS, true><<<blocks, kVtThreads, vsm, ctx->st>>>(
+                            lb_fb, ctx->off_d.as<int64_t>(), ctx->u2m_d.as<int32_t>(), ctx->A.as<double>(), U,
+                            ctx->psi_ws.as<unsigned long long>(), ctx->path_d.as<int32_t>(), ctx->gamma.as<float>(),
+                            ctx->res_upos.as<int32_t>(), rows, ctx->stats.as<double>(), ss, off_lp, ctx->logp_utt_d.as<double>())));
+        } else {
+          DISPATCH_N(N, (k_vtrain<NS, false><<<blocks, kVtThreads, vsm, ctx->st>>>(
+                            lb_fb, ctx->off_d.as<int64_t>(), ctx->u2m_d.as<int32_t>(), ctx->A.as<double>(), U,
+                            ctx->psi_ws.as<unsigned long long>(), ctx->path_d.as<int32_t>(), ctx->gamma.as<float>(),
+                            ctx->res_upos.as<int32_t>(), nullptr, ctx->stats.as<double>(), ss, off_lp, ctx->logp_utt_d.as<double>())));
+        }
+        LAUNCH_CHECK();
+        } else if (res_fb) {
         // every utterance resident in shared memory: log-emissions read once, gamma written once (fbres_kernels.cuh)
         const int grid = res_grid(ctx);
         DISPATCH_N(N, CK(cudaFuncSetAttribute(k_fb_res<NS>, cudaFuncAttributeMaxDynamicSharedMemorySize, kResSmemBytes));
@@ -1953,6 +1978,8 @@ static int estep_core(hmmcu_ctx *ctx, const int32_t *utt2model, int phases, cons
                                  ctx->res_batches.as<ResBatch>(), (int)ctx->n_res_batches, ctx->res_counter.as<int>(),
                                  ctx->gamma.as<float>(), ctx->ustats.as<double>(), ctx->logp_utt_d.as<double>())));
         LAUNCH_CHECK();
+        }
+        if (res_fb) {
         // the per-model sums of the transition statistics feed nothing before the M-step: beside the accumulate kernel
         fb_forked = !ctx->timing && (phases & 4) && ctx->mstep_fork;
         if (fb_forked) {
@@ -1963,7 +1990,7 @@ static int estep_core(hmmcu_ctx *ctx, const int32_t *utt2model, int phases, cons
                                                                         off_lp);
         LAUNCH_CHECK();
         if (fb_forked) CK(cudaEventRecord(ctx->ev_join[0], ctx->st_aux[0]));
-      } else {
+      } else if (!align) {
       const int blocks = (U + kFbUtts - 1) / kFbUtts;
       const size_t fsm = fb_smem_bytes(N);
       if (ctx->banded) {
@@ -1980,7 +2007,7 @@ static int estep_core(hmmcu_ctx *ctx, const int32_t *utt2model, int phases, cons
       LAUNCH_CHECK();
       }
     }
-    t_end(ctx, "fwdbwd");
+    t_end(ctx, tname);
     }
     // 3. mixture accumulators
     if (!(phases & 4)) {
@@ -2062,13 +2089,23 @@ static int estep_core(hmmcu_ctx *ctx, const int32_t *utt2model, int phases, cons
     if (fb_forked) CK(cudaStreamWaitEvent(ctx->st, ctx->ev_join[0], 0));
     return HMMCU_OK;
   };
-  const uint64_t key = 1u | ((ctx->use_res_fb && ctx->banded && ctx->res_fits) ? (1u << 8) : 0u) | (use_tc ? 2u : 0u) | (ws_emis ? 4u : 0u) | (ws_acc ? 8u : 0u) | (h_acc ? 32u : 0u) | (pack16 ? 64u : 0u) | (ctx->banded ? 16u : 0u);
+  const uint64_t key = 1u | ((ctx->use_res_fb && ctx->banded && ctx->res_fits) ? (1u << 8) : 0u) | (use_tc ? 2u : 0u) | (ws_emis ? 4u : 0u) | (ws_acc ? 8u : 0u) | (h_acc ? 32u : 0u) | (pack16 ? 64u : 0u) | (ctx->banded ? 16u : 0u) | (align ? (1u << 9) : 0u);
   ctx->last_tc = use_tc;
   if (phases & 4) ctx->last_acc_h = h_acc;
   // (pieces of a multi-stream E-step: plain launches)
-  const int rcq = (phases != 7 || fb_logb || acc_gamma) ? enqueue() : run_graphed(ctx, ctx->g_estep, key, enqueue);
+  const int rcq = (phases != 7 || fb_logb || acc_gamma) ? enqueue() : run_graphed(ctx, align ? ctx->g_estep_vit : ctx->g_estep, key, enqueue);
   if (rcq == HMMCU_OK && pack16) { ctx->x16_x = ctx->x_version; ctx->x16_map = ctx->map_version; }
   return rcq;
+}
+
+// the host copies of an E-step's results (each may be NULL); path[F] is written by the Viterbi alignment only
+static int estep_download(hmmcu_ctx *ctx, double *stats, double *logp_utt, int32_t *path) {
+  const int U = ctx->U;
+  if (logp_utt && U > 0) CK(cudaMemcpyAsync(logp_utt, ctx->logp_utt_d.p, sizeof(double) * U, cudaMemcpyDeviceToHost, ctx->st));
+  if (stats) CK(cudaMemcpyAsync(stats, ctx->stats.p, sizeof(double) * ctx->stats_n, cudaMemcpyDeviceToHost, ctx->st));
+  if (path && U > 0 && ctx->F > 0) CK(cudaMemcpyAsync(path, ctx->path_d.p, sizeof(int32_t) * ctx->F, cudaMemcpyDeviceToHost, ctx->st));
+  if (stats || logp_utt || path) CK(cudaStreamSynchronize(ctx->st));
+  return HMMCU_OK;
 }
 
 int hmmcu_estep(hmmcu_ctx *ctx, const int32_t *utt2model, double *stats, double *logp_utt) {
@@ -2103,10 +2140,16 @@ int hmmcu_estep(hmmcu_ctx *ctx, const int32_t *utt2model, double *stats, double 
       LAUNCH_CHECK();
     }
   }
-  if (logp_utt && U > 0) CK(cudaMemcpyAsync(logp_utt, ctx->logp_utt_d.p, sizeof(double) * U, cudaMemcpyDeviceToHost, ctx->st));
-  if (stats) CK(cudaMemcpyAsync(stats, ctx->stats.p, sizeof(double) * ctx->stats_n, cudaMemcpyDeviceToHost, ctx->st));
-  if (stats || logp_utt) CK(cudaStreamSynchronize(ctx->st));
-  return HMMCU_OK;
+  return estep_download(ctx, stats, logp_utt, nullptr);
+}
+
+int hmmcu_estep_viterbi(hmmcu_ctx *ctx, const int32_t *utt2model, double *stats, double *logp_utt, int32_t *path) {
+  if (!ctx) return HMMCU_EINVAL;
+  if (ctx->primary) return fail(ctx, HMMCU_EINVAL, "estep_viterbi: this context is a linked stream; call its primary");
+  if (!ctx->linked.empty()) return fail(ctx, HMMCU_EINVAL, "estep_viterbi: Viterbi training of multi-stream (linked) models is not supported");
+  const int rc = estep_core(ctx, utt2model, 7, nullptr, nullptr, true);
+  if (rc != HMMCU_OK) return rc;
+  return estep_download(ctx, stats, logp_utt, path);
 }
 
 // ------------------------------------------------------------------------- device-resident EM ----

@@ -12,6 +12,7 @@
 #include <string.h>
 
 #include "hmm_cuda.h"
+#include "em_loop.h"
 
 #define HM_THRESHOLD 1.0e-3 /* T-FS:37 */
 #define HM_DELTA 1          /* T-FS:38 */
@@ -413,9 +414,10 @@ int hmmh_upload_models(hmmcu_ctx *ctx, const hmmh_model *models, int V) { return
 
 /* T-FS:238-361 for V words at once and P feature streams (models[p * V + v] = stream p of word v; ctxs[p] holds
  * stream p's features; ctxs[1..] are linked to ctxs[0] here).  Every word keeps the reference's own stopping rule; a
- * word that has converged drops out of the following E-steps (its utterances are masked with -1). */
-int hmmh_train_streams(hmmcu_ctx *const *ctxs, int P, hmmh_model *models, int V, const int32_t *utt2model, int U, double *mean_logp,
-                       int *iterations, int max_iter, hmmh_allreduce_fn allreduce, void *user) {
+ * word that has converged drops out of the following E-steps (its utterances are masked with -1).  estep(ctx, map)
+ * leaves the statistics of the current models on the device: Baum-Welch (hmmh_train*) or Viterbi (hmmh_train_viterbi). */
+int hmmh_em_loop(hmmcu_ctx *const *ctxs, int P, hmmh_model *models, int V, const int32_t *utt2model, int U, double *mean_logp,
+                 int *iterations, int max_iter, hmmh_allreduce_fn allreduce, void *user, hmmh_estep_fn estep) {
   if (!ctxs || P < 1 || P > HMMH_MAX_STREAMS || !models || V < 1 || (U > 0 && !utt2model)) return HMMCU_EINVAL;
   hmmcu_ctx *ctx = ctxs[0];
   double *probab = (double *)malloc(sizeof(double) * V), *nutt = (double *)malloc(sizeof(double) * V);
@@ -442,7 +444,7 @@ int hmmh_train_streams(hmmcu_ctx *const *ctxs, int P, hmmh_model *models, int V,
       for (int u = 0; u < U; u++) map[u] = active[utt2model[u]] ? utt2model[u] : -1;
       remap = 0;
     }
-    if ((rc = hmmcu_estep(ctx, map, NULL, NULL)) != HMMCU_OK) break;
+    if ((rc = estep(ctx, map)) != HMMCU_OK) break;
     for (int p = 0; allreduce && p < P && rc == HMMCU_OK; p++) {
       int64_t n = 0;
       double *dev = hmmcu_stats_device(ctxs[p], &n);
@@ -481,6 +483,13 @@ int hmmh_train_streams(hmmcu_ctx *const *ctxs, int P, hmmh_model *models, int V,
   if (P > 1) hmmcu_link_streams(ctx, NULL, 0);
   free(probab); free(nutt); free(probab_q); free(nutt_q); free(updated); free(updated_q); free(active); free(map);
   return rc;
+}
+
+static int estep_baum_welch(hmmcu_ctx *ctx, const int32_t *map) { return hmmcu_estep(ctx, map, NULL, NULL); }
+
+int hmmh_train_streams(hmmcu_ctx *const *ctxs, int P, hmmh_model *models, int V, const int32_t *utt2model, int U, double *mean_logp,
+                       int *iterations, int max_iter, hmmh_allreduce_fn allreduce, void *user) {
+  return hmmh_em_loop(ctxs, P, models, V, utt2model, U, mean_logp, iterations, max_iter, allreduce, user, estep_baum_welch);
 }
 
 int hmmh_train(hmmcu_ctx *ctx, hmmh_model *models, int V, const int32_t *utt2model, int U, double *mean_logp,
