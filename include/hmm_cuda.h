@@ -168,6 +168,42 @@ int hmmcu_estep(hmmcu_ctx *ctx, const int32_t *utt2model, double *stats, double 
  * with HMMCU_EINVAL. */
 int hmmcu_estep_viterbi(hmmcu_ctx *ctx, const int32_t *utt2model, double *stats, double *logp_utt, int32_t *path);
 
+/* The E-step of maximum mutual information (MMI) training.  label[U] is the word of every utterance (-1 leaves it out),
+ * kappa > 0 the acoustic scale, 1 <= max_hyp <= HMMCU_MMI_MAX_HYP.  Every (utterance, word) cell is scored as
+ * hmmcu_forward_scores(ctx, ., 0) scores it (on the device, not copied back), and
+ *   P(w | u) = exp(kappa S[u][w] - logsumexp_w' kappa S[u][w'])    (double)
+ * The hypotheses of u are its label, always, with the label's posterior however small, then at most max_hyp - 1 other
+ * words in descending posterior order (lower word index first on a tie) with P >= HMMCU_MMI_MIN_POST.  The statistics
+ * (hmmcu_stats_device, and stats if not NULL) are then [2][V][hmmcu_stats_size]:
+ *   block 0, numerator     hmmcu_estep(ctx, label, ..)'s statistics, bit for bit (sum_logp and n_utt included)
+ *   block 1, denominator   sum over u and its hypotheses h of P(h | u) times the E-step statistics of u against model h
+ *                          (raw posteriors: the pruned mass is not renormalised); its tail holds the objective:
+ *                          sum_logp[v] = sum over the included utterances of word v of -log P(label | u) (a fixed order,
+ *                          bit-reproducible), n_utt[v] = their number.  The MMI objective is F = -sum_v sum_logp[v].
+ * An utterance whose label score is not finite (T < N with a left-to-right A) is left out of block 1.  One all-reduce of
+ * the whole buffer sums both blocks and the objective over the ranks.  hmmcu_mstep and hmmcu_peer_allreduce refuse
+ * this buffer (its size is not theirs); hmmcu_mstep_ebw takes it.  Linked (multi-stream) contexts are refused with
+ * HMMCU_EINVAL.  hmmcu_last_kernel_ms: "mmi_score", "mmi_post", "mmi_num", "mmi_den" time the stages, "mmi_rounds" is
+ * the number of denominator rounds (round 0: the labels; round r: every utterance's r-th other hypothesis). */
+#define HMMCU_MMI_MIN_POST 1.0e-5 /* posterior floor of a competing hypothesis */
+#define HMMCU_MMI_MAX_HYP 16      /* hypotheses per utterance, the label included */
+int hmmcu_estep_mmi(hmmcu_ctx *ctx, const int32_t *label, double kappa, int max_hyp, double *stats);
+
+/* The extended Baum-Welch update of the means and variances from hmmcu_estep_mmi's statistics, per Gaussian and
+ * dimension (hmmh_mstep_ebw is the same update on the host, operation for operation):
+ *   Q = S2c + 2 mu S1 - mu^2 S0 (= sum gamma x^2); with S0_num > 0 the numerator's (S0, S1, Q) are scaled by
+ *   1 + tau / S0_num (I-smoothing); dg, ds, dq = numerator - denominator of S0, S1, Q;
+ *   D_min = the largest real root over the dimensions of var D^2 + (dq + dg (var + mu^2) - 2 mu ds) D + (dq dg - ds^2)
+ *   (0 when none is positive); D = max(2 D_min, E S0_den);
+ *   mu' = (ds + D mu) / (dg + D),  var' = (dq + D (var + mu^2)) / (dg + D) - mu'^2 floored at 1e-5 (T-FS:39),
+ *   inv_var and det as hmmh_mstep forms them.
+ * A Gaussian with dg + D <= 0 (no occupancy in either block) is left as it is.  Mixture weights and transitions are not
+ * updated, and there is no stopping rule.  With den = 0 and tau = 0 this is the textbook ML update, whose variance is
+ * about the NEW mean (hmmh_mstep keeps the reference's variance about the old mean).  E > 1, tau >= 0.  The accuracy
+ * guard and the model images are refreshed as after hmmcu_mstep; hmmcu_em_reset's state is not touched.  Refused with
+ * HMMCU_EINVAL unless the statistics are an MMI buffer of the current model set. */
+int hmmcu_mstep_ebw(hmmcu_ctx *ctx, double E, double tau);
+
 /* Device-side statistics for multi-GPU training: after hmmcu_estep(ctx, u2m, NULL, NULL) the
  * caller all-reduces the buffer in place on hmmcu_stream() (one ncclAllReduce(sum, double) per EM
  * iteration) and then downloads it. */
@@ -324,6 +360,9 @@ int hmmh_upload_model_set(hmmcu_ctx *ctx, const hmmh_model_set *s);
 int hmmh_init_model(hmmh_model *m, const double *x, const int64_t *frame_off, int U);
 /* M-step from one model's statistics vector (T-FS:328-346, 1862-1955, 1338-1359). */
 int hmmh_mstep(hmmh_model *m, const double *stats);
+/* The extended Baum-Welch update of hmmcu_mstep_ebw on the host, from one model's numerator and denominator statistics
+ * vectors (blocks 0 and 1 of hmmcu_estep_mmi's buffer); means, inverse variances and determinants in place. */
+int hmmh_mstep_ebw(hmmh_model *m, const double *num, const double *den, double E, double tau);
 
 /* hmmcu_set_models from an array of V host models of identical topology. */
 int hmmh_upload_models(hmmcu_ctx *ctx, const hmmh_model *models, int V);
@@ -345,6 +384,14 @@ int hmmh_train(hmmcu_ctx *ctx, hmmh_model *models, int V, const int32_t *utt2mod
 int hmmh_train_viterbi(hmmcu_ctx *ctx, hmmh_model *models, int V, const int32_t *utt2model, int U,
                        double *mean_logp, int *iterations, int max_iter, hmmh_allreduce_fn allreduce,
                        void *user);
+
+/* MMI training of V words from their current models (e.g. Baum-Welch trained): upload, then per iteration
+ * hmmcu_estep_mmi(label, kappa, max_hyp), the hook on the whole [2][V][stats_size] buffer, objective[k] = F / n_utt of
+ * the models entering iteration k (F = -sum_v den.sum_logp[v], n_utt = sum_v den.n_utt[v], after the all-reduce), and
+ * hmmcu_mstep_ebw(E, tau); the models are downloaded at the end.  A fixed number of iterations, no stopping rule.
+ * objective[iterations] may be NULL.  One feature stream. */
+int hmmh_train_mmi(hmmcu_ctx *ctx, hmmh_model *models, int V, const int32_t *label, int U, double kappa, int max_hyp,
+                   double E, double tau, int iterations, double *objective, hmmh_allreduce_fn allreduce, void *user);
 
 /* The same loop for models of P feature streams: ctxs[p] holds the features of stream p, models[p * V + v] is stream p
  * of word v; ctxs[1..P-1] are linked to ctxs[0] for the duration of the call (hmmcu_link_streams). */

@@ -19,10 +19,10 @@ _lp = C.POINTER(C.c_int64)
 EXPORTS = [
     "hmmcu_create", "hmmcu_destroy", "hmmcu_last_error", "hmmcu_device_count", "hmmcu_stream", "hmmcu_synchronize",
     "hmmcu_host_alloc", "hmmcu_host_free", "hmmcu_set_option", "hmmcu_set_features", "hmmcu_set_features_device", "hmmcu_set_models",
-    "hmmcu_init_models", "hmmcu_emissions", "hmmcu_forward_scores", "hmmcu_rank", "hmmcu_stats_size", "hmmcu_estep", "hmmcu_estep_viterbi", "hmmcu_stats_device",
-    "hmmcu_stats_download", "hmmcu_em_reset", "hmmcu_mstep", "hmmcu_get_models", "hmmcu_viterbi", "hmmcu_viterbi_scores", "hmmcu_launch_count", "hmmcu_last_kernel_ms",
+    "hmmcu_init_models", "hmmcu_emissions", "hmmcu_forward_scores", "hmmcu_rank", "hmmcu_stats_size", "hmmcu_estep", "hmmcu_estep_viterbi", "hmmcu_estep_mmi", "hmmcu_stats_device",
+    "hmmcu_stats_download", "hmmcu_em_reset", "hmmcu_mstep", "hmmcu_mstep_ebw", "hmmcu_get_models", "hmmcu_viterbi", "hmmcu_viterbi_scores", "hmmcu_launch_count", "hmmcu_last_kernel_ms",
     "hmmcu_enable_timing", "hmmh_model_alloc", "hmmh_model_free", "hmmh_read_features", "hmmh_write_features",
-    "hmmh_read_model", "hmmh_write_model", "hmmh_init_model", "hmmh_mstep", "hmmh_upload_models", "hmmh_train", "hmmh_train_viterbi",
+    "hmmh_read_model", "hmmh_write_model", "hmmh_init_model", "hmmh_mstep", "hmmh_mstep_ebw", "hmmh_upload_models", "hmmh_train", "hmmh_train_viterbi", "hmmh_train_mmi",
     "hmmh_train_main", "hmmh_test_main",
     "hmmcu_features_begin", "hmmcu_features_append", "hmmcu_features_wait", "hmmcu_features_end", "hmmcu_staging", "hmmcu_link_streams", "hmmh_read_model_streams", "hmmh_write_model_streams", "hmmh_train_streams",
     "hmmh_model_set_alloc", "hmmh_model_set_free", "hmmh_read_model_set", "hmmh_write_model_set", "hmmh_upload_model_set",
@@ -108,6 +108,8 @@ def load():
     lib.hmmcu_rank.argtypes = [C.c_void_p, _dp, C.c_int, C.c_int, C.c_double, _ip, _ip]
     lib.hmmcu_estep.argtypes = [C.c_void_p, _ip, _dp, _dp]
     lib.hmmcu_estep_viterbi.argtypes = [C.c_void_p, _ip, _dp, _dp, _ip]
+    lib.hmmcu_estep_mmi.argtypes = [C.c_void_p, _ip, C.c_double, C.c_int, _dp]
+    lib.hmmcu_mstep_ebw.argtypes = [C.c_void_p, C.c_double, C.c_double]
     lib.hmmcu_stats_download.argtypes = [C.c_void_p, _dp]
     lib.hmmcu_em_reset.argtypes = [C.c_void_p]
     lib.hmmcu_mstep.argtypes = [C.c_void_p, C.c_double, _dp, _dp, _ip]
@@ -137,6 +139,9 @@ def load():
     lib.hmmh_ingest.argtypes = [C.c_void_p, C.POINTER(C.c_char_p), C.c_int, C.c_int, _lp, C.POINTER(C.c_int), C.POINTER(C.c_int),
                                 C.POINTER(IngestStats)]
     lib.hmmh_mstep.argtypes = [C.POINTER(_CModel), _dp]
+    lib.hmmh_mstep_ebw.argtypes = [C.POINTER(_CModel), _dp, _dp, C.c_double, C.c_double]
+    lib.hmmh_train_mmi.argtypes = [C.c_void_p, C.POINTER(_CModel), C.c_int, _ip, C.c_int, C.c_double, C.c_int, C.c_double, C.c_double,
+                                   C.c_int, _dp, C.c_void_p, C.c_void_p]
     lib.hmmh_upload_models.argtypes = [C.c_void_p, C.POINTER(_CModel), C.c_int]
     for f in ("hmmh_train", "hmmh_train_viterbi"):
         getattr(lib, f).argtypes = [C.c_void_p, C.POINTER(_CModel), C.c_int, _ip, C.c_int, _dp, C.POINTER(C.c_int), C.c_int,
@@ -204,6 +209,17 @@ class ModelSet:
             m.N, m.M, m.D = self.N, self.M, self.D
             m.A, m.c, m.mu, m.inv_var, m.det = _d(self.A[v]), _d(self.c[v]), _d(self.mu[v]), _d(self.iv[v]), _d(self.det[v])
         return arr
+
+
+def _allreduce_hook(allreduce):
+    """allreduce(dev_ptr, n_doubles, stream_ptr) -> None as an hmmh_allreduce_fn (None stays None)."""
+    if allreduce is None:
+        return None
+
+    def _cb(user, dev, n, stream):
+        allreduce(dev, n, stream)
+        return 0
+    return ALLREDUCE_FN(_cb)
 
 
 class Context:
@@ -354,14 +370,23 @@ class Context:
                                               path.ctypes.data_as(_ip) if want_path else None), "hmmcu_estep_viterbi")
         return stats, lpu, path
 
+    def estep_mmi(self, label, kappa, max_hyp, download=True):
+        """hmmcu_estep_mmi: the MMI E-step -> stats[2][V][stats_size] (numerator, denominator) or None."""
+        lab = np.ascontiguousarray(label, dtype=np.int32)
+        stats = np.zeros((2, self.V, stats_size(self.N, self.M, self.D))) if download else None
+        self._ck(self.lib.hmmcu_estep_mmi(self.h, lab.ctypes.data_as(_ip), float(kappa), int(max_hyp), _d(stats) if download else None),
+                 "hmmcu_estep_mmi")
+        return stats
+
     def stats_device(self):
         n = C.c_int64(0)
         p = self.lib.hmmcu_stats_device(self.h, C.byref(n))
         return p, n.value
 
     def stats_download(self):
+        """[V][stats_size], or [2][V][stats_size] after estep_mmi."""
         ss = stats_size(self.N, self.M, self.D)
-        stats = np.zeros((self.V, ss))
+        stats = np.zeros((self.V, ss)) if self.stats_device()[1] <= self.V * ss else np.zeros((2, self.V, ss))
         self._ck(self.lib.hmmcu_stats_download(self.h, _d(stats)), "hmmcu_stats_download")
         return stats
 
@@ -374,6 +399,10 @@ class Context:
         upd = np.zeros(self.V, dtype=np.int32)
         self._ck(self.lib.hmmcu_mstep(self.h, float(threshold), _d(lp), _d(nu), upd.ctypes.data_as(_ip)), "hmmcu_mstep")
         return lp, nu, upd
+
+    def mstep_ebw(self, E=2.0, tau=100.0):
+        """hmmcu_mstep_ebw: the extended Baum-Welch update of the means and variances on the device, after estep_mmi."""
+        self._ck(self.lib.hmmcu_mstep_ebw(self.h, float(E), float(tau)), "hmmcu_mstep_ebw")
 
     def get_models(self, D):
         ms = ModelSet(np.zeros((self.V, self.N, self.N)), np.zeros((self.V, self.N, self.M)), np.zeros((self.V, self.N, self.M, D)),
@@ -397,17 +426,25 @@ class Context:
         """hmmh_train_viterbi: the same loop with the Viterbi E-step (estep_viterbi), in place on `ms`."""
         return self._train(self.lib.hmmh_train_viterbi, "hmmh_train_viterbi", ms, utt2model, max_iter, allreduce)
 
+    def train_mmi(self, ms, label, kappa, max_hyp, E=2.0, tau=100.0, iterations=4, allreduce=None):
+        """hmmh_train_mmi: `iterations` MMI iterations (estep_mmi, the all-reduce, mstep_ebw) in place on `ms`
+        -> objective[iterations] (-log P(label | O) per utterance of the models entering each iteration)."""
+        lab = np.ascontiguousarray(label, dtype=np.int32)
+        cm = ms._cmodels()
+        obj = np.zeros(max(int(iterations), 1))
+        cb = _allreduce_hook(allreduce)
+        self.V, self.N, self.M = ms.V, ms.N, ms.M
+        self._ck(self.lib.hmmh_train_mmi(self.h, cm, ms.V, lab.ctypes.data_as(_ip), len(lab), float(kappa), int(max_hyp), float(E),
+                                         float(tau), int(iterations), _d(obj), C.cast(cb, C.c_void_p) if cb else None, None),
+                 "hmmh_train_mmi")
+        return obj[:int(iterations)]
+
     def _train(self, fn, what, ms, utt2model, max_iter, allreduce):
         u2m = np.ascontiguousarray(utt2model, dtype=np.int32)
         cm = ms._cmodels()
         mean = np.zeros(ms.V)
         its = np.zeros(ms.V, dtype=np.int32)
-        cb = None
-        if allreduce is not None:
-            def _cb(user, dev, n, stream):
-                allreduce(dev, n, stream)
-                return 0
-            cb = ALLREDUCE_FN(_cb)
+        cb = _allreduce_hook(allreduce)
         self.V, self.N, self.M = ms.V, ms.N, ms.M
         self._ck(fn(self.h, cm, ms.V, u2m.ctypes.data_as(_ip), len(u2m), _d(mean), its.ctypes.data_as(C.POINTER(C.c_int)),
                     int(max_iter), C.cast(cb, C.c_void_p) if cb else None, None), what)
@@ -465,6 +502,18 @@ def mstep(ms, stats):
         rc = lib.hmmh_mstep(C.byref(cm[v]), _d(stats[v]))
         if rc:
             raise HmmCudaError("hmmh_mstep failed (%d)" % rc)
+    return ms
+
+
+def mstep_ebw(ms, num, den, E=2.0, tau=100.0):
+    """hmmh_mstep_ebw on every model of the set, in place: num, den = blocks 0 and 1 ([V][stats_size]) of estep_mmi."""
+    lib = load()
+    num, den = _f64(num), _f64(den)
+    cm = ms._cmodels()
+    for v in range(ms.V):
+        rc = lib.hmmh_mstep_ebw(C.byref(cm[v]), _d(num[v]), _d(den[v]), float(E), float(tau))
+        if rc:
+            raise HmmCudaError("hmmh_mstep_ebw failed (%d)" % rc)
     return ms
 
 

@@ -93,12 +93,14 @@ __device__ __forceinline__ void store_row(uint32_t *__restrict__ p, const double
 // Outputs: gamma32[F][N] (the reference's alpha^ beta^ / c, T-FS:1709); per-model statistics head
 // (num_trans, den_trans, den_mix, sum_logp, n_utt) by double atomics, one set per utterance;
 // logp_utt[U] (0 for masked utterances).  alpha_ws / beta_ws: [F][kFbRow] workspaces of d32 words.
-template <int NS, bool BANDED>
+// WEIGHTED: utterance u's gamma rows and its transition and occupancy atomics are multiplied by w[u] (the denominator
+// of MMI training, hmmcu_estep_mmi); its log P is not.
+template <int NS, bool BANDED, bool WEIGHTED = false>
 __global__ void __launch_bounds__(kFbThreads)
 k_fb(const float *__restrict__ logb, const int64_t *__restrict__ off, const int32_t *__restrict__ u2m,
      const double *__restrict__ Aall, int U, uint32_t *__restrict__ alpha_ws, uint32_t *__restrict__ beta_ws,
      float *__restrict__ gamma, double *__restrict__ stats, int64_t stats_stride, int64_t off_sumlogp,
-     double *__restrict__ logp_utt) {
+     double *__restrict__ logp_utt, const double *__restrict__ w = nullptr) {
   extern __shared__ __align__(16) uint8_t fb_smem[];
   constexpr int US = kFbWin * NS + 2;  // per-utterance stride, padded: the 8 chain lanes hit 8 different banks
   double *bf = reinterpret_cast<double *>(fb_smem);  // [2 buffers][2 directions][kFbUtts][US]  b~
@@ -262,7 +264,8 @@ k_fb(const float *__restrict__ logb, const int64_t *__restrict__ off, const int3
     const int64_t base = off[u];
     const int T = (int)(off[u + 1] - base);
     const double *A = sA[uu];
-    const double phi = sphi[uu];
+    double phi = sphi[uu];
+    if constexpr (WEIGHTED) phi *= w[u];  // (enters sc and zs below)
     double acc_num[NS][2], acc_dt[NS], acc_dm[NS], acc_m = 0.0;
 #pragma unroll
     for (int i = 0; i < NS; i++) { acc_num[i][0] = acc_num[i][1] = 0.0; acc_dt[i] = 0.0; acc_dm[i] = 0.0; }

@@ -192,12 +192,14 @@ __device__ __forceinline__ void res_chain(int lane, int count, const int32_t *Ta
   }
 }
 
-template <int NS>
+// WEIGHTED: utterance u's gamma rows and the transition and occupancy sums of its ustats row are multiplied by w[u]
+// (the denominator of MMI training, hmmcu_estep_mmi); its log P is not.
+template <int NS, bool WEIGHTED = false>
 __global__ void __launch_bounds__(kResThreads, 1)
 k_fb_res(const float *__restrict__ logb, const int64_t *__restrict__ off, const int32_t *__restrict__ u2m,
          const double *__restrict__ Aall, const int32_t *__restrict__ order, const int32_t *__restrict__ upos,
          const ResBatch *__restrict__ batches, int nbatches, int *__restrict__ counter, float *__restrict__ gamma,
-         double *__restrict__ ustats, double *__restrict__ logp_utt) {
+         double *__restrict__ ustats, double *__restrict__ logp_utt, const double *__restrict__ w = nullptr) {
   extern __shared__ __align__(16) uint8_t res_smem[];
   const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
   const int team = warp >> 2, role = warp & 3, tt = role * 32 + lane;  // tt: thread index within the team
@@ -316,7 +318,8 @@ k_fb_res(const float *__restrict__ logb, const int64_t *__restrict__ off, const 
         a0[i] = A[i * NS + i];
         a1[i] = (i + 1 < NS) ? A[i * NS + i + 1] : 0.0;
       }
-      const double phi = S.phi[j];
+      double phi = S.phi[j];
+      if constexpr (WEIGHTED) phi *= w[S.utt[j]];  // (enters sc below)
       double acc_n0[NS], acc_n1[NS], acc_dt[NS], acc_dm[NS];
 #pragma unroll
       for (int i = 0; i < NS; i++) { acc_n0[i] = 0.0; acc_n1[i] = 0.0; acc_dt[i] = 0.0; acc_dm[i] = 0.0; }

@@ -23,6 +23,7 @@
 #include "acch_kernels.cuh"
 #include "vit_kernels.cuh"
 #include "vtrain_kernels.cuh"
+#include "mmi_kernels.cuh"
 #include "init_kernels.cuh"
 
 using namespace hmmk;
@@ -192,7 +193,11 @@ struct hmmcu_ctx {
 
   // workspaces
   DevBuf logb, logb64, post, gamma, alpha_ws, beta_ws, stats, logp_utt_d, score_d, psi_ws, path_d, tiles_dec, rank_in, rank_out;
-  int64_t stats_n = 0;
+  int64_t stats_n = 0;  // doubles of the statistics: [V][stats_size], or [2][V][stats_size] after hmmcu_estep_mmi
+  // MMI E-step: labels, round-major weights [H][U] and words [H-1][U] of the hypotheses, objective terms [U], their per-word
+  // sums [V][2], one denominator round's statistics [V][stats_size]
+  DevBuf mmi_label, mmi_w, mmi_hyp, mmi_term, mmi_obj, mmi_round;
+  int mmi_rounds = 0;
 };
 
 // k_fb_res takes the forward-backward of the current training map (otherwise k_fb does)
@@ -456,6 +461,7 @@ double hmmcu_last_kernel_ms(const hmmcu_ctx *ctx, const char *name) {
   if (strcmp(name, "dec_f16_active") == 0) return ctx->last_dec16 ? 1.0 : 0.0;
   if (strcmp(name, "acc_h_active") == 0) return ctx->last_acc_h ? 1.0 : 0.0;
   if (strcmp(name, "dec_grid") == 0) return (double)ctx->dec_grid;                // CTAs of the last k_emis_dec launch configuration
+  if (strcmp(name, "mmi_rounds") == 0) return (double)ctx->mmi_rounds;            // denominator rounds of the last hmmcu_estep_mmi
   // the k_fb_res batches of the current training map: how many, the most utterances in one, the teams that claim them
   if (strcmp(name, "res_batches") == 0) return res_fb_on(ctx) ? (double)ctx->n_res_batches : 0.0;
   if (strcmp(name, "res_batch_max") == 0) return res_fb_on(ctx) ? (double)ctx->res_batch_max : 0.0;
@@ -1516,9 +1522,9 @@ static int decode_emissions(hmmcu_ctx *ctx, int64_t fb0, int64_t fb1, bool *lay8
   return HMMCU_OK;
 }
 
-// mode 0: forward score, 1: Viterbi score
+// mode 0: forward score, 1: Viterbi score; into score_d [U][V], and copied to out_host unless it is NULL
 static int score_all(hmmcu_ctx *ctx, double *out_host, int mode, int emulate) {
-  if (!ctx || !out_host) return HMMCU_EINVAL;
+  if (!ctx) return HMMCU_EINVAL;
   if (ctx->primary) return fail(ctx, HMMCU_EINVAL, "scores: this context is a linked stream; call its primary");
   CK(cudaSetDevice(ctx->dev));
   int rc = ensure_packed(ctx);
@@ -1547,8 +1553,9 @@ static int score_all(hmmcu_ctx *ctx, double *out_host, int mode, int emulate) {
   // the scores of a batch go back to the host (copy stream) while the next batch is computed
   // (a call that fits one batch copies on the context's stream: no events, no second stream)
   const bool one_batch = ctx->off[ctx->U] - ctx->off[0] <= budget_frames;
+  const bool overlap = out_host && !one_batch;
   cudaEvent_t ev_done[2] = {nullptr, nullptr};
-  for (int k = 0; k < 2 && !one_batch; k++) CK(cudaEventCreateWithFlags(&ev_done[k], cudaEventDisableTiming));
+  for (int k = 0; k < 2 && overlap; k++) CK(cudaEventCreateWithFlags(&ev_done[k], cudaEventDisableTiming));
   struct EvGuard { cudaEvent_t *e; ~EvGuard() { for (int k = 0; k < 2; k++) if (e[k]) cudaEventDestroy(e[k]); } } ev_guard{ev_done};
   int pend_u0 = -1, pend_u1 = -1, nbatch = 0;
   auto copy_back = [&](int a, int b, cudaEvent_t ev) -> cudaError_t {
@@ -1588,7 +1595,7 @@ static int score_all(hmmcu_ctx *ctx, double *out_host, int mode, int emulate) {
     }
     LAUNCH_CHECK();
     t_end(ctx, mode == 0 ? "score" : "viterbi");
-    if (!one_batch) {
+    if (overlap) {
       CK(cudaEventRecord(ev_done[nbatch & 1], ctx->st));
       if (pend_u0 >= 0) CK(copy_back(pend_u0, pend_u1, ev_done[(nbatch - 1) & 1]));  // blocks this thread for pageable memory; the device works on
       pend_u0 = u0; pend_u1 = u1;
@@ -1596,9 +1603,9 @@ static int score_all(hmmcu_ctx *ctx, double *out_host, int mode, int emulate) {
     nbatch++;
     u0 = u1;
   }
-  if (one_batch) {
+  if (out_host && one_batch) {
     CK(cudaMemcpyAsync(out_host, ctx->score_d.p, sizeof(double) * (size_t)ctx->U * ctx->V, cudaMemcpyDeviceToHost, ctx->st));
-  } else {
+  } else if (overlap) {
     if (pend_u0 >= 0) CK(copy_back(pend_u0, pend_u1, ev_done[(nbatch - 1) & 1]));
     CK(cudaStreamSynchronize(ctx->st_copy));
   }
@@ -1606,8 +1613,10 @@ static int score_all(hmmcu_ctx *ctx, double *out_host, int mode, int emulate) {
   return HMMCU_OK;
 }
 
-int hmmcu_forward_scores(hmmcu_ctx *ctx, double *logp, int emulate_underflow) { return score_all(ctx, logp, 0, emulate_underflow); }
-int hmmcu_viterbi_scores(hmmcu_ctx *ctx, double *score) { return score_all(ctx, score, 1, 0); }
+int hmmcu_forward_scores(hmmcu_ctx *ctx, double *logp, int emulate_underflow) {
+  return logp ? score_all(ctx, logp, 0, emulate_underflow) : HMMCU_EINVAL;
+}
+int hmmcu_viterbi_scores(hmmcu_ctx *ctx, double *score) { return score ? score_all(ctx, score, 1, 0) : HMMCU_EINVAL; }
 
 int hmmcu_rank(hmmcu_ctx *ctx, const double *logp, int U, int V, double weight, int32_t *label, int32_t *second) {
   if (!ctx || !logp || !label || U < 0 || V < 1) return fail(ctx, HMMCU_EINVAL, "rank: bad arguments");
@@ -1872,8 +1881,10 @@ static int launch_pack_x16(hmmcu_ctx *ctx, cudaStream_t st) {
 // replace the context's own log-emissions in the recursions / its own state posteriors in the accumulators
 // (multi-stream models); with all phases and no replacement this is the plain single-stream E-step.  align: phase 2 is
 // the Viterbi alignment (k_vtrain) instead of forward-backward; it writes the same gamma and statistics, and its path.
+// w (device, [U]): the forward-backward weighted per utterance (an MMI denominator round), into mmi_round, not the
+// statistics buffer.
 static int estep_core(hmmcu_ctx *ctx, const int32_t *utt2model, int phases, const float *fb_logb, const float *acc_gamma,
-                      bool align = false) {
+                      bool align = false, const double *w = nullptr) {
   CK(cudaSetDevice(ctx->dev));
   int rc = ensure_packed(ctx);
   if (rc) return rc;
@@ -1922,9 +1933,10 @@ static int estep_core(hmmcu_ctx *ctx, const int32_t *utt2model, int phases, cons
   // ---- the launch sequence: statistics cleared, emissions, forward-backward, accumulators ----
   const float *lb_fb = fb_logb ? fb_logb : ctx->logb.as<float>();
   const float *gm_acc = acc_gamma ? acc_gamma : ctx->gamma.as<float>();
+  double *const sto = w ? ctx->mmi_round.as<double>() : ctx->stats.as<double>();
   const bool res_fb = res_fb_on(ctx);
   auto enqueue = [&]() -> int {
-    if (phases & 1) CK(cudaMemsetAsync(ctx->stats.p, 0, sizeof(double) * ctx->stats_n, ctx->st));
+    if (phases & 1) CK(cudaMemsetAsync(sto, 0, sizeof(double) * ctx->stats_n, ctx->st));
     if (U == 0) return HMMCU_OK;
     // masked utterances report 0 (k_fb_res writes the live ones only); cleared here, so that no memset node sits between the
     // emission kernel and k_fb_res
@@ -1961,22 +1973,30 @@ static int estep_core(hmmcu_ctx *ctx, const int32_t *utt2model, int phases, cons
           DISPATCH_N(N, (k_vtrain<NS, true><<<blocks, kVtThreads, vsm, ctx->st>>>(
                             lb_fb, ctx->off_d.as<int64_t>(), ctx->u2m_d.as<int32_t>(), ctx->A.as<double>(), U,
                             ctx->psi_ws.as<unsigned long long>(), ctx->path_d.as<int32_t>(), ctx->gamma.as<float>(),
-                            ctx->res_upos.as<int32_t>(), rows, ctx->stats.as<double>(), ss, off_lp, ctx->logp_utt_d.as<double>())));
+                            ctx->res_upos.as<int32_t>(), rows, sto, ss, off_lp, ctx->logp_utt_d.as<double>())));
         } else {
           DISPATCH_N(N, (k_vtrain<NS, false><<<blocks, kVtThreads, vsm, ctx->st>>>(
                             lb_fb, ctx->off_d.as<int64_t>(), ctx->u2m_d.as<int32_t>(), ctx->A.as<double>(), U,
                             ctx->psi_ws.as<unsigned long long>(), ctx->path_d.as<int32_t>(), ctx->gamma.as<float>(),
-                            ctx->res_upos.as<int32_t>(), nullptr, ctx->stats.as<double>(), ss, off_lp, ctx->logp_utt_d.as<double>())));
+                            ctx->res_upos.as<int32_t>(), nullptr, sto, ss, off_lp, ctx->logp_utt_d.as<double>())));
         }
         LAUNCH_CHECK();
         } else if (res_fb) {
         // every utterance resident in shared memory: log-emissions read once, gamma written once (fbres_kernels.cuh)
         const int grid = res_grid(ctx);
+        if (w) {
+          DISPATCH_N(N, CK(cudaFuncSetAttribute(k_fb_res<NS, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, kResSmemBytes));
+                     CK(launch_pdl(k_fb_res<NS, true>, grid, kResThreads, kResSmemBytes, ctx->st, lb_fb, ctx->off_d.as<int64_t>(),
+                                   ctx->u2m_d.as<int32_t>(), ctx->A.as<double>(), ctx->res_order.as<int32_t>(), ctx->res_upos.as<int32_t>(),
+                                   ctx->res_batches.as<ResBatch>(), (int)ctx->n_res_batches, ctx->res_counter.as<int>(),
+                                   ctx->gamma.as<float>(), ctx->ustats.as<double>(), ctx->logp_utt_d.as<double>(), w)));
+        } else {
         DISPATCH_N(N, CK(cudaFuncSetAttribute(k_fb_res<NS>, cudaFuncAttributeMaxDynamicSharedMemorySize, kResSmemBytes));
                    CK(launch_pdl(k_fb_res<NS>, grid, kResThreads, kResSmemBytes, ctx->st, lb_fb, ctx->off_d.as<int64_t>(),
                                  ctx->u2m_d.as<int32_t>(), ctx->A.as<double>(), ctx->res_order.as<int32_t>(), ctx->res_upos.as<int32_t>(),
                                  ctx->res_batches.as<ResBatch>(), (int)ctx->n_res_batches, ctx->res_counter.as<int>(),
-                                 ctx->gamma.as<float>(), ctx->ustats.as<double>(), ctx->logp_utt_d.as<double>())));
+                                 ctx->gamma.as<float>(), ctx->ustats.as<double>(), ctx->logp_utt_d.as<double>(), (const double *)nullptr)));
+        }
         LAUNCH_CHECK();
         }
         if (res_fb) {
@@ -1986,22 +2006,34 @@ static int estep_core(hmmcu_ctx *ctx, const int32_t *utt2model, int phases, cons
           CK(cudaEventRecord(ctx->ev_fork[0], ctx->st));
           CK(cudaStreamWaitEvent(ctx->st_aux[0], ctx->ev_fork[0], 0));
         }
-        k_fb_reduce<<<V, 1024, 0, fb_forked ? ctx->st_aux[0] : ctx->st>>>(ctx->ustats.as<double>(), N, ctx->mus_d.as<int32_t>(), V, ctx->stats.as<double>(), ss,
+        k_fb_reduce<<<V, 1024, 0, fb_forked ? ctx->st_aux[0] : ctx->st>>>(ctx->ustats.as<double>(), N, ctx->mus_d.as<int32_t>(), V, sto, ss,
                                                                         off_lp);
         LAUNCH_CHECK();
         if (fb_forked) CK(cudaEventRecord(ctx->ev_join[0], ctx->st_aux[0]));
       } else if (!align) {
       const int blocks = (U + kFbUtts - 1) / kFbUtts;
       const size_t fsm = fb_smem_bytes(N);
-      if (ctx->banded) {
+      if (w) {  // the weighted E-step of the MMI denominator
+        if (ctx->banded) {
+          DISPATCH_N(N, (cudaFuncSetAttribute(k_fb<NS, true, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)fsm), k_fb<NS, true, true><<<blocks, kFbThreads, fsm, ctx->st>>>(
+                            lb_fb, ctx->off_d.as<int64_t>(), ctx->u2m_d.as<int32_t>(), ctx->A.as<double>(), U,
+                            ctx->alpha_ws.as<uint32_t>(), ctx->beta_ws.as<uint32_t>(), ctx->gamma.as<float>(), sto,
+                            ss, off_lp, ctx->logp_utt_d.as<double>(), w)));
+        } else {
+          DISPATCH_N(N, (cudaFuncSetAttribute(k_fb<NS, false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)fsm), k_fb<NS, false, true><<<blocks, kFbThreads, fsm, ctx->st>>>(
+                            lb_fb, ctx->off_d.as<int64_t>(), ctx->u2m_d.as<int32_t>(), ctx->A.as<double>(), U,
+                            ctx->alpha_ws.as<uint32_t>(), ctx->beta_ws.as<uint32_t>(), ctx->gamma.as<float>(), sto,
+                            ss, off_lp, ctx->logp_utt_d.as<double>(), w)));
+        }
+      } else if (ctx->banded) {
         DISPATCH_N(N, (cudaFuncSetAttribute(k_fb<NS, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)fsm), k_fb<NS, true><<<blocks, kFbThreads, fsm, ctx->st>>>(
                           lb_fb, ctx->off_d.as<int64_t>(), ctx->u2m_d.as<int32_t>(), ctx->A.as<double>(), U,
-                          ctx->alpha_ws.as<uint32_t>(), ctx->beta_ws.as<uint32_t>(), ctx->gamma.as<float>(), ctx->stats.as<double>(),
+                          ctx->alpha_ws.as<uint32_t>(), ctx->beta_ws.as<uint32_t>(), ctx->gamma.as<float>(), sto,
                           ss, off_lp, ctx->logp_utt_d.as<double>())));
       } else {
         DISPATCH_N(N, (cudaFuncSetAttribute(k_fb<NS, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)fsm), k_fb<NS, false><<<blocks, kFbThreads, fsm, ctx->st>>>(
                           lb_fb, ctx->off_d.as<int64_t>(), ctx->u2m_d.as<int32_t>(), ctx->A.as<double>(), U,
-                          ctx->alpha_ws.as<uint32_t>(), ctx->beta_ws.as<uint32_t>(), ctx->gamma.as<float>(), ctx->stats.as<double>(),
+                          ctx->alpha_ws.as<uint32_t>(), ctx->beta_ws.as<uint32_t>(), ctx->gamma.as<float>(), sto,
                           ss, off_lp, ctx->logp_utt_d.as<double>())));
       }
       LAUNCH_CHECK();
@@ -2029,11 +2061,11 @@ static int estep_core(hmmcu_ctx *ctx, const int32_t *utt2model, int phases, cons
         CK(cudaFuncSetAttribute(k_accum_h, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
         CK(launch_pdl(k_accum_h, grid, kAhThreads, smem, ctx->st, ctx->acc_unitsH.as<TcTile>(), (int)ctx->n_acc_unitsH,
                       ctx->frame_ids_d.as<int32_t>(), ctx->x16.as<unsigned char>(), ctx->acc_images16.as<uint32_t>(), ctx->acc_kc.as<float>(),
-                      ctx->logb.as<float>(), gm_acc, N, M, G, D, DP, ctx->stats.as<double>(), ss, off_S0, off_S1, off_S2,
+                      ctx->logb.as<float>(), gm_acc, N, M, G, D, DP, sto, ss, off_S0, off_S1, off_S2,
                       ctx->acc_scratch.as<float>(), dsc));
         LAUNCH_CHECK();
       }
-      CK(launch_pdl(k_finalize_slots, dim3(G, V), 64 * kFinParts, 0, ctx->st, ctx->stats.as<double>(), ss, G, D, DP, 2 * DP, (G + 127) / 128,
+      CK(launch_pdl(k_finalize_slots, dim3(G, V), 64 * kFinParts, 0, ctx->st, sto, ss, G, D, DP, 2 * DP, (G + 127) / 128,
                     off_S0, off_S1, off_S2, ctx->ctr.as<double>(), ctx->mu.as<double>(), ctx->acc_scratch.as<float>(),
                     ctx->acc_slot_start_h.as<int32_t>(), ctx->acc_slot_ids_h.as<int32_t>(), dsc));
       LAUNCH_CHECK();
@@ -2045,10 +2077,10 @@ static int estep_core(hmmcu_ctx *ctx, const int32_t *utt2model, int phases, cons
         k_accum_ws<<<grid, kAccWsThreads, smem, ctx->st>>>(ctx->acc_units64.as<TcTile>(), (int)ctx->n_acc_units64, ctx->frame_ids_d.as<int32_t>(),
                                                            ctx->x32.as<float>(), ctx->acc_images.as<float>(), ctx->acc_kc.as<float>(),
                                                            ctx->logb.as<float>(), gm_acc, N, M, G, D, DP,
-                                                           ctx->stats.as<double>(), ss, off_S0, off_S1, off_S2, ctx->acc_scratch.as<float>());
+                                                           sto, ss, off_S0, off_S1, off_S2, ctx->acc_scratch.as<float>());
         LAUNCH_CHECK();
       }
-      k_finalize_slots<<<dim3(G, V), 64 * kFinParts, 0, ctx->st>>>(ctx->stats.as<double>(), ss, G, D, DP, tc_kp2(2 * DP), (G + 127) / 128, off_S0,
+      k_finalize_slots<<<dim3(G, V), 64 * kFinParts, 0, ctx->st>>>(sto, ss, G, D, DP, tc_kp2(2 * DP), (G + 127) / 128, off_S0,
                                                                   off_S1, off_S2, ctx->ctr.as<double>(), ctx->mu.as<double>(),
                                                                   ctx->acc_scratch.as<float>(), ctx->acc_slot_start.as<int32_t>(),
                                                                   ctx->acc_slot_ids.as<int32_t>());
@@ -2061,11 +2093,11 @@ static int estep_core(hmmcu_ctx *ctx, const int32_t *utt2model, int phases, cons
         k_accum_tc<<<grid, kTcThreads, smem, ctx->st>>>(ctx->acc_units.as<TcTile>(), (int)ctx->n_acc_units, ctx->frame_ids_d.as<int32_t>(),
                                                         ctx->x32.as<float>(), ctx->acc_images.as<float>(), ctx->acc_kc.as<float>(),
                                                         ctx->logb.as<float>(), gm_acc, N, M, G, D, DP,
-                                                        ctx->stats.as<double>(), ss, off_S0, off_S1, off_S2);
+                                                        sto, ss, off_S0, off_S1, off_S2);
         LAUNCH_CHECK();
       }
       const int64_t total = (int64_t)V * G * D;
-      k_finalize_stats<<<(unsigned)((total + 255) / 256), 256, 0, ctx->st>>>(ctx->stats.as<double>(), ss, V, G, D, off_S0, off_S1,
+      k_finalize_stats<<<(unsigned)((total + 255) / 256), 256, 0, ctx->st>>>(sto, ss, V, G, D, off_S0, off_S1,
                                                                             off_S2, ctx->ctr.as<double>(), ctx->mu.as<double>());
       LAUNCH_CHECK();
     } else {
@@ -2078,10 +2110,10 @@ static int estep_core(hmmcu_ctx *ctx, const int32_t *utt2model, int phases, cons
       k_accum_simt<<<grid, kAccThreads, smem, ctx->st>>>(ctx->x32.as<float>(), gm_acc, ctx->post.as<float>(),
                                                          ctx->mu32.as<float>(), ctx->off_d.as<int64_t>(),
                                                          ctx->mus_d.as<int32_t>(), ctx->mu_d.as<int32_t>(), N, M, D, DP, nparts,
-                                                         ctx->stats.as<double>(), ss, off_S0, off_S1, off_S2);
+                                                         sto, ss, off_S0, off_S1, off_S2);
       LAUNCH_CHECK();
       const int64_t total = (int64_t)V * G * D;
-      k_finalize_stats<<<(unsigned)((total + 255) / 256), 256, 0, ctx->st>>>(ctx->stats.as<double>(), ss, V, G, D, off_S0, off_S1,
+      k_finalize_stats<<<(unsigned)((total + 255) / 256), 256, 0, ctx->st>>>(sto, ss, V, G, D, off_S0, off_S1,
                                                                             off_S2, ctx->ctr.as<double>(), nullptr);
       LAUNCH_CHECK();
     }
@@ -2093,7 +2125,8 @@ static int estep_core(hmmcu_ctx *ctx, const int32_t *utt2model, int phases, cons
   ctx->last_tc = use_tc;
   if (phases & 4) ctx->last_acc_h = h_acc;
   // (pieces of a multi-stream E-step: plain launches)
-  const int rcq = (phases != 7 || fb_logb || acc_gamma) ? enqueue() : run_graphed(ctx, align ? ctx->g_estep_vit : ctx->g_estep, key, enqueue);
+  // (weighted: the rounds of the MMI denominator, each with its own map: plain launches, the graph slots stay as they are)
+  const int rcq = (phases != 7 || fb_logb || acc_gamma || w) ? enqueue() : run_graphed(ctx, align ? ctx->g_estep_vit : ctx->g_estep, key, enqueue);
   if (rcq == HMMCU_OK && pack16) { ctx->x16_x = ctx->x_version; ctx->x16_map = ctx->map_version; }
   return rcq;
 }
@@ -2167,23 +2200,87 @@ int hmmcu_em_reset(hmmcu_ctx *ctx) {
   return HMMCU_OK;
 }
 
+// The tail of a device M-step, once the new parameters are in place (enqueued after t_begin(ctx, "mstep")): the
+// accuracy-guard scan, the re-packing of the training path's model forms, and the control block back to the host.
+// The warp-specialised tensor-core path will want its packed model forms again right after the M-step: they are rebuilt
+// here, inside the same launch sequence, instead of lazily by the next E-step.
+static bool mstep_repacks(const hmmcu_ctx *ctx) {
+  return ctx->train_path == 2 && !ctx->pack_dirty && !ctx->ws_train.dirty && !ctx->acc_dirty && !ctx->kc_dirty &&
+         ctx->have_features && ctx->Dm == ctx->D;
+}
+static int mstep_tail_enqueue(hmmcu_ctx *ctx, bool repack) {
+  const int V = ctx->V;
+  int rc2;
+  // The accuracy-guard scan and the second W packer do not feed the main chain (new parameters -> kc -> emission
+  // images): they run on side streams, joined before the control block is read back.  With the per-kernel timers
+  // on everything stays on one stream, so that the timers keep their meaning.
+  const bool fork = !ctx->timing && ctx->mstep_fork;
+  auto on_stream = [&](cudaStream_t side, auto launch) -> int {
+    cudaStream_t keep = ctx->st;
+    ctx->st = side;
+    const int r = launch();
+    ctx->st = keep;
+    return r;
+  };
+  if (fork) {
+    CK(cudaEventRecord(ctx->ev_fork[0], ctx->st));
+    CK(cudaStreamWaitEvent(ctx->st_aux[0], ctx->ev_fork[0], 0));
+    if ((rc2 = on_stream(ctx->st_aux[0], [&] { return launch_kappa(ctx, ctx->ctl_d.as<double>() + 3 * V); })) != HMMCU_OK) return rc2;
+    CK(cudaEventRecord(ctx->ev_join[0], ctx->st_aux[0]));
+  } else {
+    if ((rc2 = launch_kappa(ctx, ctx->ctl_d.as<double>() + 3 * V)) != HMMCU_OK) return rc2;
+  }
+  t_end(ctx, "mstep");
+  if (repack) {
+    t_begin(ctx, "pack");
+    if ((rc2 = launch_pack_kc(ctx)) != HMMCU_OK) return rc2;
+    if (fork) {
+      CK(cudaEventRecord(ctx->ev_fork[1], ctx->st));
+      CK(cudaStreamWaitEvent(ctx->st_aux[1], ctx->ev_fork[1], 0));
+      if ((rc2 = on_stream(ctx->st_aux[1], [&] { return launch_pack_acc(ctx); })) != HMMCU_OK) return rc2;
+      CK(cudaEventRecord(ctx->ev_join[1], ctx->st_aux[1]));
+    }
+    if ((rc2 = launch_pack_ws(ctx, ctx->ws_train)) != HMMCU_OK) return rc2;
+    if (fork) CK(cudaStreamWaitEvent(ctx->st, ctx->ev_join[1], 0));
+    else if ((rc2 = launch_pack_acc(ctx)) != HMMCU_OK) return rc2;
+    t_end(ctx, "pack");
+  }
+  if (fork) CK(cudaStreamWaitEvent(ctx->st, ctx->ev_join[0], 0));
+  CK(cudaMemcpyAsync(ctx->ctl_h, ctx->ctl_d.p, sizeof(double) * (3 * (size_t)V + 1), cudaMemcpyDeviceToHost, ctx->st));
+  return HMMCU_OK;
+}
+// after the stream has been synchronised: the guard value, and which packed forms are now stale
+static void mstep_tail_finish(hmmcu_ctx *ctx, bool repack) {
+  ctx->kappa = ctx->ctl_h[3 * ctx->V];
+  ctx->kappa_stale = false;
+  if (repack) {  // the forms of the training path are current; every other packed form is stale
+    ctx->simt_dirty = true;
+    ctx->tc_train.dirty = true;
+    ctx->tc_dec.dirty = true;
+    ctx->ws_dec.dirty = true;
+  } else {
+    ctx->pack_dirty = true;
+  }
+}
+// the control block and the extremes' scratch of the guard scan
+static int mstep_prepare(hmmcu_ctx *ctx) {
+  int rc = ensure_ctl(ctx);
+  if (rc) return rc;
+  CK(ctx->upd_d.ensure(sizeof(int) * ctx->V));
+  const int DP = round_up(ctx->Dm + 1, 4);
+  CK(ctx->ext_d.ensure(sizeof(unsigned long long) * (2 * DP + 1)));
+  return HMMCU_OK;
+}
+
 int hmmcu_mstep(hmmcu_ctx *ctx, double threshold, double *sum_logp, double *n_utt, int32_t *updated) {
   if (!ctx || !ctx->have_models || ctx->stats_n != hmmcu_stats_size(ctx->N, ctx->M, ctx->Dm) * ctx->V || !ctx->em_old.p)
     return fail(ctx, HMMCU_EINVAL, "mstep: needs hmmcu_em_reset and an E-step on the current model set");
   CK(cudaSetDevice(ctx->dev));
   const int V = ctx->V;
-  int rc = ensure_ctl(ctx);
+  int rc = mstep_prepare(ctx);
   if (rc) return rc;
   const int64_t ssz = hmmcu_stats_size(ctx->N, ctx->M, ctx->Dm);
-  CK(ctx->upd_d.ensure(sizeof(int) * V));
-  {
-    const int DP = round_up(ctx->Dm + 1, 4);
-    CK(ctx->ext_d.ensure(sizeof(unsigned long long) * (2 * DP + 1)));
-  }
-  // The warp-specialised tensor-core path will want its packed model forms again right after this M-step: they
-  // are rebuilt here, inside the same launch sequence, instead of lazily by the next E-step.
-  const bool repack = ctx->train_path == 2 && !ctx->pack_dirty && !ctx->ws_train.dirty && !ctx->acc_dirty && !ctx->kc_dirty &&
-                      ctx->have_features && ctx->Dm == ctx->D;
+  const bool repack = mstep_repacks(ctx);
   auto enqueue = [&]() -> int {
     t_begin(ctx, "mstep");
     k_mstep_ctl<<<(V + 127) / 128, 128, 0, ctx->st>>>(ctx->stats.as<double>(), ssz, V, threshold, ctx->em_old.as<double>(),
@@ -2193,44 +2290,7 @@ int hmmcu_mstep(hmmcu_ctx *ctx, double threshold, double *sum_logp, double *n_ut
                   1.0e-5 /* FINITE_PROBAB, T-FS:39 */, ctx->upd_d.as<int>(), ctx->A.as<double>(), ctx->c.as<double>(),
                   ctx->mu.as<double>(), ctx->iv.as<double>(), ctx->det.as<double>()));
     LAUNCH_CHECK();
-    int rc2;
-    // The accuracy-guard scan and the second W packer do not feed the main chain (new parameters -> kc -> emission
-    // images): they run on side streams, joined before the control block is read back.  With the per-kernel timers
-    // on everything stays on one stream, so that the timers keep their meaning.
-    const bool fork = !ctx->timing && ctx->mstep_fork;
-    auto on_stream = [&](cudaStream_t side, auto launch) -> int {
-      cudaStream_t keep = ctx->st;
-      ctx->st = side;
-      const int r = launch();
-      ctx->st = keep;
-      return r;
-    };
-    if (fork) {
-      CK(cudaEventRecord(ctx->ev_fork[0], ctx->st));
-      CK(cudaStreamWaitEvent(ctx->st_aux[0], ctx->ev_fork[0], 0));
-      if ((rc2 = on_stream(ctx->st_aux[0], [&] { return launch_kappa(ctx, ctx->ctl_d.as<double>() + 3 * V); })) != HMMCU_OK) return rc2;
-      CK(cudaEventRecord(ctx->ev_join[0], ctx->st_aux[0]));
-    } else {
-      if ((rc2 = launch_kappa(ctx, ctx->ctl_d.as<double>() + 3 * V)) != HMMCU_OK) return rc2;
-    }
-    t_end(ctx, "mstep");
-    if (repack) {
-      t_begin(ctx, "pack");
-      if ((rc2 = launch_pack_kc(ctx)) != HMMCU_OK) return rc2;
-      if (fork) {
-        CK(cudaEventRecord(ctx->ev_fork[1], ctx->st));
-        CK(cudaStreamWaitEvent(ctx->st_aux[1], ctx->ev_fork[1], 0));
-        if ((rc2 = on_stream(ctx->st_aux[1], [&] { return launch_pack_acc(ctx); })) != HMMCU_OK) return rc2;
-        CK(cudaEventRecord(ctx->ev_join[1], ctx->st_aux[1]));
-      }
-      if ((rc2 = launch_pack_ws(ctx, ctx->ws_train)) != HMMCU_OK) return rc2;
-      if (fork) CK(cudaStreamWaitEvent(ctx->st, ctx->ev_join[1], 0));
-      else if ((rc2 = launch_pack_acc(ctx)) != HMMCU_OK) return rc2;
-      t_end(ctx, "pack");
-    }
-    if (fork) CK(cudaStreamWaitEvent(ctx->st, ctx->ev_join[0], 0));
-    CK(cudaMemcpyAsync(ctx->ctl_h, ctx->ctl_d.p, sizeof(double) * (3 * (size_t)V + 1), cudaMemcpyDeviceToHost, ctx->st));
-    return HMMCU_OK;
+    return mstep_tail_enqueue(ctx, repack);
   };
   uint64_t tbits;
   memcpy(&tbits, &threshold, sizeof(tbits));
@@ -2241,16 +2301,7 @@ int hmmcu_mstep(hmmcu_ctx *ctx, double threshold, double *sum_logp, double *n_ut
     if (n_utt) n_utt[v] = ctx->ctl_h[V + v];
     if (updated) updated[v] = ctx->ctl_h[2 * V + v] != 0.0;
   }
-  ctx->kappa = ctx->ctl_h[3 * V];
-  ctx->kappa_stale = false;
-  if (repack) {  // the forms of the training path are current; every other packed form is stale
-    ctx->simt_dirty = true;
-    ctx->tc_train.dirty = true;
-    ctx->tc_dec.dirty = true;
-    ctx->ws_dec.dirty = true;
-  } else {
-    ctx->pack_dirty = true;
-  }
+  mstep_tail_finish(ctx, repack);
   return HMMCU_OK;
 }
 
@@ -2543,3 +2594,120 @@ int hmmcu_viterbi(hmmcu_ctx *ctx, const int32_t *utt2model, double *score, int32
   return HMMCU_OK;
 }
 
+
+// ------------------------------------------------------------------------------- MMI training ----
+// hmmcu_estep_mmi: every cell scored into score_d (the computation of hmmcu_forward_scores, no copy-back), the
+// posteriors and hypotheses (k_mmi_post; only the hypotheses' words come back, set_train_map builds its tiles on the
+// host), the numerator (the plain E-step of the label map: block 0), the denominator in rounds (the weighted E-step of
+// each round's map into mmi_round, added into block 1 in round order), and block 1's tail (k_mmi_tail, copied in last).
+int hmmcu_estep_mmi(hmmcu_ctx *ctx, const int32_t *label, double kappa, int max_hyp, double *stats) {
+  if (!ctx) return HMMCU_EINVAL;
+  if (ctx->primary) return fail(ctx, HMMCU_EINVAL, "estep_mmi: this context is a linked stream; call its primary");
+  if (!ctx->linked.empty()) return fail(ctx, HMMCU_EINVAL, "estep_mmi: MMI training of multi-stream (linked) models is not supported");
+  if (!(kappa > 0.0) || max_hyp < 1 || max_hyp > HMMCU_MMI_MAX_HYP)
+    return fail(ctx, HMMCU_EINVAL, "estep_mmi: needs kappa > 0 and 1 <= max_hyp <= %d (kappa=%g, max_hyp=%d)", HMMCU_MMI_MAX_HYP, kappa, max_hyp);
+  CK(cudaSetDevice(ctx->dev));
+  int rc = ensure_packed(ctx);
+  if (rc) return rc;
+  const int U = ctx->U, V = ctx->V, H = max_hyp;
+  if (U > 0 && !label) return fail(ctx, HMMCU_EINVAL, "estep_mmi: label is NULL");
+  for (int u = 0; u < U; u++)
+    if (label[u] < -1 || label[u] >= V) return fail(ctx, HMMCU_EINVAL, "label[%d]=%d out of range", u, label[u]);
+  const int64_t ss = hmmcu_stats_size(ctx->N, ctx->M, ctx->D), n1 = ss * V;
+  // the whole [2][V][ss] buffer first: the E-steps below only ever grow it, so they keep it
+  CK(ctx->stats.ensure(sizeof(double) * 2 * n1));
+  CK(ctx->mmi_round.ensure(sizeof(double) * n1));
+  CK(ctx->mmi_obj.ensure(sizeof(double) * 2 * V));
+  std::vector<int32_t> hyp_h((size_t)(H - 1) * U);
+  if (U > 0) {
+    t_begin(ctx, "mmi_score");
+    if ((rc = score_all(ctx, nullptr, 0, 0)) != HMMCU_OK) return rc;
+    t_end(ctx, "mmi_score");
+    CK(ctx->mmi_label.ensure(sizeof(int32_t) * U));
+    CK(ctx->mmi_w.ensure(sizeof(double) * H * (size_t)U));
+    CK(ctx->mmi_hyp.ensure(sizeof(int32_t) * std::max(H - 1, 1) * (size_t)U));
+    CK(ctx->mmi_term.ensure(sizeof(double) * U));
+    CK(cudaMemcpyAsync(ctx->mmi_label.p, label, sizeof(int32_t) * U, cudaMemcpyHostToDevice, ctx->st));
+    t_begin(ctx, "mmi_post");
+    k_mmi_post<<<(U + kMmiWarps - 1) / kMmiWarps, kMmiWarps * 32, 0, ctx->st>>>(ctx->score_d.as<double>(), ctx->mmi_label.as<int32_t>(), U, V,
+                                                                               kappa, H, HMMCU_MMI_MIN_POST, ctx->mmi_w.as<double>(),
+                                                                               ctx->mmi_hyp.as<int32_t>(), ctx->mmi_term.as<double>());
+    LAUNCH_CHECK();
+    t_end(ctx, "mmi_post");
+    if (H > 1) CK(cudaMemcpyAsync(hyp_h.data(), ctx->mmi_hyp.p, sizeof(int32_t) * hyp_h.size(), cudaMemcpyDeviceToHost, ctx->st));
+    CK(cudaStreamSynchronize(ctx->st));
+  }
+  t_begin(ctx, "mmi_num");
+  if ((rc = estep_core(ctx, label, 7, nullptr, nullptr)) != HMMCU_OK) return rc;
+  t_end(ctx, "mmi_num");
+  double *blk1 = ctx->stats.as<double>() + n1;
+  CK(cudaMemsetAsync(blk1, 0, sizeof(double) * n1, ctx->st));
+  ctx->mmi_rounds = 0;
+  if (U > 0) {
+    // per-word objective terms while mus_d / mu_d hold the label map's grouping
+    k_mmi_tail<<<(V + 7) / 8, 256, 0, ctx->st>>>(ctx->mmi_term.as<double>(), ctx->mus_d.as<int32_t>(), ctx->mu_d.as<int32_t>(), V,
+                                                 ctx->mmi_obj.as<double>());
+    LAUNCH_CHECK();
+    t_begin(ctx, "mmi_den");
+    const int addb = (int)std::min<int64_t>((n1 + 255) / 256, (int64_t)ctx->sm_count * 8);
+    std::vector<int32_t> map(label, label + U);
+    for (int r = 0; r < H; r++) {
+      if (r > 0) {  // the r-th other hypothesis of every utterance; they are filled in rank order, so an empty round ends them
+        bool any = false;
+        for (int u = 0; u < U; u++) any |= (map[u] = hyp_h[(size_t)(r - 1) * U + u]) >= 0;
+        if (!any) break;
+      }
+      if ((rc = estep_core(ctx, map.data(), 7, nullptr, nullptr, false, ctx->mmi_w.as<double>() + (size_t)r * U)) != HMMCU_OK) return rc;
+      k_add_f64<<<addb, 256, 0, ctx->st>>>(blk1, ctx->mmi_round.as<double>(), n1);
+      LAUNCH_CHECK();
+      ctx->mmi_rounds++;
+    }
+    t_end(ctx, "mmi_den");
+    CK(cudaMemcpy2DAsync(blk1 + ss - 2, sizeof(double) * ss, ctx->mmi_obj.p, 2 * sizeof(double), 2 * sizeof(double), V,
+                         cudaMemcpyDeviceToDevice, ctx->st));
+  }
+  ctx->stats_n = 2 * n1;
+  if (stats) CK(cudaMemcpyAsync(stats, ctx->stats.p, sizeof(double) * ctx->stats_n, cudaMemcpyDeviceToHost, ctx->st));
+  CK(cudaStreamSynchronize(ctx->st));
+  return HMMCU_OK;
+}
+
+// hmmcu_mstep_ebw: k_mstep_ebw over the numerator and denominator blocks, then the tail every device M-step runs
+int hmmcu_mstep_ebw(hmmcu_ctx *ctx, double E, double tau) {
+  if (!ctx) return HMMCU_EINVAL;
+  if (!ctx->have_models || ctx->stats_n != 2 * hmmcu_stats_size(ctx->N, ctx->M, ctx->Dm) * ctx->V)
+    return fail(ctx, HMMCU_EINVAL, "mstep_ebw: needs an hmmcu_estep_mmi on the current model set");
+  if (!(E > 1.0) || !(tau >= 0.0)) return fail(ctx, HMMCU_EINVAL, "mstep_ebw: needs E > 1 and tau >= 0 (E=%g, tau=%g)", E, tau);
+  CK(cudaSetDevice(ctx->dev));
+  int rc = mstep_prepare(ctx);
+  if (rc) return rc;
+  const int64_t ss = hmmcu_stats_size(ctx->N, ctx->M, ctx->Dm);
+  const bool repack = mstep_repacks(ctx);
+  t_begin(ctx, "mstep");
+  k_mstep_ebw<<<dim3((ctx->G + 7) / 8, ctx->V), 256, 0, ctx->st>>>(ctx->stats.as<double>(), ctx->stats.as<double>() + ss * ctx->V, ss, ctx->N,
+                                                                  ctx->M, ctx->Dm, E, tau, 1.0e-5 /* FINITE_PROBAB, T-FS:39 */,
+                                                                  ctx->mu.as<double>(), ctx->iv.as<double>(), ctx->det.as<double>());
+  LAUNCH_CHECK();
+  if ((rc = mstep_tail_enqueue(ctx, repack)) != HMMCU_OK) return rc;
+  CK(cudaStreamSynchronize(ctx->st));
+  mstep_tail_finish(ctx, repack);
+  return HMMCU_OK;
+}
+
+// hmmh_train_mmi's read-back of the objective after the all-reduce: F = -sum_v den.sum_logp[v] and sum_v den.n_utt[v],
+// summed over the words in index order (library-internal)
+extern "C" __attribute__((visibility("hidden"))) int hmmcu_mmi_objective(hmmcu_ctx *ctx, double *F, double *n_utt) {
+  if (!ctx || !F || !n_utt) return HMMCU_EINVAL;
+  const int64_t ss = hmmcu_stats_size(ctx->N, ctx->M, ctx->Dm);
+  if (ctx->stats_n != 2 * ss * ctx->V) return fail(ctx, HMMCU_EINVAL, "mmi_objective: no MMI statistics");
+  CK(cudaSetDevice(ctx->dev));
+  std::vector<double> t(2 * (size_t)ctx->V);
+  CK(cudaMemcpy2DAsync(t.data(), 2 * sizeof(double), ctx->stats.as<double>() + ss * ctx->V + ss - 2, sizeof(double) * ss, 2 * sizeof(double),
+                       ctx->V, cudaMemcpyDeviceToHost, ctx->st));
+  CK(cudaStreamSynchronize(ctx->st));
+  double f = 0.0, n = 0.0;
+  for (int v = 0; v < ctx->V; v++) { f -= t[2 * v]; n += t[2 * v + 1]; }
+  *F = f;
+  *n_utt = n;
+  return HMMCU_OK;
+}

@@ -13,6 +13,7 @@
 
 #include "hmm_cuda.h"
 #include "em_loop.h"
+#include "../ebw_math.h"
 
 #define HM_THRESHOLD 1.0e-3 /* T-FS:37 */
 #define HM_DELTA 1          /* T-FS:38 */
@@ -218,6 +219,36 @@ int hmmh_mstep(hmmh_model *m, const double *stats) {
   return HMMCU_OK;
 }
 
+/* Extended Baum-Welch update of the means and variances (hmmcu_mstep_ebw; the arithmetic of ebw_math.h, shared with
+ * k_mstep_ebw).  num / den: one model's numerator and denominator statistics vectors.  Variances about the NEW mean. */
+int hmmh_mstep_ebw(hmmh_model *m, const double *num, const double *den, double E, double tau) {
+  if (!m || !num || !den || !(E > 1.0) || !(tau >= 0.0)) return HMMCU_EINVAL;
+  const int N = m->N, M = m->M, D = m->D;
+  const size_t G = (size_t)N * M, oS0 = (size_t)N * N + 2 * (size_t)N, oS1 = oS0 + G, oS2 = oS1 + G * D;
+  double *ds = (double *)malloc(sizeof(double) * 3 * (size_t)D), *dq = ds + D, *var = dq + D;
+  if (!ds) return HMMCU_ENOMEM;
+  for (size_t k = 0; k < G; k++) {
+    double *mu = m->mu + k * D, *iv = m->inv_var + k * D;
+    const double s0n = num[oS0 + k], s0d = den[oS0 + k];
+    const double sc = ebw_scale(s0n, tau), dg = s0n * sc - s0d;
+    double dmin = 0.0;
+    for (int d = 0; d < D; d++) {
+      const size_t i1 = oS1 + k * D + d, i2 = oS2 + k * D + d;
+      ds[d] = num[i1] * sc - den[i1];
+      dq[d] = ebw_q(num[i2], num[i1], s0n, mu[d]) * sc - ebw_q(den[i2], den[i1], s0d, mu[d]);
+      var[d] = 1.0 / iv[d];
+      dmin = fmax(dmin, ebw_root(dg, ds[d], dq[d], mu[d], var[d]));
+    }
+    const double Dc = fmax(2.0 * dmin, E * s0d);
+    if (!(dg + Dc > 0.0)) continue; /* no occupancy in either block: unchanged */
+    for (int d = 0; d < D; d++) ebw_update(dg, ds[d], dq[d], mu[d], var[d], Dc, HM_FLOOR, &mu[d], &var[d]);
+    memcpy(iv, var, sizeof(double) * D);
+    m->det[k] = det_then_invert(iv, D);
+  }
+  free(ds);
+  return HMMCU_OK;
+}
+
 /* ------------------------------------------------------------------ initial model ----------- */
 /* creating_initial_model T-FS:732-1317.  Segment k of an utterance of T frames is [seg[k], seg[k+1]):
  * T/N frames each, the first T%N segments one longer (T-FS:1005-1013). */
@@ -412,6 +443,28 @@ static int upload_models(hmmcu_ctx *ctx, const hmmh_model *models, int V) {
 
 int hmmh_upload_models(hmmcu_ctx *ctx, const hmmh_model *models, int V) { return upload_models(ctx, models, V); }
 
+/* The context's models back into the caller's V structs */
+int hmmh_download_models(hmmcu_ctx *ctx, hmmh_model *mp, int V) {
+  const int N = mp[0].N, M = mp[0].M, D = mp[0].D;
+  const size_t g = (size_t)N * M;
+  double *A = (double *)malloc(sizeof(double) * V * N * N), *c = (double *)malloc(sizeof(double) * V * g);
+  double *mu = (double *)malloc(sizeof(double) * V * g * D), *iv = (double *)malloc(sizeof(double) * V * g * D);
+  double *det = (double *)malloc(sizeof(double) * V * g);
+  int rc;
+  if (!A || !c || !mu || !iv || !det) rc = HMMCU_ENOMEM;
+  else if ((rc = hmmcu_get_models(ctx, A, c, mu, iv, det)) == HMMCU_OK) {
+    for (int v = 0; v < V; v++) {
+      memcpy(mp[v].A, A + (size_t)v * N * N, sizeof(double) * N * N);
+      memcpy(mp[v].c, c + v * g, sizeof(double) * g);
+      memcpy(mp[v].mu, mu + v * g * D, sizeof(double) * g * D);
+      memcpy(mp[v].inv_var, iv + v * g * D, sizeof(double) * g * D);
+      memcpy(mp[v].det, det + v * g, sizeof(double) * g);
+    }
+  }
+  free(A); free(c); free(mu); free(iv); free(det);
+  return rc;
+}
+
 /* T-FS:238-361 for V words at once and P feature streams (models[p * V + v] = stream p of word v; ctxs[p] holds
  * stream p's features; ctxs[1..] are linked to ctxs[0] here).  Every word keeps the reference's own stopping rule; a
  * word that has converged drops out of the following E-steps (its utterances are masked with -1).  estep(ctx, map)
@@ -461,25 +514,7 @@ int hmmh_em_loop(hmmcu_ctx *const *ctxs, int P, hmmh_model *models, int V, const
       if (!updated[v]) { active[v] = 0; n_active--; remap = 1; }
     }
   }
-  for (int p = 0; p < P && rc == HMMCU_OK; p++) {  /* bring the trained parameters back into the caller's structs */
-    hmmh_model *mp = models + (size_t)p * V;
-    const int N = mp[0].N, M = mp[0].M, D = mp[0].D;
-    const size_t g = (size_t)N * M;
-    double *A = (double *)malloc(sizeof(double) * V * N * N), *c = (double *)malloc(sizeof(double) * V * g);
-    double *mu = (double *)malloc(sizeof(double) * V * g * D), *iv = (double *)malloc(sizeof(double) * V * g * D);
-    double *det = (double *)malloc(sizeof(double) * V * g);
-    if (!A || !c || !mu || !iv || !det) rc = HMMCU_ENOMEM;
-    else if ((rc = hmmcu_get_models(ctxs[p], A, c, mu, iv, det)) == HMMCU_OK) {
-      for (int v = 0; v < V; v++) {
-        memcpy(mp[v].A, A + (size_t)v * N * N, sizeof(double) * N * N);
-        memcpy(mp[v].c, c + v * g, sizeof(double) * g);
-        memcpy(mp[v].mu, mu + v * g * D, sizeof(double) * g * D);
-        memcpy(mp[v].inv_var, iv + v * g * D, sizeof(double) * g * D);
-        memcpy(mp[v].det, det + v * g, sizeof(double) * g);
-      }
-    }
-    free(A); free(c); free(mu); free(iv); free(det);
-  }
+  for (int p = 0; p < P && rc == HMMCU_OK; p++) rc = hmmh_download_models(ctxs[p], models + (size_t)p * V, V);
   if (P > 1) hmmcu_link_streams(ctx, NULL, 0);
   free(probab); free(nutt); free(probab_q); free(nutt_q); free(updated); free(updated_q); free(active); free(map);
   return rc;
