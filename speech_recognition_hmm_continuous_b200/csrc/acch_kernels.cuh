@@ -25,7 +25,9 @@
 //     keeps 22 bits down to |x| = r / 512 (q: r / 8; with q in GEMM2 a one-frame Gaussian near the centre of data with
 //     r / sigma ~ 1000 missed the variance by 2e-4).
 // The weights w <= 1 are scaled by 2^14 (exact; a weight down to 2^-17 keeps 22 bits) and the sums are scaled back in double by
-// k_finalize_slots.
+// k_finalize_slots.  A weighted E-step (an MMI denominator round, whose weights carry the round's word posteriors, 1e-5 ..
+// 1e-3 and below) adds wshift to that exponent, so that its largest weight comes to [2^13, 2^14) as well; wback = 2^-wshift
+// undoes it in double (wshift 0, wback 1: unweighted E-steps are unchanged bit for bit).
 //
 // 13 warps: 0-7 epilogue (L -> w in place in tensor memory, drains of S, W images), 8-9 weight exponents (one thread per
 // frame: log2 gamma - logb log2 e for every state), 10 bulk-copy producer, 11 GEMM1 issuer, 12 GEMM2 issuer.
@@ -149,7 +151,7 @@ __global__ void __launch_bounds__(kAhThreads, 1)
 k_accum_h(const TcTile *__restrict__ units, int nunits, const int32_t *__restrict__ frame_ids, const unsigned char *__restrict__ x16,
           const uint32_t *__restrict__ images, const float *__restrict__ kcT, const float *__restrict__ logb, const float *__restrict__ gamma,
           int N, int M, int G, int D, int DP, double *__restrict__ stats, int64_t stats_stride, int64_t off_S0, int64_t off_S1, int64_t off_S2,
-          float *__restrict__ scratch, const float *__restrict__ dsc) {
+          float *__restrict__ scratch, const float *__restrict__ dsc, float wshift, double wback) {
   extern __shared__ __align__(1024) uint8_t smem_raw[];
   constexpr int NST = kAhStages, SUB = kAhSub;
   const int KP = 2 * DP, NK1 = KP / 16;
@@ -228,7 +230,7 @@ k_accum_h(const TcTile *__restrict__ units, int nunits, const int32_t *__restric
         float cf = kNegInf;
         // (+ 14: the weights' scale 2^14.  cf is ~ +200 and rounded to 2^-16 as it is; added to kc in the epilogue the 14 would
         // cost another rounding of that size)
-        if (cur.gm[st] > 0.f && cur.lb[st] > kNegInf) cf = fmaf(cur.lb[st], -1.4426950408889634f, __log2f(cur.gm[st]) + kAhWLog2);
+        if (cur.gm[st] > 0.f && cur.lb[st] > kNegInf) cf = fmaf(cur.lb[st], -1.4426950408889634f, __log2f(cur.gm[st]) + (kAhWLog2 + wshift));
         sts_f32(cfs + st * SUB * 4, cf);
       }
       mbar_arrive_a(x_full + 8 * s);
@@ -427,7 +429,7 @@ k_accum_h(const TcTile *__restrict__ units, int nunits, const int32_t *__restric
             double *stp = stats + (int64_t)cur_v * stats_stride;
             for (int k = c8_beg * 8; k < c8_end * 8; k++) {
               const uint32_t a = my_acc + (uint32_t)k * 512;
-              const double val = (double)lds_f32(a) * (double)__ldg(dsc + k);
+              const double val = (double)lds_f32(a) * ((double)__ldg(dsc + k) * wback);
               sts_f32(a, 0.f);
               if (g < G) {
                 if (k < D) atomicAdd(stp + off_S1 + (int64_t)g * D + k, val);

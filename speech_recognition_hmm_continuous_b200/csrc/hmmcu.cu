@@ -1882,9 +1882,9 @@ static int launch_pack_x16(hmmcu_ctx *ctx, cudaStream_t st) {
 // (multi-stream models); with all phases and no replacement this is the plain single-stream E-step.  align: phase 2 is
 // the Viterbi alignment (k_vtrain) instead of forward-backward; it writes the same gamma and statistics, and its path.
 // w (device, [U]): the forward-backward weighted per utterance (an MMI denominator round), into mmi_round, not the
-// statistics buffer.
+// statistics buffer; k_accum_h scales its weights by a further 2^wshift (acch_kernels.cuh).
 static int estep_core(hmmcu_ctx *ctx, const int32_t *utt2model, int phases, const float *fb_logb, const float *acc_gamma,
-                      bool align = false, const double *w = nullptr) {
+                      bool align = false, const double *w = nullptr, int wshift = 0) {
   CK(cudaSetDevice(ctx->dev));
   int rc = ensure_packed(ctx);
   if (rc) return rc;
@@ -2062,12 +2062,12 @@ static int estep_core(hmmcu_ctx *ctx, const int32_t *utt2model, int phases, cons
         CK(launch_pdl(k_accum_h, grid, kAhThreads, smem, ctx->st, ctx->acc_unitsH.as<TcTile>(), (int)ctx->n_acc_unitsH,
                       ctx->frame_ids_d.as<int32_t>(), ctx->x16.as<unsigned char>(), ctx->acc_images16.as<uint32_t>(), ctx->acc_kc.as<float>(),
                       ctx->logb.as<float>(), gm_acc, N, M, G, D, DP, sto, ss, off_S0, off_S1, off_S2,
-                      ctx->acc_scratch.as<float>(), dsc));
+                      ctx->acc_scratch.as<float>(), dsc, (float)wshift, ldexp(1.0, -wshift)));
         LAUNCH_CHECK();
       }
       CK(launch_pdl(k_finalize_slots, dim3(G, V), 64 * kFinParts, 0, ctx->st, sto, ss, G, D, DP, 2 * DP, (G + 127) / 128,
                     off_S0, off_S1, off_S2, ctx->ctr.as<double>(), ctx->mu.as<double>(), ctx->acc_scratch.as<float>(),
-                    ctx->acc_slot_start_h.as<int32_t>(), ctx->acc_slot_ids_h.as<int32_t>(), dsc));
+                    ctx->acc_slot_start_h.as<int32_t>(), ctx->acc_slot_ids_h.as<int32_t>(), dsc, ldexp(1.0, -wshift)));
       LAUNCH_CHECK();
     } else if (ws_acc) {
       const size_t smem = ws_acc_smem_bytes(2 * DP);
@@ -2619,6 +2619,7 @@ int hmmcu_estep_mmi(hmmcu_ctx *ctx, const int32_t *label, double kappa, int max_
   CK(ctx->mmi_round.ensure(sizeof(double) * n1));
   CK(ctx->mmi_obj.ensure(sizeof(double) * 2 * V));
   std::vector<int32_t> hyp_h((size_t)(H - 1) * U);
+  std::vector<double> w_h((size_t)H * U);
   if (U > 0) {
     t_begin(ctx, "mmi_score");
     if ((rc = score_all(ctx, nullptr, 0, 0)) != HMMCU_OK) return rc;
@@ -2635,6 +2636,7 @@ int hmmcu_estep_mmi(hmmcu_ctx *ctx, const int32_t *label, double kappa, int max_
     LAUNCH_CHECK();
     t_end(ctx, "mmi_post");
     if (H > 1) CK(cudaMemcpyAsync(hyp_h.data(), ctx->mmi_hyp.p, sizeof(int32_t) * hyp_h.size(), cudaMemcpyDeviceToHost, ctx->st));
+    CK(cudaMemcpyAsync(w_h.data(), ctx->mmi_w.p, sizeof(double) * w_h.size(), cudaMemcpyDeviceToHost, ctx->st));
     CK(cudaStreamSynchronize(ctx->st));
   }
   t_begin(ctx, "mmi_num");
@@ -2657,7 +2659,13 @@ int hmmcu_estep_mmi(hmmcu_ctx *ctx, const int32_t *label, double kappa, int max_
         for (int u = 0; u < U; u++) any |= (map[u] = hyp_h[(size_t)(r - 1) * U + u]) >= 0;
         if (!any) break;
       }
-      if ((rc = estep_core(ctx, map.data(), 7, nullptr, nullptr, false, ctx->mmi_w.as<double>() + (size_t)r * U)) != HMMCU_OK) return rc;
+      // the round's largest weight w_max = f 2^e, f in [0.5, 1): k_accum_h scales the round by 2^-e more (at most 2^60)
+      double wmax = 0.0;
+      for (int u = 0; u < U; u++) wmax = std::max(wmax, w_h[(size_t)r * U + u]);
+      int e = 0;
+      if (wmax > 0.0) frexp(wmax, &e);
+      const int wshift = std::min(std::max(-e, 0), 60);
+      if ((rc = estep_core(ctx, map.data(), 7, nullptr, nullptr, false, ctx->mmi_w.as<double>() + (size_t)r * U, wshift)) != HMMCU_OK) return rc;
       k_add_f64<<<addb, 256, 0, ctx->st>>>(blk1, ctx->mmi_round.as<double>(), n1);
       LAUNCH_CHECK();
       ctx->mmi_rounds++;

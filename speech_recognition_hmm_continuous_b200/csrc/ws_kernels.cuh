@@ -1138,7 +1138,7 @@ __global__ void __launch_bounds__(64 * kFinParts)
 k_finalize_slots(double *__restrict__ stats, int64_t stats_stride, int G, int D, int DP, int KP2, int nRB, int64_t off_S0,
                  int64_t off_S1, int64_t off_S2, const double *__restrict__ ctr, const double *__restrict__ mu,
                  const float *__restrict__ scratch, const int32_t *__restrict__ slot_start, const int32_t *__restrict__ slot_ids,
-                 const float *__restrict__ dsc = nullptr) {  // dsc: per-column factors of k_accum_h's scaled sums (powers of two)
+                 const float *__restrict__ dsc = nullptr, double wback = 1.0) {  // dsc, wback: k_accum_h's scale factors (powers of two)
   const int v = blockIdx.y, g = blockIdx.x, d = threadIdx.x & 63, part = threadIdx.x >> 6;
   const bool lived = d < D;
   double *st = stats + (int64_t)v * stats_stride;
@@ -1153,8 +1153,8 @@ k_finalize_slots(double *__restrict__ stats, int64_t stats_stride, int G, int D,
     if (lived) { s1 += (double)sl[d]; s2 += (double)sl[DP + d]; }
   }
   if (dsc) {
-    s0 *= (double)dsc[D];
-    if (lived) { s1 *= (double)dsc[d]; s2 *= (double)dsc[DP + d]; }
+    s0 *= (double)dsc[D] * wback;
+    if (lived) { s1 *= (double)dsc[d] * wback; s2 *= (double)dsc[DP + d] * wback; }
   }
   sp[part][0][d] = s0; sp[part][1][d] = s1; sp[part][2][d] = s2;
   // the statistics the atomic path may have left (CTAs that walked through many small images)

@@ -56,7 +56,7 @@ def _check_buffer(ctx, ms, x, off, label, S, kappa, H, stats, exact=True):
         sp, wp = api.split_stats(stats[1, v], N, M, D), api.split_stats(want[1, v], N, M, D)
         if wp["S0"].sum() > 0:
             _assert_mixture_stats(sp, types.SimpleNamespace(S0=wp["S0"], S1=wp["S1"], S2c=wp["S2c"]), x)
-        for name in ("den_trans", "den_mix"):
+        for name in ("num_trans", "den_trans", "den_mix"):
             assert np.allclose(sp[name], wp[name], rtol=RTOL, atol=1e-6 * max(np.abs(wp[name]).max(), 1.0)), (v, name)
         inc = [u for u in range(len(label)) if label[u] == v and np.isfinite(term[u])]
         assert stats[1, v, ss - 1] == len(inc)
